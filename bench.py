@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py — benchmark of the edwards25519 hot path (BASELINE.json metric), with parity checks in the code path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 20] [--no-extras]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 20] [--no-extras] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes, on rank 0, what the last timed step returned: the statuses of the device-resident verify
+(verify_status.npy) and of the host-buffer verify (e2e_verify_status.npy), as float32.  The inputs depend only on the
+arguments, so two builds can be compared output for output.
 
 Headline (config.workload): BASELINE.json configs[1] — batched EdDSA verification
 (eddsa::verify_with_checks, sign/eddsa/eddsa_sig.rs:159-212) of 2^20 random keys / 64-byte messages / signatures
@@ -36,6 +40,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the source tree, which may be read-only
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -198,6 +203,24 @@ def die(msg: str):
     os._exit(3)     # non-zero for the driver; os._exit so that no other rank's barrier can hang the exit
 
 
+DUMP_BYTES = 60 << 20     # all files of --dump-outputs together, .npy headers included, stay under 64 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes every array as out_dir/<name>.npy in float32.  An array larger than its equal share of DUMP_BYTES is cut
+    to a fixed sample: the elements at sorted indices drawn with seed 0 (the same for every run of the same size),
+    whose indices go to <name>_index.npy as float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a).reshape(-1)
+        if 4 * a.size > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // 12, replace=False))
+            np.save(os.path.join(out_dir, name + "_index.npy"), idx.astype(np.float64))
+            a = a[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 def cpu_verify_baseline(C, pk, msg, off, sig, gpu_status, budget_s: float, threads: int):
     """Times the oracle's C port on a bounded prefix (adaptive: ~budget_s of CPU work) and checks the GPU statuses of
     that prefix against it."""
@@ -280,7 +303,10 @@ def main():
     ap.add_argument("--log2n", type=int, default=20)
     ap.add_argument("--no-extras", action="store_true", help="headline only (configs 1, 3, 4, 5 and the stage measurements are skipped)")
     ap.add_argument("--msm-max-log2", type=int, default=26)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the statuses of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -405,6 +431,9 @@ def main():
     clocks = sampler.stop()
     total_ms = ev[0].elapsed_time(ev[-1])
     kernel_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
+    dumped = {}
+    if args.dump_outputs and rank == 0:
+        dumped["verify_status"] = d_st.cpu().numpy()
     # the two launches of a step one by one: events recorded by the library around each launch, read back after
     # every step (a second pass, so that the read-back's synchronisation stays out of the timed region above)
     ctx.verify_kernel_timing(True)
@@ -446,6 +475,8 @@ def main():
             mctx.verify_batch(h_pk, h_msg, h_off, h_sig, out=h_out)
         e2e_s = time.perf_counter() - t0
         e2e_launches = mctx.launches - ml0
+        if args.dump_outputs:
+            dumped["e2e_verify_status"] = h_out.copy()
         if not (h_out == big_expect).all():
             die("e2e statuses (multi-device context) differ from the expected ones")
         e2e_value = world * n * args.steps / e2e_s
@@ -485,6 +516,8 @@ def main():
             dist.destroy_process_group()
         return
 
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
     kernel_s = statistics.mean(kernel_ms) * 1e-3
     achieved = n * IMAD_EQ_PER_VERIFY / kernel_s
     prep_s, main_s = statistics.mean(k_prep_ms) * 1e-3, statistics.mean(k_main_ms) * 1e-3
