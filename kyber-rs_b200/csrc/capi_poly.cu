@@ -7,9 +7,9 @@
 // commitments -> cached form into scratch slots 8 (cached) / 9 (bad flags); then the eval kernel.
 //   d_shares != 0           verdicts of the share checks into d_out (one byte per item)
 //   d_shares == 0, d_out    encodings of the evaluations into d_out, per-item status into d_status
-//   d_shares == 0, !d_out   the evaluations stay as (X, Y, Z) in scratch slot KB_SLOT_XYZ, status into d_status
+//   d_shares == 0, !d_out   the evaluations stay as (X, Y, Z) in scratch, *d_xyz points at them; status into d_status
 int kb_poly_run(kb_ctx* ctx, size_t npoly, size_t t, const void* d_commits, int limbs, size_t m, const uint32_t* d_poly_id, const uint32_t* d_idx, size_t n_verifiers,
-                       const uint8_t* d_shares, uint8_t* d_out, uint8_t* d_status, cudaStream_t st)
+                       const uint8_t* d_shares, uint8_t* d_out, uint8_t* d_status, const uint32_t** d_xyz, cudaStream_t st)
 {
     uint32_t* cached;
     uint8_t* bad;
@@ -27,7 +27,10 @@ int kb_poly_run(kb_ctx* ctx, size_t npoly, size_t t, const void* d_commits, int 
         KB_SCRATCH(KB_SLOT_XYZ, 96 * m, xyz);
         k_poly_eval<<<kb_blocks(m, KB_THREADS), KB_THREADS, 0, st>>>(m, npoly, t, cached, bad, d_poly_id, d_idx, n_verifiers, nullptr, xyz, d_status, nullptr, ctx->base_table);
         KB_LAUNCHED();
-        if (!d_out) return KB_OK;   // the caller goes on with the uncompressed values in KB_SLOT_XYZ
+        if (!d_out) {   // the caller goes on with the uncompressed values
+            *d_xyz = xyz;
+            return KB_OK;
+        }
         k_compress_batch<<<kb_blocks((m + KB_INV_K - 1) / KB_INV_K, KB_THREADS), KB_THREADS, 0, st>>>(m, xyz, d_status, d_out);
         KB_LAUNCHED();
     }
@@ -223,7 +226,7 @@ int kb_dkg_round_run(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, const voi
 {
     const size_t h = kb_dkg_plan(ctx, n, t, ndealers);
     if (h) return kb_dkg_fd_run(ctx, n, t, ndealers, h, d_commits, limbs, d_shares, d_verdict, st);
-    return kb_poly_run(ctx, ndealers, t, d_commits, limbs, n * ndealers, nullptr, nullptr, n, d_shares, d_verdict, nullptr, st);
+    return kb_poly_run(ctx, ndealers, t, d_commits, limbs, n * ndealers, nullptr, nullptr, n, d_shares, d_verdict, nullptr, nullptr, st);
 }
 
 extern "C" {
@@ -266,7 +269,7 @@ static int kb_poly_host(kb_ctx* ctx, size_t npoly, size_t t, const uint8_t* comm
         KB_SCRATCH(2, 32 * m, d_sh);
         KB_H2D(d_sh, shares, 32 * m);
     }
-    int rc = kb_poly_run(ctx, npoly, t, d_c, 0, m, d_pid, d_idx, 0, d_sh, d_o, d_st, ctx->stream);
+    int rc = kb_poly_run(ctx, npoly, t, d_c, 0, m, d_pid, d_idx, 0, d_sh, d_o, d_st, nullptr, ctx->stream);
     if (rc != KB_OK) return rc;
     KB_D2H(out, d_o, out_bytes);
     if (status && !shares) KB_D2H(status, d_st, m);

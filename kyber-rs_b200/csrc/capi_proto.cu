@@ -146,9 +146,10 @@ int kb_vss_rabin_verify_deals_batch(kb_ctx* ctx, size_t npoly, size_t t, const u
     KB_H2D(d_f, f_shares, 32 * m);
     KB_H2D(d_g, g_shares, 32 * m);
     KB_H2D(d_h, h_point, 32);
-    int rc = kb_poly_run(ctx, npoly, t, d_c, 0, m, d_pid, d_idx, 0, nullptr, nullptr, d_st, ctx->stream);
+    const uint32_t* evals;
+    int rc = kb_poly_run(ctx, npoly, t, d_c, 0, m, d_pid, d_idx, 0, nullptr, nullptr, d_st, &evals, ctx->stream);
     if (rc == KB_OK) {
-        k_rabin_finish<<<kb_blocks(m, KB_THREADS), KB_THREADS, 64 * 8 * 96, ctx->stream>>>(m, (const uint32_t*)ctx->slot[KB_SLOT_XYZ], d_st, d_f, d_g, d_h, ctx->base_table, d_v);
+        k_rabin_finish<<<kb_blocks(m, KB_THREADS), KB_THREADS, 64 * 8 * 96, ctx->stream>>>(m, evals, d_st, d_f, d_g, d_h, ctx->base_table, d_v);
         ctx->launches++;
         const cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) rc = kb_fail(ctx, e, "launch");
@@ -217,9 +218,10 @@ int kb_dss_verify_partials(kb_ctx* ctx, size_t t, const uint8_t* random_commits,
         free(hp);
         if (e != cudaSuccess) return kb_fail(ctx, e, "dss index upload");
         KB_H2D(d_p, partials, 32 * m);
-        int rc = kb_poly_run(ctx, 2, t, d_c, 0, 2 * m, d_pid, d_idx, 0, nullptr, nullptr, d_st, ctx->stream);
+        const uint32_t* evals;
+        int rc = kb_poly_run(ctx, 2, t, d_c, 0, 2 * m, d_pid, d_idx, 0, nullptr, nullptr, d_st, &evals, ctx->stream);
         if (rc != KB_OK) return rc;
-        k_dss_finish<<<kb_blocks(m, KB_THREADS), KB_THREADS, 0, ctx->stream>>>(m, (const uint32_t*)ctx->slot[KB_SLOT_XYZ], d_st, d_hash, d_p, ctx->comb, d_v);
+        k_dss_finish<<<kb_blocks(m, KB_THREADS), KB_THREADS, 0, ctx->stream>>>(m, evals, d_st, d_hash, d_p, ctx->comb, d_v);
         KB_LAUNCHED();
         KB_D2H(verdict, d_v, m);
     }
@@ -336,7 +338,7 @@ int kb_dkg_resharing_key(kb_ctx* ctx, size_t new_t, size_t k, const uint32_t* id
         KB_CUDA(cudaMemcpyAsync(d_one, hv, 8, cudaMemcpyHostToDevice, ctx->stream));
         KB_H2D(d_sh, share32, 32);
         KB_CUDA(cudaStreamSynchronize(ctx->stream));   // hv is on this stack frame
-        rc = kb_poly_run(ctx, 1, new_t, d_o, 0, 1, d_one, d_one + 1, 0, d_sh, d_v, nullptr, ctx->stream);
+        rc = kb_poly_run(ctx, 1, new_t, d_o, 0, 1, d_one, d_one + 1, 0, d_sh, d_v, nullptr, nullptr, ctx->stream);
         cudaMemsetAsync(d_sh, 0, 32, ctx->stream);
         if (rc != KB_OK) {
             cudaStreamSynchronize(ctx->stream);

@@ -10,8 +10,6 @@
 #define KB_FE_SUBMASK
 #include "ctx.cuh"
 #include "kernels.cuh"
-// per-signature scratch of the verifiers: 304-byte records (half-size-scalar path) / 96-byte points (full-length path)
-static_assert(KB_VERIFY_SCRATCH_BYTES == 4 * KB_HALF_REC_WORDS, "ctx.cuh: KB_VERIFY_SCRATCH_BYTES");
 int kb_verify_launch(kb_ctx* ctx, size_t n, const uint8_t* d_pk, const uint8_t* d_msg, const uint64_t* d_msg_off, uint64_t msg_base, const uint8_t* d_sig, uint8_t* d_status, int schnorr,
                             uint32_t* xyz, uint8_t* fl, cudaStream_t st)
 {
@@ -19,7 +17,7 @@ int kb_verify_launch(kb_ctx* ctx, size_t n, const uint8_t* d_pk, const uint8_t* 
     const unsigned g1 = kb_blocks(n, th), g2 = kb_blocks((n + KB_INV_K - 1) / KB_INV_K, KB_THREADS);
     const bool tm = ctx->timing != 0;
     if (!ctx->verify_full) {
-        // the 96-byte-per-item xyz scratch of the full-length path is not needed; `xyz` carries the 304-byte records
+        // the 96-byte-per-item xyz scratch of the full-length path is not needed; `xyz` carries the records
         const unsigned gp = kb_blocks(n, KB_THREADS);
         if (tm) cudaEventRecord(ctx->tev[0], st);
         if (ctx->verify_split == 2 || (ctx->verify_split && n >= (size_t)ctx->sm_count * KB_THREADS)) {   // 2: every batch size (tests)

@@ -144,7 +144,9 @@ int kb_dev_end(kb_ctx* ctx, cudaStream_t st);
 // capi_verify.cu: the two launches of a signature-verification batch on device buffers
 int kb_verify_launch(kb_ctx* ctx, size_t n, const uint8_t* d_pk, const uint8_t* d_msg, const uint64_t* d_msg_off, uint64_t msg_base, const uint8_t* d_sig, uint8_t* d_status, int schnorr,
                      uint32_t* xyz, uint8_t* fl, cudaStream_t st);
-#define KB_VERIFY_SCRATCH_BYTES 304   // per signature in `xyz` (4 * KB_HALF_REC_WORDS)
+// bytes per signature of the `xyz` scratch: one record of the half-size-scalar path (kernels.cuh), more than the 96 of the
+// full-length path
+#define KB_VERIFY_SCRATCH_BYTES (4 * KB_HALF_REC_WORDS)
 // bytes of the `fl` scratch of kb_verify_launch: one flag byte per signature (full-length path) or, for the half-size-scalar
 // path, the order in which the main kernel walks the records — uint32 perm[n], uint8 keys[n], 2 x 129 counters
 #define KB_VERIFY_FLAG_BYTES(n) (5 * (size_t)(n) + 4096)
@@ -154,5 +156,5 @@ int kb_msm_run(kb_ctx* ctx, size_t n, const uint8_t* d_scalars, const void* d_po
 // capi_poly.cu: a deal-verification round on device buffers (commitments as 32-byte encodings, or as the reference's
 // 40-limb in-memory form when limbs != 0)
 int kb_poly_run(kb_ctx* ctx, size_t npoly, size_t t, const void* d_commits, int limbs, size_t m, const uint32_t* d_poly_id, const uint32_t* d_idx, size_t n_verifiers,
-                const uint8_t* d_shares, uint8_t* d_out, uint8_t* d_status, cudaStream_t st);
+                const uint8_t* d_shares, uint8_t* d_out, uint8_t* d_status, const uint32_t** d_xyz, cudaStream_t st);
 int kb_dkg_round_run(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, const void* d_commits, int limbs, const uint8_t* d_shares, uint8_t* d_verdict, cudaStream_t st);

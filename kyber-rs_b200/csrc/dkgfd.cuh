@@ -210,21 +210,6 @@ KB_HD size_t kb_fd_part_len(size_t t, size_t h, size_t q) { return (q + 1) * h <
 #define KB_FD_CONV_MINBLOCKS 3
 #endif
 
-__device__ __forceinline__ void kb_fd_load(ge_p3& p, const uint32_t* o)
-{
-    kb_load_fe(p.X, o);
-    kb_load_fe(p.Y, o + 8);
-    kb_load_fe(p.Z, o + 16);
-    kb_load_fe(p.T, o + 24);
-}
-__device__ __forceinline__ void kb_fd_store(uint32_t* o, const ge_p3& p)
-{
-    kb_store_fe(o, p.X);
-    kb_store_fe(o + 8, p.Y);
-    kb_store_fe(o + 16, p.Z);
-    kb_store_fe(o + 24, p.T);
-}
-
 // dec[j][d] = commitment j of dealer d, decoded; dealer_bad[d] |= 1 if any commitment does not decode
 static __global__ void __launch_bounds__(KB_THREADS) k_fd_decode(size_t nd, size_t t, const uint8_t* commits, uint32_t* dec, uint32_t* dealer_bad)
 {
@@ -238,7 +223,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_fd_decode(size_t nd, size
         ge_identity(p);
         atomicOr(dealer_bad + d, 1u);
     }
-    kb_fd_store(KB_FD_AT(dec, j, d, nd), p);
+    kb_store_p3_w128(KB_FD_AT(dec, j, d, nd), p);
 }
 // The same from the reference's in-memory / serde form of a Point: X, Y, Z, T as 10 signed 25.5-bit limbs each
 // (ge.rs:75-83).  That form is not validated by the reference (SURVEY §8f-3); here an element that is not a
@@ -253,7 +238,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_fd_decode_limbs(size_t nd
         ge_identity(p);
         atomicOr(dealer_bad + d, 1u);
     }
-    kb_fd_store(KB_FD_AT(dec, j, d, nd), p);
+    kb_store_p3_w128(KB_FD_AT(dec, j, d, nd), p);
 }
 
 // Stage A, iteration s = 1 .. h-1.  Block q of a dealer has length hq; it is right-aligned in the iteration count
@@ -284,14 +269,14 @@ static __global__ void __launch_bounds__(KB_FD_CONV_THREADS, KB_FD_CONV_MINBLOCK
         hq = hl;
     }
     ge_p3 v, lower;
-    if (k == 1) kb_fd_load(lower, KB_FD_AT(dec, q * h + (hq - sq), d, nd));
-    else kb_fd_load(lower, KB_FD_AT(src, q * h + k - 1, d, nd));
+    if (k == 1) kb_load_p3_w128(lower, KB_FD_AT(dec, q * h + (hq - sq), d, nd));
+    else kb_load_p3_w128(lower, KB_FD_AT(src, q * h + k - 1, d, nd));
     const bool has_self = k < sq;
-    if (has_self) kb_fd_load(v, KB_FD_AT(src, q * h + k, d, nd));
+    if (has_self) kb_load_p3_w128(v, KB_FD_AT(src, q * h + k, d, nd));
     kb_naf kn;
     kb_naf_from(kn, (uint64_t)k);
     kb_fd_conv_cell(v, lower, has_self, kn);
-    kb_fd_store(KB_FD_AT(dst, q * h + k, d, nd), v);
+    kb_store_p3_w128(KB_FD_AT(dst, q * h + k, d, nd), v);
 }
 
 // ---- Stage A for SMALL rounds: one cell on FOUR lanes -----------------------------------------------------------------
@@ -423,15 +408,15 @@ static __global__ void __launch_bounds__(KB_FD_CONV_THREADS) k_fd_conv_q4(size_t
         hq = hl;
     }
     ge_p3 v, lower;
-    if (k == 1) kb_fd_load(lower, KB_FD_AT(dec, q * h + (hq - sq), d, nd));
-    else kb_fd_load(lower, KB_FD_AT(src, q * h + k - 1, d, nd));
+    if (k == 1) kb_load_p3_w128(lower, KB_FD_AT(dec, q * h + (hq - sq), d, nd));
+    else kb_load_p3_w128(lower, KB_FD_AT(src, q * h + k - 1, d, nd));
     const bool has_self = k < sq;
-    if (has_self) kb_fd_load(v, KB_FD_AT(src, q * h + k, d, nd));
+    if (has_self) kb_load_p3_w128(v, KB_FD_AT(src, q * h + k, d, nd));
     else ge_identity(v);
     kb_naf kn;
     kb_naf_from(kn, (uint64_t)k);
     kb_q4_conv_cell(v, lower, has_self, kn);
-    if ((threadIdx.x & 3) == 0) kb_fd_store(KB_FD_AT(dst, q * h + k, d, nd), v);
+    if ((threadIdx.x & 3) == 0) kb_store_p3_w128(KB_FD_AT(dst, q * h + k, d, nd), v);
 }
 
 // Stage C.  Block = one (dealer, block q); thread = order k.  All n steps in one launch: per step every lane turns its
@@ -466,8 +451,8 @@ static __global__ void __launch_bounds__(MAXH, MINB) k_fd_steps(size_t nd, size_
     const unsigned nlive = (unsigned)((hq + 31) / 32);
     ge_p3 p;
     ge_identity(p);
-    if (k == 0) kb_fd_load(p, KB_FD_AT(dec, q * h, d, nd));
-    else if (k < hq) kb_fd_load(p, KB_FD_AT(diffs, q * h + k, d, nd));
+    if (k == 0) kb_load_p3_w128(p, KB_FD_AT(dec, q * h, d, nd));
+    else if (k < hq) kb_load_p3_w128(p, KB_FD_AT(diffs, q * h + k, d, nd));
     const bool top = k + 1 >= hq;   // nothing above: the operand is the identity
     // barrier ids: pair (w, w + 1) uses FULL = 1 + 2 w and EMPTY = 2 + 2 w  (<= 14 for 8 warps; 0 is __syncthreads)
     const unsigned full_up = 1 + 2 * warp, empty_up = 2 + 2 * warp;            // as the consumer of the warp above
@@ -481,13 +466,7 @@ static __global__ void __launch_bounds__(MAXH, MINB) k_fd_steps(size_t nd, size_
         ge_to_cached(c, p);
         if (warp > 0) {
             kb_bar_sync(empty_dn);   // the warp below has read the previous operand
-            if (lane == 0) {
-                uint32_t* o = xch + 32 * warp;
-                kb_store_fe(o, c.YpX);
-                kb_store_fe(o + 8, c.YmX);
-                kb_store_fe(o + 16, c.T2d);
-                kb_store_fe(o + 24, c.Z);
-            }
+            if (lane == 0) kb_store_cached_w128(xch + 32 * warp, c);
             __syncwarp();
             kb_bar_arrive(full_dn);
         }
@@ -503,13 +482,7 @@ static __global__ void __launch_bounds__(MAXH, MINB) k_fd_steps(size_t nd, size_
         const bool above_live = warp + 1 < nlive && 32u * (warp + 1) <= reach;
         if (above_live) {
             kb_bar_sync(full_up);
-            if (lane == 31) {
-                const uint32_t* o = xch + 32 * (warp + 1);
-                kb_load_fe(c.YpX, o);
-                kb_load_fe(c.YmX, o + 8);
-                kb_load_fe(c.T2d, o + 16);
-                kb_load_fe(c.Z, o + 24);
-            }
+            if (lane == 31) kb_load_cached_w128(c, xch + 32 * (warp + 1));
             __syncwarp();
             // the warp above only waits for this if it will produce again: at its next step it is live iff 32 (w+1) <= reach - 1
             if (32u * (warp + 1) + 1 <= reach) kb_bar_arrive(empty_up);
@@ -518,7 +491,7 @@ static __global__ void __launch_bounds__(MAXH, MINB) k_fd_steps(size_t nd, size_
         }
         if (top) ge_cached_identity(c);
         ge_add<true>(p, p, c);
-        if (k == 0) kb_fd_store(evals + ((q * n + i) * nd + d) * 32, p);
+        if (k == 0) kb_store_p3_w128(evals + ((q * n + i) * nd + d) * 32, p);
     }
 }
 
@@ -543,7 +516,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_fd_check(size_t nd, size_
     uint32_t pw9[9 * (KB_FD_MAX_PARTS - 1)];
     for (int w = 0; w < 9 * nt; w++) pw9[w] = pw[i * 9 * nt + w];
     ge_p3 v;
-    kb_fd_combine(v, nt, pw9, tbl, e, [&](int q, ge_p3& P) { kb_fd_load(P, evals + (((size_t)q * n + i) * nd + d) * 32); });
+    kb_fd_combine(v, nt, pw9, tbl, e, [&](int q, ge_p3& P) { kb_load_p3_w128(P, evals + (((size_t)q * n + i) * nd + d) * 32); });
     uint32_t s[8];
     int8_t es[64];
     kb_load32(s, shares, slot);
@@ -584,7 +557,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_fd_check_q4(size_t nd, si
     for (int q = 0; q < nt; q++) {
         uint32_t pw9[9];
         for (int w = 0; w < 9; w++) pw9[w] = pw[i * 9 * nt + 9 * q + w];
-        kb_fd_load(P, evals + (((size_t)(q + 1) * n + i) * nd + d) * 32);
+        kb_load_p3_w128(P, evals + (((size_t)(q + 1) * n + i) * nd + d) * 32);
         if (pw9[8]) {
             fe_neg(P.X, P.X);
             fe_neg(P.T, P.T);
@@ -616,7 +589,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_fd_check_q4(size_t nd, si
             }
         }
     }
-    kb_fd_load(P, evals + ((size_t)i * nd + d) * 32);
+    kb_load_p3_w128(P, evals + ((size_t)i * nd + d) * 32);
     ge_cached c0;
     ge_to_cached(c0, P);
     kb_q4_addsub(W, c0, false);

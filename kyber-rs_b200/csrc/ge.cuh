@@ -42,6 +42,107 @@ KB_FN void ge_precomp_identity(ge_precomp& c)
     fe_set(c.ymx, 1);
     fe_set(c.xy2d, 0);
 }
+
+// ---- the forms in which kernels hand points to each other through device memory, 8 little-endian words per coordinate:
+//   extended point  X, Y, Z, T          32 words
+//   cached operand  Y+X, Y-X, 2dT, Z    32 words
+//   affine entry    y+x, y-x, 2dxy      24 words (the MSM's points)
+// The suffix is the width of each access: _w32 moves single words (the host emulation compiles these), _w128 moves 16 bytes
+// at a time.  Each site keeps the width it has; switching one changes its kernel's code and would need a measurement.
+KB_FN void kb_store_p3_w32(uint32_t* o, const ge_p3& p)
+{
+    KB_UNROLL
+    for (int k = 0; k < 8; k++) {
+        o[k] = p.X.v[k];
+        o[8 + k] = p.Y.v[k];
+        o[16 + k] = p.Z.v[k];
+        o[24 + k] = p.T.v[k];
+    }
+}
+KB_FN void kb_load_p3_w32(ge_p3& p, const uint32_t* o)
+{
+    KB_UNROLL
+    for (int k = 0; k < 8; k++) {
+        p.X.v[k] = o[k];
+        p.Y.v[k] = o[8 + k];
+        p.Z.v[k] = o[16 + k];
+        p.T.v[k] = o[24 + k];
+    }
+}
+KB_FN void kb_store_precomp_w32(uint32_t* o, const ge_precomp& q)
+{
+    KB_UNROLL
+    for (int k = 0; k < 8; k++) {
+        o[k] = q.ypx.v[k];
+        o[8 + k] = q.ymx.v[k];
+        o[16 + k] = q.xy2d.v[k];
+    }
+}
+KB_FN void kb_load_precomp_w32(ge_precomp& q, const uint32_t* o)
+{
+    KB_UNROLL
+    for (int k = 0; k < 8; k++) {
+        q.ypx.v[k] = o[k];
+        q.ymx.v[k] = o[8 + k];
+        q.xy2d.v[k] = o[16 + k];
+    }
+}
+#if !defined(KB_HOST_EMU)
+__device__ __forceinline__ void kb_load_fe(fe& f, const uint32_t* p)
+{
+    const uint4* q = reinterpret_cast<const uint4*>(p);
+    uint4 a = q[0], b = q[1];
+    f.v[0] = a.x; f.v[1] = a.y; f.v[2] = a.z; f.v[3] = a.w;
+    f.v[4] = b.x; f.v[5] = b.y; f.v[6] = b.z; f.v[7] = b.w;
+}
+__device__ __forceinline__ void kb_store_fe(uint32_t* p, const fe& f)
+{
+    uint4* q = reinterpret_cast<uint4*>(p);
+    q[0] = make_uint4(f.v[0], f.v[1], f.v[2], f.v[3]);
+    q[1] = make_uint4(f.v[4], f.v[5], f.v[6], f.v[7]);
+}
+__device__ __forceinline__ void kb_store_p3_w128(uint32_t* o, const ge_p3& p)
+{
+    kb_store_fe(o, p.X);
+    kb_store_fe(o + 8, p.Y);
+    kb_store_fe(o + 16, p.Z);
+    kb_store_fe(o + 24, p.T);
+}
+__device__ __forceinline__ void kb_load_p3_w128(ge_p3& p, const uint32_t* o)
+{
+    kb_load_fe(p.X, o);
+    kb_load_fe(p.Y, o + 8);
+    kb_load_fe(p.Z, o + 16);
+    kb_load_fe(p.T, o + 24);
+}
+// the parts of an extended point that a reader needs, in the order it reads them
+__device__ __forceinline__ void kb_load_p3_xy_w128(fe& x, fe& y, const uint32_t* o)
+{
+    kb_load_fe(x, o);
+    kb_load_fe(y, o + 8);
+}
+__device__ __forceinline__ void kb_load_p3_z_w128(fe& z, const uint32_t* o) { kb_load_fe(z, o + 16); }
+__device__ __forceinline__ void kb_store_cached_w128(uint32_t* o, const ge_cached& c)
+{
+    kb_store_fe(o, c.YpX);
+    kb_store_fe(o + 8, c.YmX);
+    kb_store_fe(o + 16, c.T2d);
+    kb_store_fe(o + 24, c.Z);
+}
+__device__ __forceinline__ void kb_load_cached_w128(ge_cached& c, const uint32_t* o)
+{
+    kb_load_fe(c.YpX, o);
+    kb_load_fe(c.YmX, o + 8);
+    kb_load_fe(c.T2d, o + 16);
+    kb_load_fe(c.Z, o + 24);
+}
+__device__ __forceinline__ void kb_store_precomp_w128(uint32_t* o, const ge_precomp& q)
+{
+    kb_store_fe(o, q.ypx);
+    kb_store_fe(o + 8, q.ymx);
+    kb_store_fe(o + 16, q.xy2d);
+}
+#endif
 // ge.rs:99 write_cached
 KB_FN void ge_to_cached(ge_cached& r, const ge_p3& p)
 {

@@ -22,19 +22,6 @@ __device__ __forceinline__ void kb_store32(uint8_t* base, size_t i, const uint32
     p[0] = make_uint4(w[0], w[1], w[2], w[3]);
     p[1] = make_uint4(w[4], w[5], w[6], w[7]);
 }
-__device__ __forceinline__ void kb_load_fe(fe& f, const uint32_t* p)
-{
-    const uint4* q = reinterpret_cast<const uint4*>(p);
-    uint4 a = q[0], b = q[1];
-    f.v[0] = a.x; f.v[1] = a.y; f.v[2] = a.z; f.v[3] = a.w;
-    f.v[4] = b.x; f.v[5] = b.y; f.v[6] = b.z; f.v[7] = b.w;
-}
-__device__ __forceinline__ void kb_store_fe(uint32_t* p, const fe& f)
-{
-    uint4* q = reinterpret_cast<uint4*>(p);
-    q[0] = make_uint4(f.v[0], f.v[1], f.v[2], f.v[3]);
-    q[1] = make_uint4(f.v[4], f.v[5], f.v[6], f.v[7]);
-}
 // streaming (evict-first) variants for data that crosses HBM exactly once — the records between the two verify
 // launches — so that it does not push the per-thread tables out of L2
 __device__ __forceinline__ void kb_load_fe_cs(fe& f, const uint32_t* p)
@@ -109,6 +96,17 @@ __device__ __forceinline__ void kb_store_xyz(uint32_t* xyz, size_t i, const ge_p
     kb_store_fe(o + 8, p.Y);
     kb_store_fe(o + 16, p.Z);
 }
+__device__ __forceinline__ void kb_load_xyz_xy(fe& x, fe& y, const uint32_t* xyz, size_t i)
+{
+    kb_load_fe(x, xyz + 24 * i);
+    kb_load_fe(y, xyz + 24 * i + 8);
+}
+__device__ __forceinline__ void kb_load_xyz_z(fe& z, const uint32_t* xyz, size_t i) { kb_load_fe(z, xyz + 24 * i + 16); }
+__device__ __forceinline__ void kb_load_xyz(fe& x, fe& y, fe& z, const uint32_t* xyz, size_t i)
+{
+    kb_load_xyz_xy(x, y, xyz, i);
+    kb_load_xyz_z(z, xyz, i);
+}
 // calls emit(i, enc[8]) for every item of this thread's group, enc = canonical encoding
 template <typename F>
 __device__ __forceinline__ void kb_batch_compress(size_t n, const uint32_t* xyz, F emit)
@@ -118,11 +116,11 @@ __device__ __forceinline__ void kb_batch_compress(size_t n, const uint32_t* xyz,
     const int cnt = (n - base < KB_INV_K) ? (int)(n - base) : KB_INV_K;
     fe pref[KB_INV_K];
     fe acc, z;
-    kb_load_fe(acc, xyz + 24 * base + 16);
+    kb_load_xyz_z(acc, xyz, base);
     pref[0] = acc;
 #pragma unroll 1
     for (int k = 1; k < cnt; k++) {
-        kb_load_fe(z, xyz + 24 * (base + k) + 16);
+        kb_load_xyz_z(z, xyz, base + k);
         fe_mul(acc, acc, z);
         pref[k] = acc;
     }
@@ -133,14 +131,13 @@ __device__ __forceinline__ void kb_batch_compress(size_t n, const uint32_t* xyz,
         fe zinv;
         if (k > 0) {
             fe_mul(zinv, inv, pref[k - 1]);
-            kb_load_fe(z, xyz + 24 * (base + k) + 16);
+            kb_load_xyz_z(z, xyz, base + k);
             fe_mul(inv, inv, z);
         } else {
             zinv = inv;
         }
         ge_p3 p;
-        kb_load_fe(p.X, xyz + 24 * (base + k));
-        kb_load_fe(p.Y, xyz + 24 * (base + k) + 8);
+        kb_load_xyz_xy(p.X, p.Y, xyz, base + k);
         uint32_t enc[8];
         ge_compress_with_zinv(enc, p, zinv);
         emit(base + k, enc);
@@ -319,11 +316,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_point_decompress(size_t n
     ge_p3 p;
     const uint32_t ok = ge_decompress(p, w);
     if (!ok) ge_identity(p);
-    uint32_t* o = out128 + 32 * i;
-    kb_store_fe(o, p.X);
-    kb_store_fe(o + 8, p.Y);
-    kb_store_fe(o + 16, p.Z);
-    kb_store_fe(o + 24, p.T);
+    kb_store_p3_w128(out128 + 32 * i, p);
     if (status) status[i] = (uint8_t)(ok ^ 1u);
 }
 // 128-byte form -> (X, Y, Z) for the batch compressor; Z = 0 encodes as 32 zero bytes (fe_invert(0) = 0, ge.rs:112-122)
@@ -332,10 +325,8 @@ static __global__ void __launch_bounds__(KB_THREADS) k_points_from_raw(size_t n,
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     ge_p3 p;
-    const uint32_t* o = in128 + 32 * i;
-    kb_load_fe(p.X, o);
-    kb_load_fe(p.Y, o + 8);
-    kb_load_fe(p.Z, o + 16);
+    kb_load_p3_xy_w128(p.X, p.Y, in128 + 32 * i);
+    kb_load_p3_z_w128(p.Z, in128 + 32 * i);
     const uint32_t z0 = fe_is_zero(p.Z);
     if (z0) ge_identity(p);
     kb_store_xyz(xyz, i, p);
@@ -523,9 +514,97 @@ static __global__ void __launch_bounds__(KB_THREADS) k_verify_stage2(size_t n, c
 // verdict from a projective identity test (no inversion).  Two launches so that the two phases — which have
 // very different code (decompression / SHA-512 / Euclid vs. the doubling loop) and register needs — do not
 // compete for the instruction cache on one SM:
-//   k_verify_half_prep   checks, decompress A and R, h, (u, v), u*s mod L   -> 304-byte record per signature
+//   k_verify_half_prep   checks, decompress A and R, h, (u, v), u*s mod L   -> a record per signature
 //   k_verify_half_main   digit strings, two tables, the 33-window loop        -> status
+// The record of one signature, KB_HALF_REC_WORDS 32-bit words, written and read only through the accessors below.  It
+// crosses HBM exactly once, so its accesses are streaming (__stcs / __ldcs; the sort reads u and v through __ldg):
+//   words  0 .. 23   -A as affine X, Y, T             words 24 .. 47   -R as affine X, Y, T
+//   words 48 .. 71   u*s mod L, u, |v|
+//   word  72         flags | window count << 8 | sign(v) << 16 (the main kernel turns -A into A' = -sign(v) A)
+//   word  73         the "decodes" bits of the split preparation (bit 0: A, bit 1: R)
 #define KB_HALF_REC_WORDS 76
+__device__ __forceinline__ uint32_t* kb_rec_at(uint32_t* recs, size_t i) { return recs + KB_HALF_REC_WORDS * i; }
+__device__ __forceinline__ const uint32_t* kb_rec_at(const uint32_t* recs, size_t i) { return recs + KB_HALF_REC_WORDS * i; }
+// point part k: -A (k = 0) or -R (k = 1)
+__device__ __forceinline__ void kb_rec_store_point(uint32_t* o, int k, const fe& x, const fe& y, const fe& t)
+{
+    kb_store_fe_cs(o + 24 * k, x);
+    kb_store_fe_cs(o + 24 * k + 8, y);
+    kb_store_fe_cs(o + 24 * k + 16, t);
+}
+__device__ __forceinline__ void kb_rec_store_scalars(uint32_t* o, const kb_half_sc& sc)
+{
+    uint4* q = reinterpret_cast<uint4*>(o + 48);
+    __stcs(q + 0, make_uint4(sc.w[0], sc.w[1], sc.w[2], sc.w[3]));
+    __stcs(q + 1, make_uint4(sc.w[4], sc.w[5], sc.w[6], sc.w[7]));
+    __stcs(q + 2, make_uint4(sc.u[0], sc.u[1], sc.u[2], sc.u[3]));
+    __stcs(q + 3, make_uint4(sc.u[4], sc.u[5], sc.u[6], sc.u[7]));
+    __stcs(q + 4, make_uint4(sc.v[0], sc.v[1], sc.v[2], sc.v[3]));
+    __stcs(q + 5, make_uint4(sc.v[4], sc.v[5], sc.v[6], sc.v[7]));
+}
+__device__ __forceinline__ uint32_t kb_rec_pack72(uint32_t f, int nwin, uint32_t vneg) { return f | ((uint32_t)nwin << 8) | (vneg << 16); }
+__device__ __forceinline__ uint32_t kb_rec_flags72(uint32_t w72) { return w72 & 0xffu; }
+__device__ __forceinline__ uint32_t kb_rec_rest72(uint32_t w72) { return w72 & 0x1ff00u; }   // window count, sign(v) in place
+__device__ __forceinline__ void kb_rec_unpack72(uint32_t w72, uint32_t& f, int& nwin, uint32_t& vneg)
+{
+    f = kb_rec_flags72(w72);
+    nwin = (int)((w72 >> 8) & 0xffu);
+    vneg = (w72 >> 16) & 1u;
+}
+// word 72 alone: the split preparation's scalars kernel, which leaves word 73 to the points kernel
+__device__ __forceinline__ void kb_rec_store72(uint32_t* o, uint32_t w72) { __stcs(o + 72, w72); }
+__device__ __forceinline__ void kb_rec_store73(uint32_t* o, uint32_t dec) { __stcs(o + 73, dec); }
+// the last store of a preparation: word 72 in one 16-byte store that clears words 73 .. 75
+__device__ __forceinline__ void kb_rec_store72_clear73(uint32_t* o, uint32_t w72) { __stcs(reinterpret_cast<uint4*>(o + 72), make_uint4(w72, 0u, 0u, 0u)); }
+__device__ __forceinline__ void kb_rec_load72_73(const uint32_t* o, uint32_t& w72, uint32_t& dec)
+{
+    const uint4 a = __ldcs(reinterpret_cast<const uint4*>(o + 72));
+    w72 = a.x;
+    dec = a.y;
+}
+// what a signature off the fast path hands to the main kernel: operands (0, 1, 0) and scalars 0 (word 72 is the caller's)
+__device__ __forceinline__ void kb_rec_store_neutral(uint32_t* o)
+{
+    const uint4 z = make_uint4(0u, 0u, 0u, 0u), one = make_uint4(1u, 0u, 0u, 0u);
+    uint4* r = reinterpret_cast<uint4*>(o);
+    KB_UNROLL
+    for (int k = 0; k < 12; k++) __stcs(r + k, (k == 2 || k == 8) ? one : z);
+    uint4* q = reinterpret_cast<uint4*>(o + 48);
+    KB_UNROLL
+    for (int k = 0; k < 6; k++) __stcs(q + k, z);
+}
+// u and v, for the sort by loop length
+__device__ __forceinline__ void kb_rec_load_uv(uint32_t* u, uint32_t* v, const uint32_t* o)
+{
+    const uint4* q = reinterpret_cast<const uint4*>(o + 48);
+    uint4 a;
+    a = __ldg(q + 2); u[0] = a.x; u[1] = a.y; u[2] = a.z; u[3] = a.w;
+    a = __ldg(q + 3); u[4] = a.x; u[5] = a.y; u[6] = a.z; u[7] = a.w;
+    a = __ldg(q + 4); v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w;
+    a = __ldg(q + 5); v[4] = a.x; v[5] = a.y; v[6] = a.z; v[7] = a.w;
+}
+// the whole record, with A' = -sign(v) A in place of -A
+__device__ __forceinline__ void kb_rec_load(kb_half_rec& rec, const uint32_t* o)
+{
+    kb_load_fe_cs(rec.ax, o);
+    kb_load_fe_cs(rec.ay, o + 8);
+    kb_load_fe_cs(rec.at, o + 16);
+    kb_load_fe_cs(rec.rx, o + 24);
+    kb_load_fe_cs(rec.ry, o + 32);
+    kb_load_fe_cs(rec.rt, o + 40);
+    const uint4* q = reinterpret_cast<const uint4*>(o + 48);
+    uint4 a;
+    a = __ldcs(q + 0); rec.w[0] = a.x; rec.w[1] = a.y; rec.w[2] = a.z; rec.w[3] = a.w;
+    a = __ldcs(q + 1); rec.w[4] = a.x; rec.w[5] = a.y; rec.w[6] = a.z; rec.w[7] = a.w;
+    a = __ldcs(q + 2); rec.u[0] = a.x; rec.u[1] = a.y; rec.u[2] = a.z; rec.u[3] = a.w;
+    a = __ldcs(q + 3); rec.u[4] = a.x; rec.u[5] = a.y; rec.u[6] = a.z; rec.u[7] = a.w;
+    a = __ldcs(q + 4); rec.v[0] = a.x; rec.v[1] = a.y; rec.v[2] = a.z; rec.v[3] = a.w;
+    a = __ldcs(q + 5); rec.v[4] = a.x; rec.v[5] = a.y; rec.v[6] = a.z; rec.v[7] = a.w;
+    a = __ldcs(q + 6);
+    uint32_t vneg;
+    kb_rec_unpack72(a.x, rec.f, rec.nwin, vneg);
+    sig_half_apply_vneg(rec.ax, rec.at, vneg);
+}
 #ifndef KB_VERIFY_PREP_MINBLOCKS
 #define KB_VERIFY_PREP_MINBLOCKS 5
 #endif
@@ -569,7 +648,7 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_PREP_MINBLOCKS) k
     kb_load32(pw, pk, i);
     kb_load32(sw, sig, 2 * i);
     kb_load32(sw + 8, sig, 2 * i + 1);
-    uint32_t* o = recs + KB_HALF_REC_WORDS * i;
+    uint32_t* o = kb_rec_at(recs, i);
     uint32_t dec = 0, f = 0, vneg = 0;
     int nwin = 0;
     KB_NOUNROLL
@@ -586,42 +665,26 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_PREP_MINBLOCKS) k
 #endif
                 fe x, y, t;
                 dec |= sig_half_point(x, y, t, k ? sw : pw) << k;
-                kb_store_fe_cs(o + 24 * k, x);
-                kb_store_fe_cs(o + 24 * k + 8, y);
-                kb_store_fe_cs(o + 24 * k + 16, t);
+                kb_rec_store_point(o, k, x, y, t);
             }
         } else {
             // msg_off holds offsets into the caller's whole message array; `msg` points at byte msg_base of it
             const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
             kb_half_sc sc;
             sig_half_scalars<SCHNORR>(sc, pw, sw, msg + (lo - msg_base), hi - lo);
-            uint4* q = reinterpret_cast<uint4*>(o + 48);
-            __stcs(q + 0, make_uint4(sc.w[0], sc.w[1], sc.w[2], sc.w[3]));
-            __stcs(q + 1, make_uint4(sc.w[4], sc.w[5], sc.w[6], sc.w[7]));
-            __stcs(q + 2, make_uint4(sc.u[0], sc.u[1], sc.u[2], sc.u[3]));
-            __stcs(q + 3, make_uint4(sc.u[4], sc.u[5], sc.u[6], sc.u[7]));
-            __stcs(q + 4, make_uint4(sc.v[0], sc.v[1], sc.v[2], sc.v[3]));
-            __stcs(q + 5, make_uint4(sc.v[4], sc.v[5], sc.v[6], sc.v[7]));
+            kb_rec_store_scalars(o, sc);
             f = sc.f;
             vneg = sc.vneg;
             nwin = sc.nwin;
         }
     }
     f = sig_half_flags<SCHNORR>(f, dec);
-    uint4* q = reinterpret_cast<uint4*>(o + 48);
     if (!(f & KB_F_FAST)) {
-        // off the fast path (rare): neutral operands, no windows
-        const uint4 z = make_uint4(0u, 0u, 0u, 0u), one = make_uint4(1u, 0u, 0u, 0u);
-        uint4* r = reinterpret_cast<uint4*>(o);
-        KB_UNROLL
-        for (int k = 0; k < 12; k++) __stcs(r + k, (k == 2 || k == 8) ? one : z);
-        KB_UNROLL
-        for (int k = 0; k < 6; k++) __stcs(q + k, z);
+        kb_rec_store_neutral(o);   // off the fast path (rare): neutral operands, no windows
         nwin = 0;
         vneg = 0;
     }
-    // word 72: flags | window count << 8 | sign(v) << 16 (the main kernel turns -A into A' = -sign(v) A)
-    __stcs(q + 6, make_uint4(f | ((uint32_t)nwin << 8) | (vneg << 16), 0u, 0u, 0u));
+    kb_rec_store72_clear73(o, kb_rec_pack72(f, nwin, vneg));
 }
 // ---- the preparation as TWO kernels that share the SMs (KB_VERIFY_SPLIT=1, capi_verify.cu).  The phases of
 // k_verify_half_prep load different pipes and run one after the other in every block; here the "scalars" phase is a
@@ -635,7 +698,7 @@ static __global__ void __launch_bounds__(KB_THREADS, MINB) k_verify_half_points(
 {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) i = n - 1;   // tail threads redo the last item (same values, same address) so that they reach the barriers
-    uint32_t* o = recs + KB_HALF_REC_WORDS * i;
+    uint32_t* o = kb_rec_at(recs, i);
     uint32_t dec = 0;
     KB_NOUNROLL
     for (int k = 0; k < 2; k++) {
@@ -645,11 +708,9 @@ static __global__ void __launch_bounds__(KB_THREADS, MINB) k_verify_half_points(
         else kb_load32(w, pk, i);
         fe x, y, t;
         dec |= sig_half_point(x, y, t, w) << k;
-        kb_store_fe_cs(o + 24 * k, x);
-        kb_store_fe_cs(o + 24 * k + 8, y);
-        kb_store_fe_cs(o + 24 * k + 16, t);
+        kb_rec_store_point(o, k, x, y, t);
     }
-    __stcs(o + 73, dec);
+    kb_rec_store73(o, dec);
 }
 template <bool SCHNORR>
 static __global__ void __launch_bounds__(KB_THREADS, 4) k_verify_half_scalars(size_t n, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off, uint64_t msg_base, const uint8_t* sig, uint32_t* recs,
@@ -671,15 +732,9 @@ static __global__ void __launch_bounds__(KB_THREADS, 4) k_verify_half_scalars(si
         const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
         kb_half_sc sc;
         sig_half_scalars<SCHNORR>(sc, pw, sw, msg + (lo - msg_base), hi - lo);
-        uint32_t* o = recs + KB_HALF_REC_WORDS * i;
-        uint4* q = reinterpret_cast<uint4*>(o + 48);
-        __stcs(q + 0, make_uint4(sc.w[0], sc.w[1], sc.w[2], sc.w[3]));
-        __stcs(q + 1, make_uint4(sc.w[4], sc.w[5], sc.w[6], sc.w[7]));
-        __stcs(q + 2, make_uint4(sc.u[0], sc.u[1], sc.u[2], sc.u[3]));
-        __stcs(q + 3, make_uint4(sc.u[4], sc.u[5], sc.u[6], sc.u[7]));
-        __stcs(q + 4, make_uint4(sc.v[0], sc.v[1], sc.v[2], sc.v[3]));
-        __stcs(q + 5, make_uint4(sc.v[4], sc.v[5], sc.v[6], sc.v[7]));
-        __stcs(o + 72, sc.f | ((uint32_t)sc.nwin << 8) | (sc.vneg << 16));
+        uint32_t* o = kb_rec_at(recs, i);
+        kb_rec_store_scalars(o, sc);
+        kb_rec_store72(o, kb_rec_pack72(sc.f, sc.nwin, sc.vneg));
     }
 }
 template <bool SCHNORR>
@@ -687,22 +742,16 @@ static __global__ void __launch_bounds__(256) k_verify_half_fix(size_t n, uint32
 {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    uint32_t* o = recs + KB_HALF_REC_WORDS * i;
-    uint4* q = reinterpret_cast<uint4*>(o + 48);
-    const uint4 a = __ldcs(q + 6);
-    const uint32_t f = sig_half_flags<SCHNORR>(a.x & 0xffu, a.y);
-    uint32_t rest = a.x & 0x1ff00u;   // window count, sign(v)
+    uint32_t* o = kb_rec_at(recs, i);
+    uint32_t w72, dec;
+    kb_rec_load72_73(o, w72, dec);
+    const uint32_t f = sig_half_flags<SCHNORR>(kb_rec_flags72(w72), dec);
+    uint32_t rest = kb_rec_rest72(w72);
     if (!(f & KB_F_FAST)) {
-        // off the fast path (rare): neutral operands, no windows
-        const uint4 z = make_uint4(0u, 0u, 0u, 0u), one = make_uint4(1u, 0u, 0u, 0u);
-        uint4* r = reinterpret_cast<uint4*>(o);
-        KB_UNROLL
-        for (int k = 0; k < 12; k++) __stcs(r + k, (k == 2 || k == 8) ? one : z);
-        KB_UNROLL
-        for (int k = 0; k < 6; k++) __stcs(q + k, z);
+        kb_rec_store_neutral(o);   // off the fast path (rare): neutral operands, no windows
         rest = 0;
     }
-    __stcs(q + 6, make_uint4(f | rest, 0u, 0u, 0u));
+    kb_rec_store72_clear73(o, f | rest);
 }
 // ---- order of the records for the main kernel: a counting sort by the number of digit pairs each needs (the same
 // sc_joint4_pairs the main kernel takes its trip count from), longest first.  2^20 honest signatures need 60 .. 68
@@ -716,13 +765,8 @@ static __global__ void __launch_bounds__(256) k_half_sort_count(size_t n, const 
     __syncthreads();
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) {
-        const uint4* q = reinterpret_cast<const uint4*>(recs + KB_HALF_REC_WORDS * i + 48);
         uint32_t u[8], v[8];
-        uint4 a;
-        a = __ldg(q + 2); u[0] = a.x; u[1] = a.y; u[2] = a.z; u[3] = a.w;
-        a = __ldg(q + 3); u[4] = a.x; u[5] = a.y; u[6] = a.z; u[7] = a.w;
-        a = __ldg(q + 4); v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w;
-        a = __ldg(q + 5); v[4] = a.x; v[5] = a.y; v[6] = a.z; v[7] = a.w;
+        kb_rec_load_uv(u, v, kb_rec_at(recs, i));
         const int key = sc_joint4_pairs(u, v);   // 1 .. 128
         keys[i] = (uint8_t)key;
         atomicAdd(&s_hist[key], 1u);
@@ -783,27 +827,7 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k
     if (!live) i = n - 1;
     if (perm) i = perm[i];     // the order of k_half_sort_*: records of like loop length share a block
     kb_half_rec rec;
-    {
-        const uint32_t* o = recs + KB_HALF_REC_WORDS * i;
-        kb_load_fe_cs(rec.ax, o);
-        kb_load_fe_cs(rec.ay, o + 8);
-        kb_load_fe_cs(rec.at, o + 16);
-        kb_load_fe_cs(rec.rx, o + 24);
-        kb_load_fe_cs(rec.ry, o + 32);
-        kb_load_fe_cs(rec.rt, o + 40);
-        const uint4* q = reinterpret_cast<const uint4*>(o + 48);
-        uint4 a;
-        a = __ldcs(q + 0); rec.w[0] = a.x; rec.w[1] = a.y; rec.w[2] = a.z; rec.w[3] = a.w;
-        a = __ldcs(q + 1); rec.w[4] = a.x; rec.w[5] = a.y; rec.w[6] = a.z; rec.w[7] = a.w;
-        a = __ldcs(q + 2); rec.u[0] = a.x; rec.u[1] = a.y; rec.u[2] = a.z; rec.u[3] = a.w;
-        a = __ldcs(q + 3); rec.u[4] = a.x; rec.u[5] = a.y; rec.u[6] = a.z; rec.u[7] = a.w;
-        a = __ldcs(q + 4); rec.v[0] = a.x; rec.v[1] = a.y; rec.v[2] = a.z; rec.v[3] = a.w;
-        a = __ldcs(q + 5); rec.v[4] = a.x; rec.v[5] = a.y; rec.v[6] = a.z; rec.v[7] = a.w;
-        a = __ldcs(q + 6);
-        rec.f = a.x & 0xffu;
-        rec.nwin = (int)((a.x >> 8) & 0xffu);
-        sig_half_apply_vneg(rec.ax, rec.at, (a.x >> 16) & 1u);
-    }
+    kb_rec_load(rec, kb_rec_at(recs, i));
     kb_comb_digit dw[KB_COMB_POS];
 #if KB_HALF_JOINT
     ge_cached tbl[KB_JOINT_SLOTS];
@@ -847,11 +871,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_commit_prepare(size_t nco
     const uint32_t ok = ge_decompress(p, w);
     ge_cached c;
     ge_to_cached(c, p);
-    uint32_t* o = cached + 32 * i;
-    kb_store_fe(o, c.YpX);
-    kb_store_fe(o + 8, c.YmX);
-    kb_store_fe(o + 16, c.T2d);
-    kb_store_fe(o + 24, c.Z);
+    kb_store_cached_w128(cached + 32 * i, c);
     bad[i] = (uint8_t)(ok ^ 1u);
 }
 // the same from the reference's in-memory / serde form (40 limbs per point, ge.cuh kb_point_from_limbs_checked)
@@ -864,11 +884,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_commit_prepare_limbs(size
     if (!ok) ge_identity(p);
     ge_cached c;
     ge_to_cached(c, p);
-    uint32_t* o = cached + 32 * i;
-    kb_store_fe(o, c.YpX);
-    kb_store_fe(o + 8, c.YmX);
-    kb_store_fe(o + 16, c.T2d);
-    kb_store_fe(o + 24, c.Z);
+    kb_store_cached_w128(cached + 32 * i, c);
     bad[i] = (uint8_t)(ok ^ 1u);
 }
 // PriPoly::eval (share/poly.rs:133-141) for every (polynomial d, index i): out[d * n + i] = sum_j coeffs[d][j] (i+1)^j mod L
@@ -923,10 +939,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_poly_eval(size_t m, size_
     for (size_t j = t; j-- > 0;) {
         __syncthreads();   // keeps the block's warps on the same instructions (see KB_LOCKSTEP in ops.cuh)
         ge_cached c;
-        kb_load_fe(c.YpX, cp + 32 * j);
-        kb_load_fe(c.YmX, cp + 32 * j + 8);
-        kb_load_fe(c.T2d, cp + 32 * j + 16);
-        kb_load_fe(c.Z, cp + 32 * j + 24);
+        kb_load_cached_w128(c, cp + 32 * j);
         anybad |= bp[j];
         kb_horner_step(v, xn, c);
     }

@@ -85,13 +85,7 @@ KB_FN void kb_msm_prepare_body(size_t i, const uint32_t* pw, const uint32_t* sw,
         ge_precomp_identity(q);
         kb_atomic_add(bad, 1u);
     }
-    uint32_t* o = pts + 24 * i;
-    KB_UNROLL
-    for (int k = 0; k < 8; k++) {
-        o[k] = q.ypx.v[k];
-        o[8 + k] = q.ymx.v[k];
-        o[16 + k] = q.xy2d.v[k];
-    }
+    kb_store_precomp_w32(pts + 24 * i, q);
     uint32_t mag[8], neg;
     sc_effective(mag, neg, sw);
     KB_UNROLL
@@ -129,27 +123,6 @@ KB_FN void kb_msm_scatter_body(const kb_msm_plan& pl, size_t i, const uint32_t* 
     });
 }
 
-KB_FN void kb_store_p3(uint32_t* o, const ge_p3& p)
-{
-    KB_UNROLL
-    for (int k = 0; k < 8; k++) {
-        o[k] = p.X.v[k];
-        o[8 + k] = p.Y.v[k];
-        o[16 + k] = p.Z.v[k];
-        o[24 + k] = p.T.v[k];
-    }
-}
-KB_FN void kb_load_p3(ge_p3& p, const uint32_t* o)
-{
-    KB_UNROLL
-    for (int k = 0; k < 8; k++) {
-        p.X.v[k] = o[k];
-        p.Y.v[k] = o[8 + k];
-        p.Z.v[k] = o[16 + k];
-        p.T.v[k] = o[24 + k];
-    }
-}
-
 // ---- accum: thread t owns sorted entries [t*K, (t+1)*K)
 // flags[t]: bit0 = head partial valid, bit1 = tail partial valid
 // tailb[t]: the bucket of the tail partial (what k_msm_merge would otherwise have to search for)
@@ -176,15 +149,7 @@ KB_FN void kb_msm_accum_body(const kb_msm_plan& pl, size_t t, const uint32_t* of
     uint32_t fl = 0;
     uint32_t v = sorted[s];
     ge_precomp q;
-    {
-        const uint32_t* pp = pts + 24 * (size_t)(v >> 1);
-        KB_UNROLL
-        for (int j = 0; j < 8; j++) {
-            q.ypx.v[j] = pp[j];
-            q.ymx.v[j] = pp[8 + j];
-            q.xy2d.v[j] = pp[16 + j];
-        }
-    }
+    kb_load_precomp_w32(q, pts + 24 * (size_t)(v >> 1));
     for (uint32_t k = s; k < e; k++) {
         // fetch the NEXT entry's point before the ~900-instruction addition so the gather overlaps it.  (An additional
         // prefetch.global.L2 of the entry four ahead was measured SLOWER: 15.2 against 14.8 ms at 2^22.)
@@ -193,13 +158,7 @@ KB_FN void kb_msm_accum_body(const kb_msm_plan& pl, size_t t, const uint32_t* of
         uint32_t vn = v;
         if (k + 1 < e) {
             vn = sorted[k + 1];
-            const uint32_t* pn = pts + 24 * (size_t)(vn >> 1);
-            KB_UNROLL
-            for (int j = 0; j < 8; j++) {
-                qn.ypx.v[j] = pn[j];
-                qn.ymx.v[j] = pn[8 + j];
-                qn.xy2d.v[j] = pn[16 + j];
-            }
+            kb_load_precomp_w32(qn, pts + 24 * (size_t)(vn >> 1));
         } else {
             qn = q;
         }
@@ -213,14 +172,14 @@ KB_FN void kb_msm_accum_body(const kb_msm_plan& pl, size_t t, const uint32_t* of
             const bool starts_before = offsets[b] < s;
             const bool ends_after = bend > e;
             if (starts_before) {
-                kb_store_p3(heads + 32 * t, acc);
+                kb_store_p3_w32(heads + 32 * t, acc);
                 fl |= 1u;
             } else if (ends_after) {
-                kb_store_p3(tails + 32 * t, acc);
+                kb_store_p3_w32(tails + 32 * t, acc);
                 tailb[t] = b;
                 fl |= 2u;
             } else {
-                kb_store_p3(bucket_sum + 32 * (size_t)b, acc);
+                kb_store_p3_w32(bucket_sum + 32 * (size_t)b, acc);
             }
             ge_identity(acc);
             if (k + 1 < e) {
@@ -254,16 +213,16 @@ KB_FN void kb_msm_merge_body(const kb_msm_plan& pl, size_t t, size_t nthreads, c
     }
     if (mode == 1) return;
     ge_p3 acc, h;
-    kb_load_p3(acc, tails + 32 * t);
+    kb_load_p3_w32(acc, tails + 32 * t);
     for (size_t u = t + 1; u < u_end && u < nthreads; u++) {
         if (flags[u] & 1u) {
-            kb_load_p3(h, heads + 32 * u);
+            kb_load_p3_w32(h, heads + 32 * u);
             ge_cached hc;
             ge_to_cached(hc, h);
             ge_add<true>(acc, acc, hc);
         }
     }
-    kb_store_p3(bucket_sum + 32 * (size_t)b, acc);
+    kb_store_p3_w32(bucket_sum + 32 * (size_t)b, acc);
 }
 
 // ---- reduce: group g of window w covers buckets [g*gs, (g+1)*gs) (0-based, bucket k has weight k+1)
@@ -285,7 +244,7 @@ KB_FN void kb_msm_reduce_body(const kb_msm_plan& pl, size_t tid, uint32_t groups
         const uint32_t b = w * pl.half + k;
         if (offsets[b + 1] > offsets[b]) {
             ge_p3 p;
-            kb_load_p3(p, bucket_sum + 32 * (size_t)b);
+            kb_load_p3_w32(p, bucket_sum + 32 * (size_t)b);
             ge_cached pc;
             ge_to_cached(pc, p);
             ge_add<true>(run, run, pc);
@@ -294,8 +253,8 @@ KB_FN void kb_msm_reduce_body(const kb_msm_plan& pl, size_t tid, uint32_t groups
         ge_to_cached(rc, run);
         ge_add<true>(tot, tot, rc);
     }
-    kb_store_p3(part_run + 32 * tid, run);
-    kb_store_p3(part_tot + 32 * tid, tot);
+    kb_store_p3_w32(part_run + 32 * tid, run);
+    kb_store_p3_w32(part_tot + 32 * tid, tot);
 }
 // one thread's share of a window: groups [c0, c1) -> t1 = sum tot_g, t2 = sum g * run_g
 KB_FN void kb_msm_window_chunk(ge_p3& t1, ge_p3& t2, uint32_t c0, uint32_t c1, const uint32_t* run_w, const uint32_t* tot_w)
@@ -307,12 +266,12 @@ KB_FN void kb_msm_window_chunk(ge_p3& t1, ge_p3& t2, uint32_t c0, uint32_t c1, c
     for (uint32_t g = c1; g-- > c0;) {
         ge_p3 p;
         ge_cached pc;
-        kb_load_p3(p, run_w + 32 * (size_t)g);
+        kb_load_p3_w32(p, run_w + 32 * (size_t)g);
         ge_to_cached(pc, p);
         ge_add<true>(r, r, pc);
         ge_to_cached(pc, r);
         ge_add<true>(ws, ws, pc);     // ws = sum (g - c0 + 1) run_g
-        kb_load_p3(p, tot_w + 32 * (size_t)g);
+        kb_load_p3_w32(p, tot_w + 32 * (size_t)g);
         ge_to_cached(pc, p);
         ge_add<true>(t1, t1, pc);
     }
@@ -364,7 +323,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_msm_prepare_ext(kb_msm_pl
     fe_set(acc, 1);
 #pragma unroll 1
     for (int k = 0; k < cnt; k++) {
-        kb_load_fe(z, points128 + 32 * (base + k) + 16);
+        kb_load_p3_z_w128(z, points128 + 32 * (base + k));
         const uint32_t z0 = fe_is_zero(z);
         zbad |= z0 << k;
         fe_cmov(z, one, z0);
@@ -378,7 +337,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_msm_prepare_ext(kb_msm_pl
     for (int k = cnt - 1; k >= 0; k--) {
         const size_t i = base + k;
         fe zinv;
-        kb_load_fe(z, points128 + 32 * i + 16);
+        kb_load_p3_z_w128(z, points128 + 32 * i);
         fe_cmov(z, one, (zbad >> k) & 1u);
         if (k > 0) {
             fe_mul(zinv, inv, pref[k - 1]);
@@ -387,8 +346,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_msm_prepare_ext(kb_msm_pl
             zinv = inv;
         }
         fe x, y, xx, yy, l, r;
-        kb_load_fe(x, points128 + 32 * i);
-        kb_load_fe(y, points128 + 32 * i + 8);
+        kb_load_p3_xy_w128(x, y, points128 + 32 * i);
         fe_mul(x, x, zinv);
         fe_mul(y, y, zinv);
         // on the curve:  -x^2 + y^2 = 1 + d x^2 y^2
@@ -409,10 +367,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_msm_prepare_ext(kb_msm_pl
             ge_precomp_identity(q);
             atomicAdd(bad, 1u);
         }
-        uint32_t* o = pts + 24 * i;
-        kb_store_fe(o, q.ypx);
-        kb_store_fe(o + 8, q.ymx);
-        kb_store_fe(o + 16, q.xy2d);
+        kb_store_precomp_w128(pts + 24 * i, q);
         uint32_t sw[8], mag[8], neg;
         kb_load32(sw, scalars, i);
         sc_effective(mag, neg, sw);
@@ -585,7 +540,7 @@ static __global__ void __launch_bounds__(KB_MSM_LONG_THREADS) k_msm_merge_long(s
         for (size_t u = t + 1 + threadIdx.x; u < u_end; u += KB_MSM_LONG_THREADS) {
             if (flags[u] & 1u) {
                 ge_p3 h;
-                kb_load_p3(h, heads + 32 * u);
+                kb_load_p3_w32(h, heads + 32 * u);
                 ge_cached hc;
                 ge_to_cached(hc, h);
                 ge_add<true>(s, s, hc);
@@ -593,19 +548,19 @@ static __global__ void __launch_bounds__(KB_MSM_LONG_THREADS) k_msm_merge_long(s
         }
         kb_warp_sum_point(s);
         __syncthreads();   // the previous entry's readers are done with wsum
-        if (lane == 0) kb_store_p3(wsum + 32 * warp, s);
+        if (lane == 0) kb_store_p3_w32(wsum + 32 * warp, s);
         __syncthreads();
         if (warp == 0) {
             ge_identity(s);
-            if (lane < KB_MSM_LONG_THREADS / 32) kb_load_p3(s, wsum + 32 * lane);
+            if (lane < KB_MSM_LONG_THREADS / 32) kb_load_p3_w32(s, wsum + 32 * lane);
             kb_warp_sum_point(s);
             if (lane == 0) {
                 ge_p3 tl;
-                kb_load_p3(tl, tails + 32 * t);
+                kb_load_p3_w32(tl, tails + 32 * t);
                 ge_cached tc;
                 ge_to_cached(tc, tl);
                 ge_add<true>(s, s, tc);
-                kb_store_p3(bucket_sum + 32 * (size_t)b, s);
+                kb_store_p3_w32(bucket_sum + 32 * (size_t)b, s);
             }
         }
     }
@@ -625,8 +580,8 @@ static __global__ void __launch_bounds__(256) k_msm_window_sums(kb_msm_plan pl, 
     kb_msm_window_chunk(t1, t2, c0, c1, part_run + 32 * (size_t)w * groups, part_tot + 32 * (size_t)w * groups);
     kb_warp_sum_point2(t1, t2);
     if (lane == 0) {
-        kb_store_p3(wtot + 32 * warp, t1);
-        kb_store_p3(wtot + 32 * (8 + warp), t2);
+        kb_store_p3_w32(wtot + 32 * warp, t1);
+        kb_store_p3_w32(wtot + 32 * (8 + warp), t2);
     }
     __syncthreads();
     if (warp == 0) {
@@ -634,8 +589,8 @@ static __global__ void __launch_bounds__(256) k_msm_window_sums(kb_msm_plan pl, 
         ge_identity(a);
         ge_identity(b);
         if (lane < 8) {
-            kb_load_p3(a, wtot + 32 * lane);
-            kb_load_p3(b, wtot + 32 * (8 + lane));
+            kb_load_p3_w32(a, wtot + 32 * lane);
+            kb_load_p3_w32(b, wtot + 32 * (8 + lane));
         }
         kb_warp_sum_point2(a, b);
         if (lane == 0) {
@@ -643,7 +598,7 @@ static __global__ void __launch_bounds__(256) k_msm_window_sums(kb_msm_plan pl, 
             ge_cached ac;
             ge_to_cached(ac, a);
             kb_horner_step(b, (uint64_t)gs, ac);   // b = gs * b + a
-            kb_store_p3(win_sum + 32 * w, b);
+            kb_store_p3_w32(win_sum + 32 * w, b);
         }
     }
 }
@@ -698,21 +653,21 @@ static __global__ void k_msm_finish(kb_msm_plan pl, const uint32_t* win_sum, uin
     for (uint32_t w = pl.windows; w-- > 0;) {
         for (uint32_t k = 0; k < pl.c; k++) kb_dbl_quad(tot);
         ge_p3 s;
-        kb_load_p3(s, win_sum + 32 * w);
+        kb_load_p3_w32(s, win_sum + 32 * w);
         ge_cached sc;
         ge_to_cached(sc, s);
         ge_add<true>(tot, tot, sc);
     }
     if (!first_chunk) {
         ge_p3 prev;
-        kb_load_p3(prev, acc128);
+        kb_load_p3_w32(prev, acc128);
         ge_cached pc;
         ge_to_cached(pc, prev);
         ge_add<true>(tot, tot, pc);
     }
     __syncwarp();
     if (threadIdx.x != 0) return;
-    kb_store_p3(acc128, tot);
+    kb_store_p3_w32(acc128, tot);
     if (out32) {
         uint32_t o[8];
         ge_compress(o, tot);
@@ -728,7 +683,7 @@ static __global__ void k_point_sum(size_t k, const uint32_t* partials, uint8_t* 
     ge_identity(s);
     for (size_t g = lane; g < k; g += 32) {
         ge_p3 p;
-        kb_load_p3(p, partials + 32 * g);
+        kb_load_p3_w32(p, partials + 32 * g);
         ge_cached pc;
         ge_to_cached(pc, p);
         ge_add<true>(s, s, pc);
@@ -753,12 +708,8 @@ static __global__ void __launch_bounds__(KB_THREADS) k_poly_colsum(size_t npoly,
     ge_identity(s);
     uint32_t anybad = 0;
     for (size_t d = lane; d < npoly; d += 32) {
-        const uint32_t* cp = cached + 32 * (d * t + j);
         ge_cached c;
-        kb_load_fe(c.YpX, cp);
-        kb_load_fe(c.YmX, cp + 8);
-        kb_load_fe(c.T2d, cp + 16);
-        kb_load_fe(c.Z, cp + 24);
+        kb_load_cached_w128(c, cached + 32 * (d * t + j));
         anybad |= bad[d * t + j];
         ge_add<true>(s, s, c);
     }

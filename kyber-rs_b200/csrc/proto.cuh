@@ -84,9 +84,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_find_pub(size_t nlist, co
 __device__ __forceinline__ void kb_load_xyz_ext(ge_p3& p, const uint32_t* xyz, size_t i)
 {
     fe x, y, z;
-    kb_load_fe(x, xyz + 24 * i);
-    kb_load_fe(y, xyz + 24 * i + 8);
-    kb_load_fe(z, xyz + 24 * i + 16);
+    kb_load_xyz(x, y, z, xyz, i);
     fe_mul(p.X, x, z);
     fe_mul(p.Y, y, z);
     fe_sq(p.Z, z);
@@ -133,9 +131,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_rabin_finish(size_t m, co
     ge_cached c;
     ge_to_cached(c, gh);
     ge_add<true>(fb, fb, c);
-    kb_load_fe(v.X, xyz + 24 * k);
-    kb_load_fe(v.Y, xyz + 24 * k + 8);
-    kb_load_fe(v.Z, xyz + 24 * k + 16);
+    kb_load_xyz(v.X, v.Y, v.Z, xyz, k);
     const uint32_t same = kb_proj_equal(v, fb);
     if (live) verdict[k] = (uint8_t)(same & h_ok & (bad[k] ? 0u : 1u));
 }
@@ -280,7 +276,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_wmul(size_t ncols, size_t
     ge_scalarmult<false>(h, e, tbl);
     if (!ok) ge_identity(h);
     if (!live) return;
-    kb_store_p3(out128 + 32 * (c * k + i), h);
+    kb_store_p3_w32(out128 + 32 * (c * k + i), h);
     bad[c * k + i] = (uint8_t)(ok ^ 1u);
 }
 // xyz[c] = sum_i in128[c * k + i]; status[c] = 1 if any of them was flagged.  One warp per column.
@@ -294,7 +290,7 @@ static __global__ void __launch_bounds__(KB_THREADS) k_colsum(size_t ncols, size
     uint32_t anybad = 0;
     for (size_t i = lane; i < k; i += 32) {
         ge_p3 p;
-        kb_load_p3(p, in128 + 32 * (c * k + i));
+        kb_load_p3_w32(p, in128 + 32 * (c * k + i));
         ge_cached pc;
         ge_to_cached(pc, p);
         ge_add<true>(s, s, pc);
