@@ -153,6 +153,30 @@ int kb_eddsa_verify_batch(kb_ctx* ctx, size_t n, const uint8_t* pk, const uint8_
 /* schnorr::verify_with_checks (sign/schnorr/schnorr_sig.rs:53-110) */
 int kb_schnorr_verify_batch(kb_ctx* ctx, size_t n, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off, const uint8_t* sig, uint8_t* status);
 
+/* ---- key sets: verification under registered public keys ---------------------------------------------------- */
+/* The signers of a DKG round, of DSS partial signatures or of a validator set are a small, fixed set of keys.  A key set
+ * holds, per key, a comb over A from which h*A takes 32 table additions instead of a doubling loop, and every verify
+ * call returns exactly what the general verifiers return for (keys[key_idx[i]], message i, sig[i]). */
+typedef struct kb_keyset kb_keyset;
+/* Registers nkeys public keys (32-byte encodings, exactly the bytes the verifiers would get as pk) with ctx.
+ * Each key is checked once (Point::is_canonical incl. the §A1 quirk, has_small_order on bytes, decodes), and for
+ * each key that passes, a comb kt[p][j] = (j+1)·2^(8p)·A, p = 0..31, j = 0..127, is built on the device
+ * (affine (y+x, y-x, 2dxy), 96 B per entry: 384 KiB per key, in an allocation of the key set, not in scratch).
+ * Keys that fail a check are accepted. Their signatures get the status the reference gives them.
+ * KB_ERR_ARG for nkeys == 0 or a NULL pointer, KB_ERR_NOMEM if the tables do not fit.  A key set belongs to
+ * its context (same device, errors in kb_last_error(ctx)) and must be destroyed before that context. */
+int  kb_keyset_create(kb_ctx* ctx, size_t nkeys, const uint8_t* pk, kb_keyset** out);
+void kb_keyset_destroy(kb_keyset* ks);
+/* status[i] = what kb_eddsa_verify_batch (schnorr == 0) / kb_schnorr_verify_batch (schnorr != 0) returns for
+ * (pk = keys[key_idx[i]], message i, sig[i]): same statuses and same check order.  msg / msg_off as in
+ * kb_eddsa_verify_batch.  KB_ERR_ARG if any key_idx[i] >= nkeys (checked before anything is launched). */
+int  kb_keyset_verify_batch(kb_keyset* ks, size_t n, const uint32_t* key_idx, const uint8_t* msg, const uint64_t* msg_off,
+                            const uint8_t* sig, uint8_t* status, int schnorr);
+/* device buffers + stream, ordered like every kb_dev_* call of the context.  An index >= nkeys gives status 0xFF
+ * for that item, and the kernel reads nothing of the key set for it. */
+int  kb_dev_keyset_verify(kb_keyset* ks, size_t n, const void* d_key_idx, const void* d_msg, const void* d_msg_off,
+                          const void* d_sig, void* d_status, int schnorr, void* stream);
+
 /* EdDSA::sign (sign/eddsa/eddsa_sig.rs:120-152) for n (seed, message) pairs, with the key derivation of
  * Curve::new_key_and_seed_with_input (group/edwards25519/curve.rs:74-87): a = clamp(SHA-512(seed)[0..32]),
  * prefix = SHA-512(seed)[32..64], r = SHA-512(prefix || M) mod L, R = r*B, A = a*B, h = SHA-512(R || A || M) mod L,

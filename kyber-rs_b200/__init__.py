@@ -12,6 +12,7 @@ layout the project asks for); use ``importlib.import_module("kyber-rs_b200")`` o
 """
 from .binding import (  # noqa: F401
     Context,
+    KeySet,
     MultiContext,
     KBError,
     LIB_PATH,
@@ -23,4 +24,4 @@ from .binding import (  # noqa: F401
 from . import host  # noqa: F401
 from . import sharding  # noqa: F401
 
-__all__ = ["Context", "MultiContext", "KBError", "LIB_PATH", "SIG_STATUS_NAMES", "FLAG_VARTIME", "FLAG_SHARED_POINT", "load_library", "host", "sharding"]
+__all__ = ["Context", "KeySet", "MultiContext", "KBError", "LIB_PATH", "SIG_STATUS_NAMES", "FLAG_VARTIME", "FLAG_SHARED_POINT", "load_library", "host", "sharding"]

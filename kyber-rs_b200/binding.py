@@ -44,6 +44,7 @@ EXPORTS = [
     "kb_mctx_dkg_verify_round", "kb_mctx_dkg_process_round", "kb_mctx_msm",
     "kb_dev_eddsa_verify", "kb_dev_point_mul_base", "kb_dev_point_mul", "kb_dev_msm", "kb_dev_msm_ext", "kb_dev_dkg_verify_round", "kb_dev_dkg_verify_round_limbs", "kb_dev_point_sum",
     "kb_probe_imad", "kb_verify_kernel_times",
+    "kb_keyset_create", "kb_keyset_destroy", "kb_keyset_verify_batch", "kb_dev_keyset_verify",
 ]
 
 
@@ -131,6 +132,11 @@ def load_library(path: str = LIB_PATH):
     L.kb_mctx_msm.argtypes = [vp, sz, vp, vp, vp, vp]
     L.kb_probe_imad.argtypes = [vp, i32, i32, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
     L.kb_verify_kernel_times.argtypes = [vp, i32, ctypes.POINTER(ctypes.c_float)]
+    L.kb_keyset_create.argtypes = [vp, sz, vp, ctypes.POINTER(vp)]
+    L.kb_keyset_destroy.argtypes = [vp]
+    L.kb_keyset_destroy.restype = None
+    L.kb_keyset_verify_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32]
+    L.kb_dev_keyset_verify.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32, vp]
     _LIB = L
     return L
 
@@ -524,6 +530,10 @@ class Context:
         self._check(self.L.kb_verify_kernel_times(self.h, 1, ms), "kb_verify_kernel_times")
         return float(ms[0]), float(ms[1])
 
+    def keyset(self, pk):
+        """Registers the public keys pk (nkeys x 32 encodings) for verification by key index (KeySet)."""
+        return KeySet(self, pk)
+
     # ---- device-pointer API (torch CUDA tensors; enqueues on torch's current stream) --------
     @staticmethod
     def _dp(t):
@@ -573,6 +583,49 @@ class Context:
 
     def dev_point_sum(self, k, partials, out32):
         self._check(self.L.kb_dev_point_sum(self.h, k, self._dp(partials), self._dp(out32), self._stream()), "kb_dev_point_sum")
+
+
+class KeySet:
+    """One kb_keyset: public keys registered with a Context, each with its comb on the device (384 KiB per key).
+    Signatures then name their key by index; the statuses are those of Context.verify_batch with pk = keys[key_idx]."""
+
+    def __init__(self, ctx: Context, pk):
+        self.ctx = ctx   # the key set belongs to its context and must go before it
+        self.L = ctx.L
+        self.h = None
+        p = _u8(pk, (-1, 32))
+        self.nkeys = p.shape[0]
+        h = ctypes.c_void_p()
+        ctx._check(self.L.kb_keyset_create(ctx.h, self.nkeys, _ptr(p), ctypes.byref(h)), "kb_keyset_create")
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.kb_keyset_destroy(self.h)
+            self.h = None
+
+    def __del__(self):  # pragma: no cover
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def verify_batch(self, key_idx, msg, msg_off, sig, schnorr=False, out=None):
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        sig = _u8(sig, (-1, 64))
+        msg = _u8(msg)
+        msg_off = np.ascontiguousarray(msg_off, dtype=np.uint64)
+        n = key_idx.shape[0]
+        if sig.shape[0] != n or msg_off.shape[0] != n + 1:
+            raise ValueError("KeySet.verify_batch: one key index and one signature per item, n+1 message offsets")
+        st = out if out is not None else np.empty(n, dtype=np.uint8)
+        self.ctx._check(self.L.kb_keyset_verify_batch(self.h, n, _ptr(key_idx), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(st), int(schnorr)), "kb_keyset_verify_batch")
+        return st
+
+    def dev_verify(self, n, key_idx, msg, msg_off, sig, status, schnorr=False):
+        """key_idx: n uint32 (torch int32 tensor), the rest as Context.dev_verify; an index outside the set gives status 0xFF."""
+        dp = Context._dp
+        self.ctx._check(self.L.kb_dev_keyset_verify(self.h, n, dp(key_idx), dp(msg), dp(msg_off), dp(sig), dp(status), int(schnorr), Context._stream()), "kb_dev_keyset_verify")
 
 
 class MultiContext:

@@ -46,7 +46,7 @@ __device__ __forceinline__ void kb_stage(uint32_t* dst, const uint32_t* src, int
     __syncthreads();
 }
 
-// Kernel groups: a translation unit defines KB_K_POINT / KB_K_SIGN / KB_K_POLY / KB_K_MSM for the non-template kernels it
+// Kernel groups: a translation unit defines KB_K_POINT / KB_K_SIGN / KB_K_POLY / KB_K_MSM / KB_K_KEYSET for the non-template kernels it
 // launches (nvcc compiles every __global__ function it sees, used or not).
 #if defined(KB_K_POINT)
 // ---- base-point table: table[w*8 + j] = (j+1) * 16^w * B, w = 0..63 (replaces constants.rs:89 BASE)
@@ -509,6 +509,56 @@ static __global__ void __launch_bounds__(KB_THREADS) k_verify_stage2(size_t n, c
         status[i] = (uint8_t)sig_finish<SCHNORR>(flags[i], enc, rw);
     });
 }
+
+#if defined(KB_K_KEYSET)
+// ---- key sets (ops.cuh kb_key_*, sig_keyset_stage1): verification under registered public keys.  A key set holds, per key,
+// its 32-byte encoding, one byte of facts (kb_key_facts) and its comb of KB_KEY_ENTRIES affine entries.
+// One thread per (key, comb position).
+static __global__ void __launch_bounds__(KB_THREADS) k_keyset_build(size_t nkeys, const uint8_t* pk, uint8_t* facts, ge_precomp* ktab)
+{
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nkeys * KB_KEY_POS) return;
+    const size_t k = t / KB_KEY_POS;
+    const int p = (int)(t % KB_KEY_POS);
+    uint32_t pw[8];
+    kb_load32(pw, pk, k);
+    ge_p3 A;
+    const uint32_t f = kb_key_facts(A, pw);
+    if (p == 0) facts[k] = (uint8_t)f;
+    kb_key_row(ktab + k * KB_KEY_ENTRIES + (size_t)p * KB_KEY_HALF, A, p);
+}
+// sig_stage1 of signature i under key key_idx[i]: (X, Y, Z) and the flag byte in the layout of k_verify_stage1, for
+// k_verify_stage2.  An index outside the key set reads nothing of it; the item is off the fast path and
+// k_keyset_bad_index overwrites its status.
+template <bool SCHNORR>
+static __global__ void __launch_bounds__(KB_THREADS) k_keyset_verify(size_t n, const uint32_t* key_idx, size_t nkeys, const uint8_t* kpk, const uint8_t* facts, const ge_precomp* ktab,
+                                                                     const uint8_t* msg, const uint64_t* msg_off, const uint8_t* sig, const ge_precomp* comb, uint32_t* xyz, uint8_t* flags)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t k = __ldg(key_idx + i);
+    uint32_t pw[8] = {0, 0, 0, 0, 0, 0, 0, 0}, sw[16], kf = 0;
+    const ge_precomp* kt = nullptr;
+    if (k < nkeys) {
+        kb_load32(pw, kpk, k);
+        kf = __ldg(facts + k);
+        kt = ktab + (size_t)k * KB_KEY_ENTRIES;
+    }
+    kb_load32(sw, sig, 2 * i);
+    kb_load32(sw + 8, sig, 2 * i + 1);
+    const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
+    ge_p3 Q;
+    const uint32_t f = sig_keyset_stage1<SCHNORR>(Q, kf, pw, sw, msg + lo, hi - lo, comb, kt);
+    kb_store_xyz(xyz, i, Q);
+    flags[i] = (uint8_t)f;
+}
+// status 0xFF for every item whose key index is outside the key set (runs after k_verify_stage2)
+static __global__ void __launch_bounds__(256) k_keyset_bad_index(size_t n, const uint32_t* key_idx, size_t nkeys, uint8_t* status)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && __ldg(key_idx + i) >= nkeys) status[i] = 0xFF;
+}
+#endif  // KB_K_KEYSET
 
 // ---- the same verifiers with half-size scalars (ops.cuh sig_half_*, half.cuh): 128 doublings per signature,
 // verdict from a projective identity test (no inversion).  Two launches so that the two phases — which have

@@ -901,3 +901,163 @@ KB_FN void kb_base_window(ge_precomp* win, const ge_p3& pos, int count = 8)
         ge_add<true>(m, m, pc);
     }
 }
+
+// ---------------------------------------------------------------------------------------
+// key sets: verification under registered public keys (kb_keyset_*, capi_keyset.cu)
+// ---------------------------------------------------------------------------------------
+// When A is known in advance, h*A needs no doublings: a comb over A, kt[p][j] = (j+1) * 2^(KB_KEY_BITS p) * A, gives it in
+// KB_KEY_POS mixed additions, and s*B comes from the context's comb in KB_COMB_POS more.  Q = s*B - h*A is then exactly
+// what sig_stage1 computes, and k_verify_stage2 decides compress(Q) == R bytes as for the full-length verifiers.
+// The multipliers are exact integers (never reduced mod L): a key with a small-order component has order 8L, and the
+// reference's h*A with h < L must stay exact for it.
+#define KB_KEY_BITS 8
+#define KB_KEY_POS 32
+#define KB_KEY_HALF (1 << (KB_KEY_BITS - 1))            // entries per position: (j+1) for j < KB_KEY_HALF
+#define KB_KEY_ENTRIES (KB_KEY_POS * KB_KEY_HALF)       // 4096 affine entries of 96 bytes: 384 KiB per key
+#define KB_KEY_INV 8                                    // comb entries made affine with one shared inversion
+static_assert(KB_KEY_BITS * KB_KEY_POS >= 254 && KB_KEY_BITS <= 8, "the key comb must cover 253 bits and the recoding carry; digits are int8");
+static_assert(KB_KEY_HALF % KB_KEY_INV == 0, "a position is made affine in whole groups");
+
+// The facts about a key that sig_stage1 derives from its bytes: KB_F_AC (is_canonical), KB_F_AS (small order on bytes),
+// KB_F_AOK (decodes), the last one raw — sig_keyset_flags decides per signature whether the reference reaches the decode.
+// A = the decoded point for a key that can be on the fast path, the identity otherwise (its comb is never read).
+KB_FN uint32_t kb_key_facts(ge_p3& A, const uint32_t* pk_w)
+{
+    uint32_t f = 0;
+    f |= pt_is_canonical(pk_w) ? KB_F_AC : 0u;
+    f |= pt_is_small_order_bytes(pk_w) ? KB_F_AS : 0u;
+    f |= ge_decompress(A, pk_w) ? KB_F_AOK : 0u;
+    if ((f & (KB_F_AC | KB_F_AS | KB_F_AOK)) != (KB_F_AC | KB_F_AOK)) ge_identity(A);
+    return f;
+}
+// Position p of the key comb: row[j] = (j+1) * 2^(KB_KEY_BITS p) * A in affine (y+x, y-x, 2dxy) form, j < KB_KEY_HALF, built
+// by doublings and additions of A itself.  Each group of KB_KEY_INV entries is first stored projectively in place (X, Y, Z
+// in the three fields) and then made affine with ONE inversion (Montgomery's trick, as kb_batch_compress does).
+KB_FN void kb_key_row(ge_precomp* row, const ge_p3& A, int p)
+{
+    const fe d2 = KB_FE_D2;
+    ge_p3 m = A;
+    const int ndbl = KB_KEY_BITS * p;
+    KB_NOUNROLL
+    for (int k = 0; k < ndbl; k++) ge_dbl_rt(m, m, k == ndbl - 1);
+    ge_cached pc;
+    ge_to_cached(pc, m);
+    KB_NOUNROLL
+    for (int g = 0; g < KB_KEY_HALF; g += KB_KEY_INV) {
+        fe pref[KB_KEY_INV];
+        fe acc;
+        KB_NOUNROLL
+        for (int k = 0; k < KB_KEY_INV; k++) {
+            if (g + k > 0) ge_add<true>(m, m, pc);   // m = (g + k + 1) * 2^(KB_KEY_BITS p) * A
+            row[g + k].ypx = m.X;
+            row[g + k].ymx = m.Y;
+            row[g + k].xy2d = m.Z;
+            if (k == 0) acc = m.Z;
+            else fe_mul(acc, acc, m.Z);
+            pref[k] = acc;
+        }
+        fe inv;
+        fe_invert(inv, acc);
+        KB_NOUNROLL
+        for (int k = KB_KEY_INV - 1; k >= 0; k--) {
+            ge_precomp& e = row[g + k];
+            fe zinv, x, y, xy;
+            if (k > 0) {
+                fe_mul(zinv, inv, pref[k - 1]);
+                fe_mul(inv, inv, e.xy2d);
+            } else {
+                zinv = inv;
+            }
+            fe_mul(x, e.ypx, zinv);
+            fe_mul(y, e.ymx, zinv);
+            fe_add(e.ypx, y, x);
+            fe_sub(e.ymx, y, x);
+            fe_mul(xy, x, y);
+            fe_mul(e.xy2d, xy, d2);
+        }
+    }
+}
+// NEGATED signed radix-2^KB_KEY_BITS digits of a scalar < 2^253: nd[p] = -d[p] with d[p] in (-KB_KEY_HALF, KB_KEY_HALF], so
+// that sum nd[p] 2^(KB_KEY_BITS p) = -h and every nd[p] fits an int8
+KB_FN void sc_recode_key_neg(int8_t* nd, const uint32_t* s)
+{
+    int carry = 0;
+    KB_UNROLL
+    for (int p = 0; p < KB_KEY_POS; p++) {
+        const int bit = KB_KEY_BITS * p, wi = bit >> 5, sh = bit & 31;
+        uint32_t x = s[wi] >> sh;
+        if (sh + KB_KEY_BITS > 32 && wi + 1 < 8) x |= s[wi + 1] << (32 - sh);
+        const int v = (int)(x & ((1u << KB_KEY_BITS) - 1u)) + carry;
+        carry = v > KB_KEY_HALF;
+        nd[p] = (int8_t)((carry << KB_KEY_BITS) - v);
+    }
+}
+// operand of one addition: d * entry, d != 0 selects row[|d| - 1]; d = 0 gives the identity and loads nothing
+KB_FN void kb_operand_fetch_row(kb_operand& o, int d, const ge_precomp* row)
+{
+    o.neg = (uint32_t)d >> 31;
+    const int babs = (d ^ -(int)o.neg) + (int)o.neg;
+    o.nz = (uint32_t)(babs != 0);
+    if (babs != 0) kb_ld_precomp(o.c, row + (babs - 1));
+    else ge_cached_identity(o.c);
+}
+// Q = s*B - h*A: KB_COMB_POS additions from the context comb, then KB_KEY_POS from the key comb, all mixed (the entries are
+// affine), with the operand of the next addition fetched one step ahead as in ge_triple_scalarmult_joint.
+KB_FN void ge_keyset_scalarmult(ge_p3& h, const kb_comb_digit* dw, const int8_t* nd, const ge_precomp* comb, const ge_precomp* ktab)
+{
+    const int nstep = KB_COMB_POS + KB_KEY_POS;
+    ge_identity(h);
+    kb_operand nx;
+    kb_operand_fetch_row(nx, dw[0], comb);
+    KB_NOUNROLL
+    for (int t = 0; t < nstep; t++) {
+        fe e, f, g, hh;
+        ge_cached c;
+        kb_operand_use(c, nx, true);
+        ge_add_front_z(e, f, g, hh, h, c, true);
+        const int u = t + 1;
+        if (u < KB_COMB_POS) kb_operand_fetch_row(nx, dw[u], comb + (size_t)u * KB_COMB_HALF);
+        else if (u < nstep) kb_operand_fetch_row(nx, nd[u - KB_COMB_POS], ktab + (size_t)(u - KB_COMB_POS) * KB_KEY_HALF);
+        ge_tail(h, e, f, g, hh, u < nstep);
+    }
+}
+// byte-level flags of the signature + the facts of its key -> the KB_F_* flags sig_stage1 would produce (without KB_F_FAST)
+template <bool SCHNORR>
+KB_FN uint32_t sig_keyset_flags(uint32_t kf, const uint32_t* sig_w)
+{
+    const uint32_t* r_w = sig_w;
+    const uint32_t* s_w = sig_w + 8;
+    uint32_t f = kf & (KB_F_AC | KB_F_AS);
+    f |= sc_is_canonical(s_w) ? KB_F_SC : 0u;
+    f |= pt_is_canonical(r_w) ? KB_F_RC : 0u;
+    f |= pt_is_small_order_bytes(r_w) ? KB_F_RS : 0u;
+    // EdDSA never looks at A when an earlier check fails; Schnorr decodes A before is_canonical(A)
+    const uint32_t pre_ok = (f & (KB_F_SC | KB_F_RC | KB_F_RS)) == (KB_F_SC | KB_F_RC);
+    if (SCHNORR || (pre_ok && (f & KB_F_AC))) f |= kf & KB_F_AOK;
+    return f;
+}
+// sig_stage1 for a registered key: kf = kb_key_facts of it, pk_w its bytes, ktab its comb.  Items off the fast path add
+// identities and read no table.
+template <bool SCHNORR>
+KB_FN uint32_t sig_keyset_stage1(ge_p3& Q, uint32_t kf, const uint32_t* pk_w, const uint32_t* sig_w, const uint8_t* msg, uint64_t mlen, const ge_precomp* comb, const ge_precomp* ktab)
+{
+    const uint32_t* r_w = sig_w;
+    const uint32_t* s_w = sig_w + 8;
+    const uint32_t f = sig_keyset_flags<SCHNORR>(kf, sig_w);
+    const uint32_t pre_ok = (f & (KB_F_SC | KB_F_RC | KB_F_RS)) == (KB_F_SC | KB_F_RC);
+    const bool fast = pre_ok && (f & (KB_F_AC | KB_F_AS | KB_F_AOK)) == (KB_F_AC | KB_F_AOK);
+    kb_comb_digit dw[KB_COMB_POS];
+    int8_t nd[KB_KEY_POS];
+    if (fast) {
+        uint32_t digest[16], hk[8];
+        sha512_ram(digest, r_w, pk_w, msg, mlen);
+        sc_reduce512(hk, digest);
+        sc_recode_comb(dw, s_w);
+        sc_recode_key_neg(nd, hk);
+    } else {
+        for (int p = 0; p < KB_COMB_POS; p++) dw[p] = 0;
+        for (int p = 0; p < KB_KEY_POS; p++) nd[p] = 0;
+    }
+    ge_keyset_scalarmult(Q, dw, nd, comb, ktab);
+    return fast ? (f | KB_F_FAST) : f;
+}

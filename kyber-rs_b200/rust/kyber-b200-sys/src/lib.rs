@@ -10,6 +10,11 @@ pub struct kb_ctx {
 }
 
 #[repr(C)]
+pub struct kb_keyset {
+    _private: [u8; 0],
+}
+
+#[repr(C)]
 pub struct kb_mctx {
     _private: [u8; 0],
 }
@@ -50,6 +55,12 @@ extern "C" {
 
     pub fn kb_eddsa_verify_batch(ctx: *mut kb_ctx, n: usize, pk: *const u8, msg: *const u8, msg_off: *const u64, sig: *const u8, status: *mut u8) -> c_int;
     pub fn kb_schnorr_verify_batch(ctx: *mut kb_ctx, n: usize, pk: *const u8, msg: *const u8, msg_off: *const u64, sig: *const u8, status: *mut u8) -> c_int;
+
+    // key sets: verification under registered public keys
+    pub fn kb_keyset_create(ctx: *mut kb_ctx, nkeys: usize, pk: *const u8, out: *mut *mut kb_keyset) -> c_int;
+    pub fn kb_keyset_destroy(ks: *mut kb_keyset);
+    pub fn kb_keyset_verify_batch(ks: *mut kb_keyset, n: usize, key_idx: *const u32, msg: *const u8, msg_off: *const u64, sig: *const u8, status: *mut u8, schnorr: c_int) -> c_int;
+    pub fn kb_dev_keyset_verify(ks: *mut kb_keyset, n: usize, d_key_idx: *const c_void, d_msg: *const c_void, d_msg_off: *const c_void, d_sig: *const c_void, d_status: *mut c_void, schnorr: c_int, stream: *mut c_void) -> c_int;
 
     pub fn kb_eddsa_sign_batch(ctx: *mut kb_ctx, n: usize, seeds: *const u8, msg: *const u8, msg_off: *const u64, sig: *mut u8, pk: *mut u8) -> c_int;
 

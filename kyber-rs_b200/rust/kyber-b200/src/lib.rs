@@ -146,6 +146,59 @@ pub fn verify_batch(gpu: &Gpu, items: &[(&[u8], &[u8], &[u8])], schnorr: bool) -
     Ok(res.into_iter().map(|r| r.unwrap()).collect())
 }
 
+/// Public keys registered once with a `Gpu` — the dealers of a DKG round, the participants of a DSS session, a validator
+/// set — so that their signatures are verified by key index without decompressing the key or doubling per signature.
+/// Item by item the result is what `verify_batch` returns for the same key bytes.  Borrows the `Gpu`: a key set is
+/// dropped before its context.
+pub struct KeySet<'a> {
+    gpu: &'a Gpu,
+    ks: *mut sys::kb_keyset,
+    nkeys: usize,
+}
+
+impl<'a> KeySet<'a> {
+    /// Registers `keys` (32-byte encodings, the bytes a verifier would get as the public key).  Keys that fail the
+    /// reference's checks are accepted; their signatures get the reference's error.  384 KiB of device memory per key.
+    pub fn new(gpu: &'a Gpu, keys: &[[u8; 32]]) -> Result<Self, GpuError> {
+        let flat: Vec<u8> = keys.iter().flat_map(|k| k.iter().copied()).collect();
+        let mut ks = std::ptr::null_mut();
+        gpu.check(unsafe { sys::kb_keyset_create(gpu.ctx, keys.len(), flat.as_ptr(), &mut ks) })?;
+        Ok(KeySet { gpu, ks, nkeys: keys.len() })
+    }
+    /// Items are (key index, message, signature); `schnorr` selects `schnorr::verify_with_checks` instead of
+    /// `eddsa::verify_with_checks`.  A key index outside the set is `GpuError::Arg`.
+    pub fn verify_batch(&self, items: &[(u32, &[u8], &[u8])], schnorr: bool) -> Result<Vec<Result<(), SignatureError>>, GpuError> {
+        if items.iter().any(|(k, _, _)| *k as usize >= self.nkeys) {
+            return Err(GpuError::Arg);
+        }
+        let mut res: Vec<Option<Result<(), SignatureError>>> = vec![None; items.len()];
+        let (mut key_idx, mut sig, mut msg, mut off, mut idx) = (vec![], vec![], vec![], vec![0u64], vec![]);
+        for (i, (k, m, s)) in items.iter().enumerate() {
+            if s.len() != 64 {
+                res[i] = Some(status_to_result(1)); // eddsa_sig.rs:161 / schnorr_sig.rs:68
+                continue;
+            }
+            key_idx.push(*k);
+            sig.extend_from_slice(s);
+            msg.extend_from_slice(m);
+            off.push(msg.len() as u64);
+            idx.push(i);
+        }
+        let n = idx.len();
+        let mut st = vec![0u8; n];
+        self.gpu.check(unsafe { sys::kb_keyset_verify_batch(self.ks, n, key_idx.as_ptr(), msg.as_ptr(), off.as_ptr(), sig.as_ptr(), st.as_mut_ptr(), schnorr as i32) })?;
+        for (k, i) in idx.into_iter().enumerate() {
+            res[i] = Some(status_to_result(st[k]));
+        }
+        Ok(res.into_iter().map(|r| r.unwrap()).collect())
+    }
+}
+impl Drop for KeySet<'_> {
+    fn drop(&mut self) {
+        unsafe { sys::kb_keyset_destroy(self.ks) }
+    }
+}
+
 /// Batch companion of `PubPoly::eval` / `PubPoly::check` (share/poly.rs:457-469, :526-530) — the
 /// group math of `Aggregator::verify_deal` (share/vss/pedersen/vss.rs:899-912).
 pub trait PubPolyBatch {
