@@ -239,6 +239,19 @@ int kb_find_pub_batch(kb_ctx* ctx, size_t nlist, const void* list, size_t m, con
 int kb_dkg_process_round(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_t dealer_hi, int fmt, const void* commits, const uint8_t* shares, uint8_t* verdict,
                          const uint8_t* deal_pk, const uint8_t* deal_msg, const uint64_t* deal_msg_off, const uint8_t* deal_sig, uint8_t* deal_status,
                          const uint8_t* resp_pk, const uint8_t* resp_msg, const uint64_t* resp_msg_off, const uint8_t* resp_sig, uint8_t* resp_status);
+/* kb_dkg_process_round with the participants' keys registered as key sets: the signer of deal k is dealer
+ * dealer_lo + k / n, key number dealer_lo + k / n of `dealers` (dealer keys are indexed by absolute dealer number, so a
+ * rank that owns [dealer_lo, dealer_hi) passes the whole dealer set), and the signer of response k is verifier k % n, key
+ * number k % n of `verifiers`.  verdict, deal_status and resp_status are exactly what kb_dkg_process_round returns for
+ * those keys; the arrays are laid out as there, without the two pk arrays.  dealers and verifiers may be the same key set
+ * (a new DKG: every participant deals and verifies) or two (resharing: old nodes deal, new nodes verify).
+ * KB_ERR_ARG, before anything is launched, when dealers->nkeys < dealer_hi, verifiers->nkeys < n, a key set belongs to
+ * another context, or a batch has a sig pointer but its key set is NULL.  A batch whose sig pointer is NULL is skipped.
+ * Only msg[msg_off[0] .. msg_off[m]) of each batch is copied to the device. */
+int kb_dkg_process_round_keyed(kb_ctx* ctx, const kb_keyset* dealers, const kb_keyset* verifiers,
+                               size_t n, size_t t, size_t dealer_lo, size_t dealer_hi, int fmt, const void* commits, const uint8_t* shares, uint8_t* verdict,
+                               const uint8_t* deal_msg, const uint64_t* deal_msg_off, const uint8_t* deal_sig, uint8_t* deal_status,
+                               const uint8_t* resp_msg, const uint64_t* resp_msg_off, const uint8_t* resp_sig, uint8_t* resp_status);
 /* vss::rabin verify_deal group math (share/vss/rabin/vss.rs:889-900): verdict[k] = 1 iff
  * f_shares[k]*G + g_shares[k]*H == poly[poly_id[k]].eval(idx[k]); H = derive_h(verifiers) supplied by the caller.
  * Both shares only meet constant-time table selects. */
@@ -297,6 +310,13 @@ int kb_dev_pripoly_eval(kb_ctx* ctx, size_t npoly, size_t t, const void* d_coeff
 int kb_dev_dkg_process_round(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, int fmt, const void* d_commits, const void* d_shares, void* d_verdict,
                              const void* d_deal_pk, const void* d_deal_msg, const void* d_deal_msg_off, const void* d_deal_sig, void* d_deal_status,
                              const void* d_resp_pk, const void* d_resp_msg, const void* d_resp_msg_off, const void* d_resp_sig, void* d_resp_status, void* stream);
+/* kb_dkg_process_round_keyed on device buffers for the ndealers dealers from dealer_lo on (the arrays start at the first of
+ * them; dealer keys are still indexed by absolute dealer number): the checks of the host form with dealer_hi =
+ * dealer_lo + ndealers, then ordered like every kb_dev_* call of the context. */
+int kb_dev_dkg_process_round_keyed(kb_ctx* ctx, const kb_keyset* dealers, const kb_keyset* verifiers,
+                                   size_t n, size_t t, size_t dealer_lo, size_t ndealers, int fmt, const void* d_commits, const void* d_shares, void* d_verdict,
+                                   const void* d_deal_msg, const void* d_deal_msg_off, const void* d_deal_sig, void* d_deal_status,
+                                   const void* d_resp_msg, const void* d_resp_msg_off, const void* d_resp_sig, void* d_resp_status, void* stream);
 
 /* ---- multi-device context: ONE host batch sharded over the GPUs of a box, from one process ---------------------------
  * (SURVEY §8b/§8e).  kb_mctx_create builds one kb_ctx per listed device and, for more than one device, an NCCL communicator
@@ -326,6 +346,23 @@ int kb_mctx_dkg_verify_round(kb_mctx* m, size_t n, size_t t, size_t ndealers, in
 int kb_mctx_dkg_process_round(kb_mctx* m, size_t n, size_t t, size_t ndealers, int fmt, const void* commits, const uint8_t* shares, uint8_t* verdict,
                               const uint8_t* deal_pk, const uint8_t* deal_msg, const uint64_t* deal_msg_off, const uint8_t* deal_sig, uint8_t* deal_status,
                               const uint8_t* resp_pk, const uint8_t* resp_msg, const uint64_t* resp_msg_off, const uint8_t* resp_sig, uint8_t* resp_status);
+/* Key sets over all devices.  A kb_mkeyset holds one kb_keyset per device, and each of them holds EVERY key: the keys are
+ * replicated, not sharded, so a key set of K keys takes 384 KiB x K of memory on each GPU.  kb_mctx_keyset_create builds
+ * the combs of all devices concurrently; if one device fails, the sets already built are destroyed and the error is in
+ * kb_mctx_last_error.  A kb_mkeyset must be destroyed before its kb_mctx. */
+typedef struct kb_mkeyset kb_mkeyset;
+int  kb_mctx_keyset_create(kb_mctx* m, size_t nkeys, const uint8_t* pk, kb_mkeyset** out);
+void kb_mctx_keyset_destroy(kb_mkeyset* ks);
+/* kb_keyset_verify_batch split by index over all devices.  Every key index is checked before any device starts
+ * (KB_ERR_ARG); each device copies only the message bytes of its own items. */
+int  kb_mctx_keyset_verify_batch(kb_mkeyset* ks, size_t n, const uint32_t* key_idx, const uint8_t* msg, const uint64_t* msg_off,
+                                 const uint8_t* sig, uint8_t* status, int schnorr);
+/* kb_dkg_process_round_keyed for ndealers dealers split by dealer (arrays whole, as kb_mctx_dkg_process_round has them):
+ * each device runs its dealer range against its own copy of the key sets. */
+int  kb_mctx_dkg_process_round_keyed(kb_mctx* m, const kb_mkeyset* dealers, const kb_mkeyset* verifiers, size_t n, size_t t, size_t ndealers, int fmt,
+                                     const void* commits, const uint8_t* shares, uint8_t* verdict,
+                                     const uint8_t* deal_msg, const uint64_t* deal_msg_off, const uint8_t* deal_sig, uint8_t* deal_status,
+                                     const uint8_t* resp_msg, const uint64_t* resp_msg_off, const uint8_t* resp_sig, uint8_t* resp_status);
 /* kb_msm over all devices */
 int kb_mctx_msm(kb_mctx* m, size_t n, const uint8_t* scalars, const uint8_t* points, uint8_t* out32, uint64_t* bad_points);
 

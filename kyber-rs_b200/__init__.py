@@ -14,6 +14,7 @@ from .binding import (  # noqa: F401
     Context,
     KeySet,
     MultiContext,
+    MultiKeySet,
     KBError,
     LIB_PATH,
     SIG_STATUS_NAMES,
@@ -24,4 +25,4 @@ from .binding import (  # noqa: F401
 from . import host  # noqa: F401
 from . import sharding  # noqa: F401
 
-__all__ = ["Context", "KeySet", "MultiContext", "KBError", "LIB_PATH", "SIG_STATUS_NAMES", "FLAG_VARTIME", "FLAG_SHARED_POINT", "load_library", "host", "sharding"]
+__all__ = ["Context", "KeySet", "MultiContext", "MultiKeySet", "KBError", "LIB_PATH", "SIG_STATUS_NAMES", "FLAG_VARTIME", "FLAG_SHARED_POINT", "load_library", "host", "sharding"]

@@ -45,6 +45,8 @@ EXPORTS = [
     "kb_dev_eddsa_verify", "kb_dev_point_mul_base", "kb_dev_point_mul", "kb_dev_msm", "kb_dev_msm_ext", "kb_dev_dkg_verify_round", "kb_dev_dkg_verify_round_limbs", "kb_dev_point_sum",
     "kb_probe_imad", "kb_verify_kernel_times",
     "kb_keyset_create", "kb_keyset_destroy", "kb_keyset_verify_batch", "kb_dev_keyset_verify",
+    "kb_dkg_process_round_keyed", "kb_dev_dkg_process_round_keyed",
+    "kb_mctx_keyset_create", "kb_mctx_keyset_destroy", "kb_mctx_keyset_verify_batch", "kb_mctx_dkg_process_round_keyed",
 ]
 
 
@@ -137,6 +139,13 @@ def load_library(path: str = LIB_PATH):
     L.kb_keyset_destroy.restype = None
     L.kb_keyset_verify_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32]
     L.kb_dev_keyset_verify.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32, vp]
+    L.kb_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8
+    L.kb_dev_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8 + [vp]
+    L.kb_mctx_keyset_create.argtypes = [vp, sz, vp, ctypes.POINTER(vp)]
+    L.kb_mctx_keyset_destroy.argtypes = [vp]
+    L.kb_mctx_keyset_destroy.restype = None
+    L.kb_mctx_keyset_verify_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32]
+    L.kb_mctx_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8
     _LIB = L
     return L
 
@@ -159,6 +168,25 @@ def pack_messages(msgs):
         off[1:] = np.cumsum([len(m) for m in msgs], dtype=np.uint64)
     flat = np.frombuffer(b"".join(msgs), dtype=np.uint8).copy() if int(off[-1]) else np.zeros(0, dtype=np.uint8)
     return flat, off
+
+
+def _keyed_batches(deal, resp, m, what):
+    """(ctypes args, [deal_status | None, resp_status | None], arrays to keep alive) of the two signature batches of a
+    keyed round; a batch is (msg flat, msg_off[m+1], sig[m,64]) or None."""
+    args, outs, keep = [], [], []
+    for batch in (deal, resp):
+        if batch is None:
+            args += [None] * 4
+            outs.append(None)
+            continue
+        msg, off, sig = _u8(batch[0]), np.ascontiguousarray(batch[1], dtype=np.uint64), _u8(batch[2], (-1, 64))
+        if sig.shape[0] != m or off.shape[0] != m + 1:
+            raise ValueError(f"{what}: a signature batch must hold one item per (dealer, verifier) of the range")
+        st = np.empty(m, dtype=np.uint8)
+        keep += [msg, off, sig]
+        args += [_ptr(msg), _ptr(off), _ptr(sig), _ptr(st)]
+        outs.append(st)
+    return args, outs, keep
 
 
 class Context:
@@ -431,6 +459,25 @@ class Context:
         self._check(self.L.kb_dkg_process_round(self.h, n, t, dealer_lo, dealer_hi, int(limbs), _ptr(c), _ptr(sh), _ptr(verdict), *args), "kb_dkg_process_round")
         return verdict, outs[0], outs[1]
 
+    def dkg_process_round_keyed(self, n, t, commits, shares, dealers, verifiers=None, deal=None, resp=None, dealer_lo=0, dealer_hi=None, limbs=False):
+        """dkg_process_round with the participants' keys as KeySets of this context: deal k is signed by dealer key
+        dealer_lo + k // n, response k by verifier key k % n (verifiers=None: the dealers' set).
+        deal / resp = (msg flat, msg_off[m+1], sig[m,64]) for the m = (dealer_hi-dealer_lo)*n items, or None."""
+        if verifiers is None:
+            verifiers = dealers
+        c = self._points(commits, limbs)
+        sh = _u8(shares, (-1, 32))
+        ndealers = c.shape[0] // t
+        if dealer_hi is None:
+            dealer_hi = ndealers
+        if ndealers * t != c.shape[0] or sh.shape[0] != ndealers * n or not (0 <= dealer_lo <= dealer_hi <= ndealers):
+            raise ValueError("dkg_process_round_keyed: inconsistent shapes")
+        verdict = np.zeros(ndealers * n, dtype=np.uint8)
+        args, outs, keep = _keyed_batches(deal, resp, (dealer_hi - dealer_lo) * n, "dkg_process_round_keyed")
+        self._check(self.L.kb_dkg_process_round_keyed(self.h, KeySet._h(dealers), KeySet._h(verifiers), n, t, dealer_lo, dealer_hi, int(limbs), _ptr(c), _ptr(sh), _ptr(verdict), *args),
+                    "kb_dkg_process_round_keyed")
+        return verdict, outs[0], outs[1]
+
     def vss_rabin_verify_deals_batch(self, commits, t, h_point, poly_id, idx, f_shares, g_shares):
         c = _u8(commits, (-1, 32))
         npoly = c.shape[0] // t
@@ -572,6 +619,17 @@ class Context:
             a += [self._dp(x) for x in batch] if batch is not None else [None] * 5
         self._check(self.L.kb_dev_dkg_process_round(self.h, n, t, ndealers, int(limbs), self._dp(commits), self._dp(shares), self._dp(verdict), *a, self._stream()), "kb_dev_dkg_process_round")
 
+    def dev_dkg_process_round_keyed(self, n, t, ndealers, commits, shares, verdict, dealers, verifiers=None, deal=None, resp=None, dealer_lo=0, limbs=False):
+        """dkg_process_round_keyed on CUDA tensors for the ndealers dealers from dealer_lo on (the arrays start at the first
+        of them); deal / resp = (msg, msg_off, sig, status) CUDA tensors or None."""
+        if verifiers is None:
+            verifiers = dealers
+        a = []
+        for batch in (deal, resp):
+            a += [self._dp(x) for x in batch] if batch is not None else [None] * 4
+        self._check(self.L.kb_dev_dkg_process_round_keyed(self.h, KeySet._h(dealers), KeySet._h(verifiers), n, t, dealer_lo, ndealers, int(limbs), self._dp(commits), self._dp(shares),
+                                                          self._dp(verdict), *a, self._stream()), "kb_dev_dkg_process_round_keyed")
+
     def dev_pripoly_eval(self, npoly, t, coeffs, n, out):
         self._check(self.L.kb_dev_pripoly_eval(self.h, npoly, t, self._dp(coeffs), n, self._dp(out), self._stream()), "kb_dev_pripoly_eval")
 
@@ -603,6 +661,10 @@ class KeySet:
         if getattr(self, "h", None):
             self.L.kb_keyset_destroy(self.h)
             self.h = None
+
+    @staticmethod
+    def _h(ks):
+        return ks.h if ks is not None else None
 
     def __del__(self):  # pragma: no cover
         try:
@@ -713,6 +775,28 @@ class MultiContext:
     def dkg_verify_round(self, n, t, commits, shares, limbs=False, verdict=None):
         return self.dkg_process_round(n, t, commits, shares, limbs=limbs, verdict=verdict)[0]
 
+    def keyset(self, pk):
+        """Registers the public keys pk (nkeys x 32 encodings) on every device of this context (MultiKeySet)."""
+        return MultiKeySet(self, pk)
+
+    def dkg_process_round_keyed(self, n, t, commits, shares, dealers, verifiers=None, deal=None, resp=None, limbs=False, verdict=None):
+        """dkg_process_round with the participants' keys as MultiKeySets of this context, split by dealer: deal k is
+        signed by dealer key k // n, response k by verifier key k % n (verifiers=None: the dealers' set).
+        deal / resp = (msg flat, msg_off[m+1], sig[m,64]) for the m = ndealers*n items, or None."""
+        if verifiers is None:
+            verifiers = dealers
+        c = Context._points(commits, limbs)
+        sh = _u8(shares, (-1, 32))
+        ndealers = c.shape[0] // t
+        if ndealers * t != c.shape[0] or sh.shape[0] != ndealers * n:
+            raise ValueError("dkg_process_round_keyed: inconsistent shapes")
+        if verdict is None:
+            verdict = np.zeros(ndealers * n, dtype=np.uint8)
+        args, outs, keep = _keyed_batches(deal, resp, ndealers * n, "dkg_process_round_keyed")
+        self._check(self.L.kb_mctx_dkg_process_round_keyed(self.h, KeySet._h(dealers), KeySet._h(verifiers), n, t, ndealers, int(limbs), _ptr(c), _ptr(sh), _ptr(verdict), *args),
+                    "kb_mctx_dkg_process_round_keyed")
+        return verdict, outs[0], outs[1]
+
     def msm(self, scalars, points):
         s, p = _u8(scalars, (-1, 32)), _u8(points, (-1, 32))
         assert s.shape == p.shape
@@ -720,3 +804,41 @@ class MultiContext:
         bad = np.zeros(1, dtype=np.uint64)
         self._check(self.L.kb_mctx_msm(self.h, s.shape[0], _ptr(s), _ptr(p), _ptr(out), _ptr(bad)), "kb_mctx_msm")
         return out.tobytes(), int(bad[0])
+
+
+class MultiKeySet:
+    """One kb_mkeyset: public keys registered on every device of a MultiContext.  Each device holds every key
+    (384 KiB per key on each GPU); verify_batch splits a batch by index like MultiContext.verify_batch."""
+
+    def __init__(self, mctx: MultiContext, pk):
+        self.mctx = mctx   # the key set belongs to its context and must go before it
+        self.L = mctx.L
+        self.h = None
+        p = _u8(pk, (-1, 32))
+        self.nkeys = p.shape[0]
+        h = ctypes.c_void_p()
+        mctx._check(self.L.kb_mctx_keyset_create(mctx.h, self.nkeys, _ptr(p), ctypes.byref(h)), "kb_mctx_keyset_create")
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.kb_mctx_keyset_destroy(self.h)
+            self.h = None
+
+    def __del__(self):  # pragma: no cover
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def verify_batch(self, key_idx, msg, msg_off, sig, schnorr=False, out=None):
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        sig = _u8(sig, (-1, 64))
+        msg = _u8(msg)
+        msg_off = np.ascontiguousarray(msg_off, dtype=np.uint64)
+        n = key_idx.shape[0]
+        if sig.shape[0] != n or msg_off.shape[0] != n + 1:
+            raise ValueError("MultiKeySet.verify_batch: one key index and one signature per item, n+1 message offsets")
+        st = out if out is not None else np.empty(n, dtype=np.uint8)
+        self.mctx._check(self.L.kb_mctx_keyset_verify_batch(self.h, n, _ptr(key_idx), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(st), int(schnorr)), "kb_mctx_keyset_verify_batch")
+        return st

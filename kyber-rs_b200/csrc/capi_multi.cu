@@ -196,6 +196,82 @@ int kb_mctx_dkg_verify_round(kb_mctx* m, size_t n, size_t t, size_t ndealers, in
     return kb_mctx_dkg_process_round(m, n, t, ndealers, fmt, commits, shares, verdict, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
 }
 
+// ---- key sets, replicated on every device ------------------------------------------------------------------------------
+struct kb_mkeyset {
+    kb_mctx* m;
+    size_t nkeys;
+    kb_keyset* ks[KB_MAX_DEVICES];   // ks[i] belongs to m->ctx[i] and holds every key
+};
+
+int kb_mctx_keyset_create(kb_mctx* m, size_t nkeys, const uint8_t* pk, kb_mkeyset** out)
+{
+    if (!out) return KB_ERR_ARG;
+    *out = nullptr;
+    if (!m || nkeys == 0 || !pk) return KB_ERR_ARG;
+    kb_mkeyset* mk = (kb_mkeyset*)calloc(1, sizeof(kb_mkeyset));
+    if (!mk) return KB_ERR_NOMEM;
+    mk->m = m;
+    mk->nkeys = nkeys;
+    const int rc = kb_on_all(m, [&](int i) { return kb_keyset_create(m->ctx[i], nkeys, pk, &mk->ks[i]); });
+    if (rc != KB_OK) {
+        kb_mctx_keyset_destroy(mk);
+        return rc;
+    }
+    *out = mk;
+    return KB_OK;
+}
+void kb_mctx_keyset_destroy(kb_mkeyset* mk)
+{
+    if (!mk) return;
+    for (int i = 0; i < mk->m->ndev; i++) kb_keyset_destroy(mk->ks[i]);
+    free(mk);
+}
+int kb_mctx_keyset_verify_batch(kb_mkeyset* mk, size_t n, const uint32_t* key_idx, const uint8_t* msg, const uint64_t* msg_off, const uint8_t* sig, uint8_t* status, int schnorr)
+{
+    if (!mk || (n && (!key_idx || !msg_off || !sig || !status))) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    uint32_t over = 0;
+    for (size_t i = 0; i < n; i++) over |= (uint32_t)(key_idx[i] >= mk->nkeys);
+    if (over || !kb_msg_off_ok(n, msg_off) || (msg_off[n] != msg_off[0] && !msg)) return KB_ERR_ARG;
+    kb_mctx* m = mk->m;
+    return kb_on_all(m, [&](int i) {
+        size_t lo, hi;
+        kb_shard(n, i, m->ndev, &lo, &hi);
+        if (hi == lo) return (int)KB_OK;
+        // the device is handed its own message bytes, with offsets made relative to the first of them
+        const size_t cn = hi - lo;
+        const uint64_t m0 = msg_off[lo];
+        uint64_t* off = (uint64_t*)malloc(8 * (cn + 1));
+        if (!off) return (int)KB_ERR_NOMEM;
+        for (size_t j = 0; j <= cn; j++) off[j] = msg_off[lo + j] - m0;
+        const int rc = kb_keyset_verify_batch(mk->ks[i], cn, key_idx + lo, msg ? msg + m0 : nullptr, off, sig + 64 * lo, status + lo, schnorr);
+        free(off);
+        return rc;
+    });
+}
+int kb_mctx_dkg_process_round_keyed(kb_mctx* m, const kb_mkeyset* dealers, const kb_mkeyset* verifiers, size_t n, size_t t, size_t ndealers, int fmt,
+                                    const void* commits, const uint8_t* shares, uint8_t* verdict,
+                                    const uint8_t* deal_msg, const uint64_t* deal_msg_off, const uint8_t* deal_sig, uint8_t* deal_status,
+                                    const uint8_t* resp_msg, const uint64_t* resp_msg_off, const uint8_t* resp_sig, uint8_t* resp_status)
+{
+    if (!m || !t || (n && ndealers && (!commits || !shares || !verdict))) return KB_ERR_ARG;
+    // the key-set checks of kb_dkg_process_round_keyed for the whole round, before any device starts
+    if ((deal_sig && !dealers) || (resp_sig && !verifiers)) return KB_ERR_ARG;
+    if (dealers && (dealers->m != m || dealers->nkeys < ndealers)) return KB_ERR_ARG;
+    if (verifiers && (verifiers->m != m || verifiers->nkeys < n)) return KB_ERR_ARG;
+    return kb_on_all(m, [&](int i) {
+        size_t lo, hi;
+        kb_shard(ndealers, i, m->ndev, &lo, &hi);
+        if (hi == lo) return (int)KB_OK;
+        // as kb_mctx_dkg_process_round: the signature arrays are handed over as the slice of the dealer range, whose
+        // dealer keys keep their absolute numbers
+        const size_t k0 = lo * n;
+        return kb_dkg_process_round_keyed(m->ctx[i], dealers ? dealers->ks[i] : nullptr, verifiers ? verifiers->ks[i] : nullptr, n, t, lo, hi, fmt, commits, shares, verdict,
+                                          deal_msg, deal_sig ? deal_msg_off + k0 : nullptr, deal_sig ? deal_sig + 64 * k0 : nullptr, deal_sig ? deal_status + k0 : nullptr,
+                                          resp_msg, resp_sig ? resp_msg_off + k0 : nullptr, resp_sig ? resp_sig + 64 * k0 : nullptr, resp_sig ? resp_status + k0 : nullptr);
+    });
+}
+
 // ---- sharded by points, one collective ---------------------------------------------------------------------------------
 int kb_mctx_msm(kb_mctx* m, size_t n, const uint8_t* scalars, const uint8_t* points, uint8_t* out32, uint64_t* bad_points)
 {

@@ -558,6 +558,29 @@ static __global__ void __launch_bounds__(256) k_keyset_bad_index(size_t n, const
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n && __ldg(key_idx + i) >= nkeys) status[i] = 0xFF;
 }
+// k_keyset_verify<true> for one signature batch of a DKG round (kb_dkg_process_round_keyed).  Item k = (d - dealer_lo) n + i
+// is signed by dealer dealer_lo + k / n (a deal, RESP = false) or by verifier k % n (a response, RESP = true); the caller
+// has checked that every such key is in the set, so no index array is read.  msg_off holds offsets into the caller's
+// whole message array; `msg` points at byte msg_base of it.
+template <bool RESP>
+static __global__ void __launch_bounds__(KB_THREADS) k_keyset_verify_round(size_t m, size_t n, size_t dealer_lo, const uint8_t* kpk, const uint8_t* facts, const ge_precomp* ktab,
+                                                                           const uint8_t* msg, const uint64_t* msg_off, uint64_t msg_base, const uint8_t* sig, const ge_precomp* comb,
+                                                                           uint32_t* xyz, uint8_t* flags)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const size_t k = RESP ? i % n : dealer_lo + i / n;
+    uint32_t pw[8], sw[16];
+    kb_load32(pw, kpk, k);
+    const uint32_t kf = __ldg(facts + k);
+    kb_load32(sw, sig, 2 * i);
+    kb_load32(sw + 8, sig, 2 * i + 1);
+    const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
+    ge_p3 Q;
+    const uint32_t f = sig_keyset_stage1<true>(Q, kf, pw, sw, msg + (lo - msg_base), hi - lo, comb, ktab + k * KB_KEY_ENTRIES);
+    kb_store_xyz(xyz, i, Q);
+    flags[i] = (uint8_t)f;
+}
 #endif  // KB_K_KEYSET
 
 // ---- the same verifiers with half-size scalars (ops.cuh sig_half_*, half.cuh): 128 doublings per signature,

@@ -19,6 +19,11 @@ pub struct kb_mctx {
     _private: [u8; 0],
 }
 
+#[repr(C)]
+pub struct kb_mkeyset {
+    _private: [u8; 0],
+}
+
 pub const KB_OK: c_int = 0;
 pub const KB_ERR_NCCL: c_int = -4;
 pub const KB_ERR_ARG: c_int = -1;
@@ -88,6 +93,15 @@ extern "C" {
     pub fn kb_dev_dkg_process_round(ctx: *mut kb_ctx, n: usize, t: usize, ndealers: usize, fmt: c_int, d_commits: *const c_void, d_shares: *const c_void, d_verdict: *mut c_void,
         d_deal_pk: *const c_void, d_deal_msg: *const c_void, d_deal_msg_off: *const c_void, d_deal_sig: *const c_void, d_deal_status: *mut c_void,
         d_resp_pk: *const c_void, d_resp_msg: *const c_void, d_resp_msg_off: *const c_void, d_resp_sig: *const c_void, d_resp_status: *mut c_void, stream: *mut c_void) -> c_int;
+    // DKG rounds under registered participant keys (deal k: dealer key dealer_lo + k / n, response k: verifier key k % n)
+    pub fn kb_dkg_process_round_keyed(ctx: *mut kb_ctx, dealers: *const kb_keyset, verifiers: *const kb_keyset, n: usize, t: usize, dealer_lo: usize, dealer_hi: usize, fmt: c_int,
+        commits: *const c_void, shares: *const u8, verdict: *mut u8,
+        deal_msg: *const u8, deal_msg_off: *const u64, deal_sig: *const u8, deal_status: *mut u8,
+        resp_msg: *const u8, resp_msg_off: *const u64, resp_sig: *const u8, resp_status: *mut u8) -> c_int;
+    pub fn kb_dev_dkg_process_round_keyed(ctx: *mut kb_ctx, dealers: *const kb_keyset, verifiers: *const kb_keyset, n: usize, t: usize, dealer_lo: usize, ndealers: usize, fmt: c_int,
+        d_commits: *const c_void, d_shares: *const c_void, d_verdict: *mut c_void,
+        d_deal_msg: *const c_void, d_deal_msg_off: *const c_void, d_deal_sig: *const c_void, d_deal_status: *mut c_void,
+        d_resp_msg: *const c_void, d_resp_msg_off: *const c_void, d_resp_sig: *const c_void, d_resp_status: *mut c_void, stream: *mut c_void) -> c_int;
 
     pub fn kb_dev_eddsa_verify(ctx: *mut kb_ctx, n: usize, d_pk: *const c_void, d_msg: *const c_void, d_msg_off: *const c_void, d_sig: *const c_void, d_status: *mut c_void, schnorr: c_int, stream: *mut c_void) -> c_int;
     pub fn kb_dev_point_mul_base(ctx: *mut kb_ctx, n: usize, d_scalars: *const c_void, d_out: *mut c_void, flags: u32, stream: *mut c_void) -> c_int;
@@ -116,6 +130,13 @@ extern "C" {
     pub fn kb_mctx_dkg_process_round(m: *mut kb_mctx, n: usize, t: usize, ndealers: usize, fmt: c_int, commits: *const c_void, shares: *const u8, verdict: *mut u8,
         deal_pk: *const u8, deal_msg: *const u8, deal_msg_off: *const u64, deal_sig: *const u8, deal_status: *mut u8,
         resp_pk: *const u8, resp_msg: *const u8, resp_msg_off: *const u64, resp_sig: *const u8, resp_status: *mut u8) -> c_int;
+    pub fn kb_mctx_keyset_create(m: *mut kb_mctx, nkeys: usize, pk: *const u8, out: *mut *mut kb_mkeyset) -> c_int;
+    pub fn kb_mctx_keyset_destroy(ks: *mut kb_mkeyset);
+    pub fn kb_mctx_keyset_verify_batch(ks: *mut kb_mkeyset, n: usize, key_idx: *const u32, msg: *const u8, msg_off: *const u64, sig: *const u8, status: *mut u8, schnorr: c_int) -> c_int;
+    pub fn kb_mctx_dkg_process_round_keyed(m: *mut kb_mctx, dealers: *const kb_mkeyset, verifiers: *const kb_mkeyset, n: usize, t: usize, ndealers: usize, fmt: c_int,
+        commits: *const c_void, shares: *const u8, verdict: *mut u8,
+        deal_msg: *const u8, deal_msg_off: *const u64, deal_sig: *const u8, deal_status: *mut u8,
+        resp_msg: *const u8, resp_msg_off: *const u64, resp_sig: *const u8, resp_status: *mut u8) -> c_int;
     pub fn kb_mctx_msm(m: *mut kb_mctx, n: usize, scalars: *const u8, points: *const u8, out32: *mut u8, bad_points: *mut u64) -> c_int;
 
     pub fn kb_probe_imad(ctx: *mut kb_ctx, kind: c_int, iters: c_int, macs_per_sec: *mut c_double, elapsed_ms: *mut c_double) -> c_int;

@@ -256,3 +256,48 @@ pub fn dkg_verify_round(gpu: &Gpu, n: usize, polys: &[Vec<EdPoint>], shares: &[E
     gpu.check(unsafe { sys::kb_dkg_verify_round_limbs(gpu.ctx, n, t, 0, polys.len(), limbs.as_ptr(), sh.as_ptr(), verdict.as_mut_ptr()) })?;
     Ok(verdict.into_iter().map(|v| v == 1).collect())
 }
+
+/// The flat (messages, offsets, signatures) of one keyed signature batch; a signature that is not 64 bytes long enters as
+/// 64 zero bytes and its result is replaced by the reference's length error afterwards.
+fn pack_keyed_batch(items: &[(&[u8], &[u8])]) -> (Vec<u8>, Vec<u64>, Vec<u8>) {
+    let (mut msg, mut off, mut sig) = (vec![], vec![0u64], vec![]);
+    for (m, s) in items {
+        msg.extend_from_slice(m);
+        off.push(msg.len() as u64);
+        if s.len() == 64 {
+            sig.extend_from_slice(s);
+        } else {
+            sig.extend_from_slice(&[0u8; 64]);
+        }
+    }
+    (msg, off, sig)
+}
+
+/// `dkg_verify_round` plus the two Schnorr checks of the round (dkg.rs:531 on each deal, vss.rs:943 on each response) under
+/// registered participant keys: `deals[d * n + i]` and `responses[d * n + i]` are (message, signature) of the deal dealer
+/// `d` sent to verifier `i` and of that verifier's response, signed by key `d` of `dealers` and key `i` of `verifiers`.
+/// `dealers` and `verifiers` may be the same key set (a new DKG) or two (resharing).  An empty `deals` or `responses`
+/// skips that batch.  Returns (verdict, deal results, response results), each item what the scalar calls return.
+pub fn dkg_process_round_keyed(gpu: &Gpu, dealers: &KeySet, verifiers: &KeySet, n: usize, polys: &[Vec<EdPoint>], shares: &[EdScalar],
+                               deals: &[(&[u8], &[u8])], responses: &[(&[u8], &[u8])])
+                               -> Result<(Vec<bool>, Vec<Result<(), SignatureError>>, Vec<Result<(), SignatureError>>), GpuError> {
+    let t = polys.first().map(|p| p.len()).unwrap_or(0);
+    let m = polys.len() * n;
+    assert!(polys.iter().all(|p| p.len() == t) && shares.len() == m);
+    assert!((deals.is_empty() || deals.len() == m) && (responses.is_empty() || responses.len() == m));
+    let limbs: Vec<i32> = polys.iter().flat_map(|p| pack_point_limbs(p)).collect();
+    let sh = pack_scalars(shares);
+    let mut verdict = vec![0u8; m];
+    let (dm, doff, dsig) = pack_keyed_batch(deals);
+    let (rm, roff, rsig) = pack_keyed_batch(responses);
+    let (mut dst, mut rst) = (vec![0u8; deals.len()], vec![0u8; responses.len()]);
+    let sig_ptr = |items: &[(&[u8], &[u8])], s: &Vec<u8>| if items.is_empty() { std::ptr::null() } else { s.as_ptr() };
+    gpu.check(unsafe {
+        sys::kb_dkg_process_round_keyed(gpu.ctx, dealers.ks, verifiers.ks, n, t, 0, polys.len(), 1 /* KB_POINT_LIMBS40 */, limbs.as_ptr() as *const std::os::raw::c_void, sh.as_ptr(), verdict.as_mut_ptr(),
+                                        dm.as_ptr(), doff.as_ptr(), sig_ptr(deals, &dsig), dst.as_mut_ptr(), rm.as_ptr(), roff.as_ptr(), sig_ptr(responses, &rsig), rst.as_mut_ptr())
+    })?;
+    let results = |items: &[(&[u8], &[u8])], st: Vec<u8>| -> Vec<Result<(), SignatureError>> {
+        items.iter().zip(st).map(|((_, s), x)| status_to_result(if s.len() == 64 { x } else { 1 })).collect()
+    };
+    Ok((verdict.into_iter().map(|v| v == 1).collect(), results(deals, dst), results(responses, rst)))
+}
