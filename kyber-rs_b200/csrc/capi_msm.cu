@@ -30,11 +30,7 @@ int kb_msm_run(kb_ctx* ctx, size_t n, const uint8_t* d_scalars, const void* d_po
         pl.half = 1u << (pl.c - 1);
         pl.nb = pl.windows * pl.half;
         pl.k = kb_msm_chunk_entries(cn, pl.half);
-        // bucket groups per window: fewer groups = longer serial runs in k_msm_reduce but a shorter fold in k_msm_window_sums
-        // (one block per window).  Measured (round 2, KB_MSM_GROUPS): 2^17 points 1.40 / 1.32 / 1.27 / 1.29 ms for
-        // 4096 / 2048 / 1024 / 512 groups, 2^22 points 14.76 / 14.66 / 14.68 / 14.86 ms.
-        const uint32_t gmax = ctx->msm_groups ? (uint32_t)ctx->msm_groups : (pl.half <= 8192u ? 1024u : 2048u);
-        const uint32_t groups = pl.half < gmax ? pl.half : gmax;
+        const uint32_t groups = kb_msm_groups_host(pl.half, (uint32_t)ctx->msm_groups);
         const size_t nthreads = (cn * pl.windows + pl.k - 1) / pl.k;
         uint32_t *pts, *mags, *counts, *offsets, *cursor, *sorted, *bucket_sum, *heads, *tails, *partial, *tile_sums, *long_list, *win_sum;
         uint8_t *negs, *flags;

@@ -61,6 +61,16 @@ static inline uint32_t kb_msm_window_bits_host(size_t n)
     return (uint32_t)c;
 }
 
+// bucket groups per window in the reduction: fewer groups = longer serial runs in k_msm_reduce but a shorter fold in
+// k_msm_window_sums (one block per window).  Measured (round 2, KB_MSM_GROUPS): 2^17 points 1.40 / 1.32 / 1.27 / 1.29 ms
+// for 4096 / 2048 / 1024 / 512 groups, 2^22 points 14.76 / 14.66 / 14.68 / 14.86 ms.
+// setting: the context's KB_MSM_GROUPS (0 = by window size); never more groups than buckets in a window.
+static inline uint32_t kb_msm_groups_host(uint32_t half, uint32_t setting)
+{
+    const uint32_t gmax = setting ? setting : (half <= 8192u ? 1024u : 2048u);
+    return half < gmax ? half : gmax;
+}
+
 // bits [pos, pos + c) of the 256-bit magnitude (zero beyond bit 255), c <= 16
 KB_FN uint32_t sc_bits(const uint32_t* mag, uint32_t pos, uint32_t c)
 {

@@ -417,7 +417,8 @@ int emu_point_from_limbs_checked(uint8_t* out, const int32_t* limbs)
 
 // Pippenger stage bodies of msm.cuh, run "thread by thread" on the host; the final
 // warp-shuffle tree (GPU only) is replaced by a plain sum of the same group partials.
-int emu_msm(uint8_t* out, size_t n, const uint8_t* scalars, const uint8_t* points, int c_override, int k_override)
+// c, k, groups: 0 = what the driver (capi_msm.cu) picks for n points; groups is the context's KB_MSM_GROUPS setting.
+int emu_msm_plan(uint8_t* out, size_t n, const uint8_t* scalars, const uint8_t* points, int c_override, int k_override, int groups_setting)
 {
     kb_msm_plan pl;
     pl.n = (uint32_t)n;
@@ -426,7 +427,7 @@ int emu_msm(uint8_t* out, size_t n, const uint8_t* scalars, const uint8_t* point
     pl.half = 1u << (pl.c - 1);
     pl.nb = pl.windows * pl.half;
     pl.k = k_override ? (uint32_t)k_override : kb_msm_chunk_entries(n, pl.half);
-    const uint32_t groups = pl.half < KB_MSM_GROUPS ? pl.half : KB_MSM_GROUPS;
+    const uint32_t groups = kb_msm_groups_host(pl.half, (uint32_t)groups_setting);
     const size_t nthreads = (n * pl.windows + pl.k - 1) / pl.k;
     std::vector<uint32_t> pts(24 * n + 24), mags(8 * n + 8), counts(pl.nb, 0), offsets(pl.nb + 1), cursor(pl.nb, 0), sorted(n * pl.windows + 1);
     std::vector<uint32_t> bucket_sum(32 * (size_t)pl.nb), heads(32 * nthreads + 32), tails(32 * nthreads + 32), partial(32 * (size_t)pl.windows * groups);
@@ -480,5 +481,9 @@ int emu_msm(uint8_t* out, size_t n, const uint8_t* scalars, const uint8_t* point
     ge_compress(o, tot);
     st(out, o, 8);
     return (int)bad;
+}
+int emu_msm(uint8_t* out, size_t n, const uint8_t* scalars, const uint8_t* points, int c_override, int k_override)
+{
+    return emu_msm_plan(out, n, scalars, points, c_override, k_override, 0);
 }
 }
