@@ -176,6 +176,22 @@ int  kb_keyset_verify_batch(kb_keyset* ks, size_t n, const uint32_t* key_idx, co
  * for that item, and the kernel reads nothing of the key set for it. */
 int  kb_dev_keyset_verify(kb_keyset* ks, size_t n, const void* d_key_idx, const void* d_msg, const void* d_msg_off,
                           const void* d_sig, void* d_status, int schnorr, void* stream);
+/* out[i] = compress(scalars[i] * keys[key_idx[i]]): Point::mul(s, Some(p)) with a registered p (point.rs:207,
+ * ge.rs:508), the Diffie-Hellman step dh_exchange(secret, remote_public) (dh/dh_impl.rs:74-80) of encrypted_deal and
+ * ECIES.  out and status are byte for byte what kb_point_mul_batch(ctx, n, scalars, keys[key_idx], out, status, flags)
+ * returns, for every scalar (never reduced, also >= 2^255) and every key: status[i] = 1 and out[i] = 0 when the key does
+ * not decode (status may be NULL).  A key with a comb needs no doublings: each of the 64 signed radix-16 windows selects
+ * among 8 entries of its comb and adds once (constant-time select unless KB_FLAG_VARTIME); the other keys take the path
+ * of kb_point_mul_batch.  The constant-time select reads 8 comb entries per window: with secret scalars under tens of
+ * thousands of keys that traffic outweighs the saved work (DESIGN.md section 3.8).  flags: 0 or KB_FLAG_VARTIME, anything else is KB_ERR_ARG.  KB_ERR_ARG if any key_idx[i] >=
+ * nkeys (checked before anything is launched).  Unless KB_FLAG_VARTIME is set, the scalars staged in device scratch
+ * are zeroed before the call returns. */
+int  kb_keyset_mul_batch(kb_keyset* ks, size_t n, const uint32_t* key_idx, const uint8_t* scalars, uint8_t* out,
+                         uint8_t* status, uint32_t flags);
+/* device buffers + stream, ordered like every kb_dev_* call of the context.  An index >= nkeys gives status 0xFF and
+ * out[i] = 0 for that item, and the kernel reads nothing of the key set for it. */
+int  kb_dev_keyset_mul(kb_keyset* ks, size_t n, const void* d_key_idx, const void* d_scalars, void* d_out, void* d_status,
+                       uint32_t flags, void* stream);
 
 /* EdDSA::sign (sign/eddsa/eddsa_sig.rs:120-152) for n (seed, message) pairs, with the key derivation of
  * Curve::new_key_and_seed_with_input (group/edwards25519/curve.rs:74-87): a = clamp(SHA-512(seed)[0..32]),
@@ -357,6 +373,10 @@ void kb_mctx_keyset_destroy(kb_mkeyset* ks);
  * (KB_ERR_ARG); each device copies only the message bytes of its own items. */
 int  kb_mctx_keyset_verify_batch(kb_mkeyset* ks, size_t n, const uint32_t* key_idx, const uint8_t* msg, const uint64_t* msg_off,
                                  const uint8_t* sig, uint8_t* status, int schnorr);
+/* kb_keyset_mul_batch split by index over all devices, each against its own copy of the key set.  Flags and every key
+ * index are checked before any device starts (KB_ERR_ARG). */
+int  kb_mctx_keyset_mul_batch(kb_mkeyset* ks, size_t n, const uint32_t* key_idx, const uint8_t* scalars, uint8_t* out,
+                              uint8_t* status, uint32_t flags);
 /* kb_dkg_process_round_keyed for ndealers dealers split by dealer (arrays whole, as kb_mctx_dkg_process_round has them):
  * each device runs its dealer range against its own copy of the key sets. */
 int  kb_mctx_dkg_process_round_keyed(kb_mctx* m, const kb_mkeyset* dealers, const kb_mkeyset* verifiers, size_t n, size_t t, size_t ndealers, int fmt,

@@ -47,6 +47,7 @@ EXPORTS = [
     "kb_keyset_create", "kb_keyset_destroy", "kb_keyset_verify_batch", "kb_dev_keyset_verify",
     "kb_dkg_process_round_keyed", "kb_dev_dkg_process_round_keyed",
     "kb_mctx_keyset_create", "kb_mctx_keyset_destroy", "kb_mctx_keyset_verify_batch", "kb_mctx_dkg_process_round_keyed",
+    "kb_keyset_mul_batch", "kb_dev_keyset_mul", "kb_mctx_keyset_mul_batch",
 ]
 
 
@@ -139,12 +140,15 @@ def load_library(path: str = LIB_PATH):
     L.kb_keyset_destroy.restype = None
     L.kb_keyset_verify_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32]
     L.kb_dev_keyset_verify.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32, vp]
+    L.kb_keyset_mul_batch.argtypes = [vp, sz, vp, vp, vp, vp, u32]
+    L.kb_dev_keyset_mul.argtypes = [vp, sz, vp, vp, vp, vp, u32, vp]
     L.kb_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8
     L.kb_dev_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8 + [vp]
     L.kb_mctx_keyset_create.argtypes = [vp, sz, vp, ctypes.POINTER(vp)]
     L.kb_mctx_keyset_destroy.argtypes = [vp]
     L.kb_mctx_keyset_destroy.restype = None
     L.kb_mctx_keyset_verify_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32]
+    L.kb_mctx_keyset_mul_batch.argtypes = [vp, sz, vp, vp, vp, vp, u32]
     L.kb_mctx_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8
     _LIB = L
     return L
@@ -689,6 +693,25 @@ class KeySet:
         dp = Context._dp
         self.ctx._check(self.L.kb_dev_keyset_verify(self.h, n, dp(key_idx), dp(msg), dp(msg_off), dp(sig), dp(status), int(schnorr), Context._stream()), "kb_dev_keyset_verify")
 
+    def mul_batch(self, key_idx, scalars, flags=0):
+        """(out, status) = Context.point_mul_batch(scalars, keys[key_idx], flags) byte for byte, from the keys' combs:
+        Point::mul(s, Some(pk)) of dh_exchange.  flags: 0 or FLAG_VARTIME."""
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        s = _u8(scalars, (-1, 32))
+        n = key_idx.shape[0]
+        if s.shape[0] != n:
+            raise ValueError("KeySet.mul_batch: one key index per scalar")
+        out = np.empty_like(s)
+        st = np.empty(n, dtype=np.uint8)
+        self.ctx._check(self.L.kb_keyset_mul_batch(self.h, n, _ptr(key_idx), _ptr(s), _ptr(out), _ptr(st), flags), "kb_keyset_mul_batch")
+        return out, st
+
+    def dev_mul(self, n, key_idx, scalars, out, status, flags=0):
+        """key_idx: n uint32 (torch int32 tensor), scalars / out n x 32 bytes, status n bytes (or None) on the device, on torch's
+        current stream; an index outside the set gives status 0xFF and 32 zero bytes."""
+        dp = Context._dp
+        self.ctx._check(self.L.kb_dev_keyset_mul(self.h, n, dp(key_idx), dp(scalars), dp(out), dp(status), flags, Context._stream()), "kb_dev_keyset_mul")
+
 
 class MultiContext:
     """One kb_mctx: the GPUs `devices` of this box driven from one process; every call takes the whole host batch."""
@@ -842,3 +865,15 @@ class MultiKeySet:
         st = out if out is not None else np.empty(n, dtype=np.uint8)
         self.mctx._check(self.L.kb_mctx_keyset_verify_batch(self.h, n, _ptr(key_idx), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(st), int(schnorr)), "kb_mctx_keyset_verify_batch")
         return st
+
+    def mul_batch(self, key_idx, scalars, flags=0):
+        """KeySet.mul_batch split by index over the devices."""
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        s = _u8(scalars, (-1, 32))
+        n = key_idx.shape[0]
+        if s.shape[0] != n:
+            raise ValueError("MultiKeySet.mul_batch: one key index per scalar")
+        out = np.empty_like(s)
+        st = np.empty(n, dtype=np.uint8)
+        self.mctx._check(self.L.kb_mctx_keyset_mul_batch(self.h, n, _ptr(key_idx), _ptr(s), _ptr(out), _ptr(st), flags), "kb_mctx_keyset_mul_batch")
+        return out, st

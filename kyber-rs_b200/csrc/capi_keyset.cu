@@ -193,6 +193,63 @@ int kb_keyset_verify_batch(kb_keyset* ks, size_t n, const uint32_t* key_idx, con
     return KB_OK;
 }
 
+// ---- Point::mul(s, Some(keys[key_idx[i]])): k_keyset_mul, then the batch compression of kb_dev_point_mul
+int kb_dev_keyset_mul(kb_keyset* ks, size_t n, const void* d_key_idx, const void* d_scalars, void* d_out, void* d_status, uint32_t flags, void* stream)
+{
+    if (!ks) return KB_ERR_ARG;
+    kb_ctx* ctx = ks->ctx;
+    if ((flags & ~KB_FLAG_VARTIME) || (n && (!d_key_idx || !d_scalars || !d_out))) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    KB_DEV_ENTER(st);
+    uint32_t* xyz;
+    uint8_t* bad = (uint8_t*)d_status;
+    KB_SCRATCH(KB_SLOT_XYZ, 96 * n, xyz);
+    if (!bad) KB_SCRATCH(KB_SLOT_FLAGS, n, bad);
+    const unsigned th = kb_item_threads(ctx, n);
+    const uint32_t* idx = (const uint32_t*)d_key_idx;
+    const uint8_t* sc = (const uint8_t*)d_scalars;
+    if (flags & KB_FLAG_VARTIME)
+        k_keyset_mul<false><<<kb_blocks(n, th), th, 0, st>>>(n, idx, ks->nkeys, ks->pk, ks->facts, ks->table, sc, xyz, bad);
+    else
+        k_keyset_mul<true><<<kb_blocks(n, th), th, 0, st>>>(n, idx, ks->nkeys, ks->pk, ks->facts, ks->table, sc, xyz, bad);
+    KB_LAUNCHED();
+    k_compress_batch<<<kb_blocks((n + KB_INV_K - 1) / KB_INV_K, KB_THREADS), KB_THREADS, 0, st>>>(n, xyz, bad, (uint8_t*)d_out);
+    KB_LAUNCHED();
+    KB_DEV_RETURN(st, KB_OK);
+}
+// plain staging as kb_point_mul_batch: copy in, the two launches, copy out, all on the context's stream
+int kb_keyset_mul_batch(kb_keyset* ks, size_t n, const uint32_t* key_idx, const uint8_t* scalars, uint8_t* out, uint8_t* status, uint32_t flags)
+{
+    if (!ks) return KB_ERR_ARG;
+    kb_ctx* ctx = ks->ctx;
+    KB_ENTER();
+    if ((flags & ~KB_FLAG_VARTIME) || (n && (!key_idx || !scalars || !out))) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    uint32_t over = 0;
+    for (size_t i = 0; i < n; i++) over |= (uint32_t)(key_idx[i] >= ks->nkeys);
+    if (over) return KB_ERR_ARG;
+    uint8_t *d_s, *d_o, *d_st;
+    uint32_t* d_idx;
+    KB_SCRATCH(0, 32 * n, d_s);
+    KB_SCRATCH(1, 32 * n, d_o);
+    KB_SCRATCH(2, 4 * n, d_idx);
+    KB_SCRATCH(3, n, d_st);
+    KB_H2D(d_s, scalars, 32 * n);
+    KB_H2D(d_idx, key_idx, 4 * n);
+    const int rc = kb_dev_keyset_mul(ks, n, d_idx, d_s, d_o, d_st, flags, ctx->stream);
+    // scalars that are not declared public (KB_FLAG_VARTIME) do not outlive the call in device scratch
+    if (!(flags & KB_FLAG_VARTIME)) KB_CUDA(cudaMemsetAsync(d_s, 0, 32 * n, ctx->stream));
+    if (rc != KB_OK) {
+        cudaStreamSynchronize(ctx->stream);
+        return rc;
+    }
+    KB_D2H(out, d_o, 32 * n);
+    if (status) KB_D2H(status, d_st, n);
+    KB_SYNC();
+    return KB_OK;
+}
+
 int kb_dev_dkg_process_round_keyed(kb_ctx* ctx, const kb_keyset* dealers, const kb_keyset* verifiers, size_t n, size_t t, size_t dealer_lo, size_t ndealers, int fmt, const void* d_commits,
                                    const void* d_shares, void* d_verdict, const void* d_deal_msg, const void* d_deal_msg_off, const void* d_deal_sig, void* d_deal_status,
                                    const void* d_resp_msg, const void* d_resp_msg_off, const void* d_resp_sig, void* d_resp_status, void* stream)

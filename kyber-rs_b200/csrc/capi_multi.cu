@@ -249,6 +249,21 @@ int kb_mctx_keyset_verify_batch(kb_mkeyset* mk, size_t n, const uint32_t* key_id
         return rc;
     });
 }
+int kb_mctx_keyset_mul_batch(kb_mkeyset* mk, size_t n, const uint32_t* key_idx, const uint8_t* scalars, uint8_t* out, uint8_t* status, uint32_t flags)
+{
+    if (!mk || (flags & ~KB_FLAG_VARTIME) || (n && (!key_idx || !scalars || !out))) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    uint32_t over = 0;
+    for (size_t i = 0; i < n; i++) over |= (uint32_t)(key_idx[i] >= mk->nkeys);
+    if (over) return KB_ERR_ARG;
+    kb_mctx* m = mk->m;
+    return kb_on_all(m, [&](int i) {
+        size_t lo, hi;
+        kb_shard(n, i, m->ndev, &lo, &hi);
+        if (hi == lo) return (int)KB_OK;
+        return kb_keyset_mul_batch(mk->ks[i], hi - lo, key_idx + lo, scalars + 32 * lo, out + 32 * lo, status ? status + lo : nullptr, flags);
+    });
+}
 int kb_mctx_dkg_process_round_keyed(kb_mctx* m, const kb_mkeyset* dealers, const kb_mkeyset* verifiers, size_t n, size_t t, size_t ndealers, int fmt,
                                     const void* commits, const uint8_t* shares, uint8_t* verdict,
                                     const uint8_t* deal_msg, const uint64_t* deal_msg_off, const uint8_t* deal_sig, uint8_t* deal_status,

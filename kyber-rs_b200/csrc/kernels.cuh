@@ -581,6 +581,31 @@ static __global__ void __launch_bounds__(KB_THREADS) k_keyset_verify_round(size_
     kb_store_xyz(xyz, i, Q);
     flags[i] = (uint8_t)f;
 }
+// ---- Point::mul(s, Some(A)) for registered keys: item i = scalars[i] * keys[key_idx[i]] (ops.cuh kb_keyset_mul_one), (X, Y, Z)
+// in the layout of k_mul for k_compress_batch with status as its `bad` array.  An index outside the key set reads nothing of
+// it and gives the identity with status 0xFF.  No block barrier: items of one block take different paths.
+template <bool CT>
+static __global__ void __launch_bounds__(KB_THREADS) k_keyset_mul(size_t n, const uint32_t* key_idx, size_t nkeys, const uint8_t* kpk, const uint8_t* facts, const ge_precomp* ktab,
+                                                                  const uint8_t* scalars, uint32_t* xyz, uint8_t* status)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t k = __ldg(key_idx + i);
+    ge_p3 h;
+    uint32_t st = 0xFF;
+    if (k < nkeys) {
+        uint32_t s[8], pw[8];
+        int8_t e[64];
+        kb_load32(s, scalars, i);
+        kb_load32(pw, kpk, k);
+        sc_recode16(e, s);
+        st = kb_keyset_mul_one<CT>(h, __ldg(facts + k), pw, e, ktab + (size_t)k * KB_KEY_ENTRIES);
+    } else {
+        ge_identity(h);
+    }
+    kb_store_xyz(xyz, i, h);
+    status[i] = (uint8_t)st;
+}
 #endif  // KB_K_KEYSET
 
 // ---- the same verifiers with half-size scalars (ops.cuh sig_half_*, half.cuh): 128 doublings per signature,

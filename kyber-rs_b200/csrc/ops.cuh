@@ -135,8 +135,9 @@ KB_FN void ge_build_table8(ge_cached* tbl, const ge_p3& p)
 #define KB_LOCKSTEP() __syncthreads()
 #endif
 // h = a * P, ge_scalar_mult (ge.rs:508-568): signed radix-16 fixed window over the
-// per-thread table tbl[8]; e = sc_recode16(a).
-template <bool CT>
+// per-thread table tbl[8]; e = sc_recode16(a).  LOCKSTEP = false drops the block barrier, for callers
+// that run it in a divergent branch (k_keyset_mul).
+template <bool CT, bool LOCKSTEP = true>
 KB_FN void ge_scalarmult(ge_p3& h, const int8_t* e, const ge_cached* tbl)
 {
     ge_cached c;
@@ -145,7 +146,7 @@ KB_FN void ge_scalarmult(ge_p3& h, const int8_t* e, const ge_cached* tbl)
     // enough for the instruction cache
     KB_NOUNROLL
     for (int i = 63; i >= 0; i--) {
-        KB_LOCKSTEP();
+        if (LOCKSTEP) { KB_LOCKSTEP(); }
         if (i != 63) {
             KB_NOUNROLL
             for (int k = 0; k < 4; k++) ge_dbl_rt(h, h, k == 3);
@@ -1060,4 +1061,74 @@ KB_FN uint32_t sig_keyset_stage1(ge_p3& Q, uint32_t kf, const uint32_t* pk_w, co
     }
     ge_keyset_scalarmult(Q, dw, nd, comb, ktab);
     return fast ? (f | KB_F_FAST) : f;
+}
+
+// ---------------------------------------------------------------------------------------
+// key sets: scalar multiplication of a registered key, Point::mul(s, Some(A)) (kb_keyset_mul_*, capi_keyset.cu)
+// ---------------------------------------------------------------------------------------
+// The key comb already holds every entry of a signed radix-16 comb over A: window w needs (j+1) * 16^w * A, j = 0..7, and
+// 16^w = 2^(KB_KEY_BITS p) * 16^(w & 1) with p = w / 2, so that is kt[p][j] for an even w and kt[p][16 j + 15] for an odd
+// one.  s*A is then 64 mixed additions like ge_scalarmult_base: no doublings, no decompression, no per-thread table.
+static_assert(KB_KEY_BITS == 8, "two radix-16 windows per key-comb position");
+
+// ge_select_precomp over the entries row[j * stride], j = 0..7 (stride 1 or 16, public).  CT=true reads all 8 entries and
+// keeps the hit with conditional moves (no digit-dependent address or branch); CT=false loads the one it needs.
+template <bool CT>
+KB_FN void ge_select_precomp_strided(ge_precomp& c, const ge_precomp* row, int stride, int d)
+{
+    const uint32_t neg = (uint32_t)d >> 31;
+    const int babs = (d ^ -(int)neg) + (int)neg;
+    ge_precomp_identity(c);
+    ge_cached t;
+    if (CT) {
+        KB_NOUNROLL
+        for (int j = 0; j < 8; j++) {
+            const uint32_t hit = (uint32_t)(babs == j + 1);
+            kb_ld_precomp(t, row + (size_t)j * stride);
+            fe_cmov(c.ypx, t.YpX, hit);
+            fe_cmov(c.ymx, t.YmX, hit);
+            fe_cmov(c.xy2d, t.T2d, hit);
+        }
+    } else if (babs != 0) {
+        kb_ld_precomp(t, row + (size_t)(babs - 1) * stride);
+        c.ypx = t.YpX;
+        c.ymx = t.YmX;
+        c.xy2d = t.T2d;
+    }
+    ge_precomp_cneg(c, neg);
+}
+// h = a * A from the key comb kt of A, e = sc_recode16(a): the sum of e[w] * 16^w * A over the 64 windows, which is the
+// group element ge_scalarmult gives for the same digits (the comb's multiples are exact, never reduced mod L).
+template <bool CT>
+KB_FN void ge_keyset_mul(ge_p3& h, const int8_t* e, const ge_precomp* ktab)
+{
+    ge_precomp c;
+    ge_identity(h);
+    KB_NOUNROLL
+    for (int w = 0; w < 64; w++) {
+        const int odd = w & 1;
+        ge_select_precomp_strided<CT>(c, ktab + (size_t)(w >> 1) * KB_KEY_HALF + (odd ? 15 : 0), odd ? 16 : 1, e[w]);
+        ge_madd<true>(h, h, c);
+    }
+}
+// One item: h = a * A for the registered key with facts kf (kb_key_facts), bytes pk_w and comb kt.  A key without a real
+// comb (small order, not canonical or not decodable: its comb holds identities) takes the path of k_mul instead, without
+// the block barrier; the key is public, so the branch is too.  Returns k_mul's status: 1 (and the identity) when the key
+// does not decode.
+template <bool CT>
+KB_FN uint32_t kb_keyset_mul_one(ge_p3& h, uint32_t kf, const uint32_t* pk_w, const int8_t* e, const ge_precomp* kt)
+{
+    if ((kf & (KB_F_AC | KB_F_AS | KB_F_AOK)) == (KB_F_AC | KB_F_AOK)) {
+        ge_keyset_mul<CT>(h, e, kt);
+        return 0;
+    }
+    ge_p3 p;
+    if (!ge_decompress(p, pk_w)) {
+        ge_identity(h);
+        return 1;
+    }
+    ge_cached tbl[8];
+    ge_build_table8(tbl, p);
+    ge_scalarmult<CT, false>(h, e, tbl);
+    return 0;
 }

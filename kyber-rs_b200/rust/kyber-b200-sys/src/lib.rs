@@ -66,6 +66,8 @@ extern "C" {
     pub fn kb_keyset_destroy(ks: *mut kb_keyset);
     pub fn kb_keyset_verify_batch(ks: *mut kb_keyset, n: usize, key_idx: *const u32, msg: *const u8, msg_off: *const u64, sig: *const u8, status: *mut u8, schnorr: c_int) -> c_int;
     pub fn kb_dev_keyset_verify(ks: *mut kb_keyset, n: usize, d_key_idx: *const c_void, d_msg: *const c_void, d_msg_off: *const c_void, d_sig: *const c_void, d_status: *mut c_void, schnorr: c_int, stream: *mut c_void) -> c_int;
+    pub fn kb_keyset_mul_batch(ks: *mut kb_keyset, n: usize, key_idx: *const u32, scalars: *const u8, out: *mut u8, status: *mut u8, flags: u32) -> c_int;
+    pub fn kb_dev_keyset_mul(ks: *mut kb_keyset, n: usize, d_key_idx: *const c_void, d_scalars: *const c_void, d_out: *mut c_void, d_status: *mut c_void, flags: u32, stream: *mut c_void) -> c_int;
 
     pub fn kb_eddsa_sign_batch(ctx: *mut kb_ctx, n: usize, seeds: *const u8, msg: *const u8, msg_off: *const u64, sig: *mut u8, pk: *mut u8) -> c_int;
 
@@ -133,6 +135,7 @@ extern "C" {
     pub fn kb_mctx_keyset_create(m: *mut kb_mctx, nkeys: usize, pk: *const u8, out: *mut *mut kb_mkeyset) -> c_int;
     pub fn kb_mctx_keyset_destroy(ks: *mut kb_mkeyset);
     pub fn kb_mctx_keyset_verify_batch(ks: *mut kb_mkeyset, n: usize, key_idx: *const u32, msg: *const u8, msg_off: *const u64, sig: *const u8, status: *mut u8, schnorr: c_int) -> c_int;
+    pub fn kb_mctx_keyset_mul_batch(ks: *mut kb_mkeyset, n: usize, key_idx: *const u32, scalars: *const u8, out: *mut u8, status: *mut u8, flags: u32) -> c_int;
     pub fn kb_mctx_dkg_process_round_keyed(m: *mut kb_mctx, dealers: *const kb_mkeyset, verifiers: *const kb_mkeyset, n: usize, t: usize, ndealers: usize, fmt: c_int,
         commits: *const c_void, shares: *const u8, verdict: *mut u8,
         deal_msg: *const u8, deal_msg_off: *const u64, deal_sig: *const u8, deal_status: *mut u8,

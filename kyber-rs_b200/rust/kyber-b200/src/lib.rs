@@ -192,6 +192,27 @@ impl<'a> KeySet<'a> {
         }
         Ok(res.into_iter().map(|r| r.unwrap()).collect())
     }
+    /// Batch companion of `Point::mul(s, Some(pk))` for registered keys — the `dh_exchange(secret, remote_public)` step
+    /// (dh/dh_impl.rs:74-80) of `encrypted_deal` and ECIES.  Items are (key index, scalar); the result is what
+    /// `BatchPoint::mul_batch` returns for the same key bytes, from the keys' combs.  The scalars are secret: the table
+    /// select is constant-time.  A key index outside the set is `GpuError::Arg`, a key that does not decode
+    /// `GpuError::InvalidPoint`.
+    pub fn mul_batch(&self, items: &[(u32, EdScalar)]) -> Result<Vec<EdPoint>, GpuError> {
+        if items.iter().any(|(k, _)| *k as usize >= self.nkeys) {
+            return Err(GpuError::Arg);
+        }
+        let n = items.len();
+        let key_idx: Vec<u32> = items.iter().map(|(k, _)| *k).collect();
+        let scalars: Vec<EdScalar> = items.iter().map(|(_, s)| s.clone()).collect();
+        let s = pack_scalars(&scalars);
+        let mut out = vec![0u8; 32 * n];
+        let mut st = vec![0u8; n];
+        self.gpu.check(unsafe { sys::kb_keyset_mul_batch(self.ks, n, key_idx.as_ptr(), s.as_ptr(), out.as_mut_ptr(), st.as_mut_ptr(), 0) })?;
+        if let Some(i) = st.iter().position(|&x| x != 0) {
+            return Err(GpuError::InvalidPoint(i));
+        }
+        Ok(unpack_points(&out))
+    }
 }
 impl Drop for KeySet<'_> {
     fn drop(&mut self) {
