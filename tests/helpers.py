@@ -241,6 +241,30 @@ def load_c_oracle():
 
 
 L_ORDER = 2**252 + 27742317777372353535851937790883648493
+P_FIELD = 2**255 - 19
+
+# field elements (8 x 32-bit limbs, any value below 2^256) at the carry and wrap edges of the limb arithmetic
+FE_EDGE = [0, 1, 2, 19, 38, P_FIELD - 1, P_FIELD, P_FIELD + 1, 2**255 - 1, 2**255, 2**255 + 18, 2**255 + 19, 2**256 - 1, 2**256 - 38, 2**256 - 39, 2**256 - 19,
+           2**256 - 2**32, 2**224 - 1]
+
+
+def half_step_special_inputs():
+    """Challenges on which the lattice step sc_half (csrc/half.cuh) is hardest: rationals k/m of 8L (short vectors with
+    tiny u, the Lehmer batches' awkward cases), powers of two and their small multiples, Fibonacci numbers (all
+    quotients 1), and a few hand-picked values."""
+    L = L_ORDER
+    N = 8 * L
+    special = [0, 1, 2, 3, 7, 8, L - 1, L - 2, L // 2, L // 3, 2**128, 2**127 + 1, 2**64, 2**200 + 5, (N // 3) % L, (N // 5 + 1) % L]
+    for m in range(1, 400):
+        for k in (1, 2, m // 2 + 1, m - 1):
+            for d in (-2, -1, 0, 1, 2, 2**64, 2**128 + 1):
+                special.append(((N * k) // m + d) % L)
+    special += [(mul << e) % L for e in range(1, 253, 3) for mul in (1, 3, 5)]
+    fa, fb = 1, 1
+    while fb < L:
+        special.append(fb)
+        fa, fb = fb, fa + fb
+    return special
 
 
 def xof_bytes(seed: str, n: int) -> bytes:

@@ -1,7 +1,8 @@
 """Host emulation of the per-thread device math (tests/emu/emu.cpp compiles the SAME headers the
 GPU kernels inline, with KB_HOST_EMU) against the oracles.  CPU only.  This is how the field /
 curve / scalar / hash / verify / Pippenger logic is checked on a machine with no GPU; the PTX
-carry-chain primitives themselves are covered by the -m gpu tests."""
+carry-chain primitives themselves are tested on the device, at their carry and wrap edges and bit
+for bit against this host build, by tests/test_gpu_field_edges.py."""
 import ctypes
 import hashlib
 import os
@@ -11,7 +12,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from helpers import ROOT, load_c_oracle, load_sign_input, make_mixed_order_sigs, make_sig_batch
+from helpers import FE_EDGE, ROOT, half_step_special_inputs, load_c_oracle, load_sign_input, make_mixed_order_sigs, make_sig_batch
 from oracle import ed25519_bigint as O
 
 P = O.P
@@ -49,7 +50,7 @@ def test_field_ops(emu):
         return out.raw
 
     rnd = random.Random(7)
-    edge = [0, 1, 2, 19, 38, P - 1, P, P + 1, 2**255 - 1, 2**255, 2**255 + 18, 2**255 + 19, 2**256 - 1, 2**256 - 38, 2**256 - 39, 2**256 - 19, 2**256 - 2**32, 2**224 - 1]
+    edge = list(FE_EDGE)
     vals = edge + [rnd.getrandbits(256) for _ in range(150)]
     for x in vals:
         for y in rnd.sample(vals, 8) + edge[:8]:
@@ -169,18 +170,7 @@ def test_half_size_lattice_step(emu):
     rnd = random.Random(23)
     out = ctypes.create_string_buffer(64)
     N = 8 * O.L
-    special = [0, 1, 2, 3, 7, 8, O.L - 1, O.L - 2, O.L // 2, O.L // 3, 2**128, 2**127 + 1, 2**64, 2**200 + 5, (N // 3) % O.L, (N // 5 + 1) % O.L]
-    # rationals k/m of the modulus (short vectors with tiny u, the Lehmer batches' awkward cases), powers of two,
-    # Fibonacci numbers (all quotients 1)
-    for m in range(1, 400):
-        for k in (1, 2, m // 2 + 1, m - 1):
-            for d in (-2, -1, 0, 1, 2, 2**64, 2**128 + 1):
-                special.append(((N * k) // m + d) % O.L)
-    special += [(mul << e) % O.L for e in range(1, 253, 3) for mul in (1, 3, 5)]
-    fa, fb = 1, 1
-    while fb < O.L:
-        special.append(fb)
-        fa, fb = fb, fa + fb
+    special = half_step_special_inputs()
     worst = 0
     for k in range(len(special) + 20000):
         h = special[k] if k < len(special) else rnd.randrange(O.L)
