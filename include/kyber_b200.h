@@ -38,6 +38,8 @@ extern "C" {
 /* Environment switches read once by kb_ctx_create (tests, tuning and A/B measurements; none changes a result):
  *   KB_VERIFY_FULL=1          signature verifiers: the full-length (253-doubling) kernels instead of the half-size-scalar ones
  *   KB_VERIFY_MIN_WINDOWS=k   half-size-scalar verifier: lower bound on the block-uniform window count (tests)
+ *   KB_VERIFY_FORCE_REDO=k    half-size-scalar verifier: every k-th thread of the main kernel redoes its table and loop with
+ *                             the exact field arithmetic, as a thread whose short-wrap counter was raised does (tests)
  *   KB_VERIFY_CHUNK=n         host-buffer verify calls: largest pipelined chunk in signatures (default: 16 waves of the main
  *                             kernel = 16 x SMs x 512; the chunks grow x4 from a third of a wave up to this cap)
  *   KB_VERIFY_CHUNK_LOG2=k    the same cap as a power of two

@@ -122,6 +122,9 @@ int kb_ctx_create(int device, kb_ctx** out)
         const char* vw = getenv("KB_VERIFY_MIN_WINDOWS");
         const int vwn = vw ? atoi(vw) : 0;
         ctx->verify_min_windows = (vwn > KB_HALF_MIN_WINDOWS && vwn <= 64) ? vwn : KB_HALF_MIN_WINDOWS;
+        const char* vr = getenv("KB_VERIFY_FORCE_REDO");
+        const int vrn = vr ? atoi(vr) : 0;
+        ctx->verify_force_redo = (vrn > 0 && vrn <= 1024) ? vrn : 0;
         ok = ok && cudaStreamSynchronize(ctx->stream) == cudaSuccess && cudaGetLastError() == cudaSuccess;
     }
     if (!ok) {

@@ -65,8 +65,8 @@ int kb_verify_launch(kb_ctx* ctx, size_t n, const uint8_t* d_pk, const uint8_t* 
             perm = pm;
         }
 #endif
-        if (schnorr) k_verify_half_main<true><<<g1, th, 0, st>>>(n, xyz, perm, d_status, ctx->comb, ctx->verify_min_windows);
-        else k_verify_half_main<false><<<g1, th, 0, st>>>(n, xyz, perm, d_status, ctx->comb, ctx->verify_min_windows);
+        if (schnorr) k_verify_half_main<true><<<g1, th, 0, st>>>(n, xyz, perm, d_status, ctx->comb, ctx->verify_min_windows, ctx->verify_force_redo);
+        else k_verify_half_main<false><<<g1, th, 0, st>>>(n, xyz, perm, d_status, ctx->comb, ctx->verify_min_windows, ctx->verify_force_redo);
         KB_LAUNCHED();
         if (tm) {
             cudaEventRecord(ctx->tev[2], st);

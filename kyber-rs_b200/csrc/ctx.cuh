@@ -32,6 +32,7 @@ struct kb_ctx {
     int fd_steps_wide, fd_steps_minb;   // KB_FD_STEPS_WIDE / KB_FD_STEPS_MINB: variants of the step kernel (tuning)
     int fd_parts;            // KB_FD_PARTS: number of coefficient blocks of the forward-difference round (0 = by cost)
     int verify_min_windows;  // KB_VERIFY_MIN_WINDOWS (tests): lower bound on the block-uniform window count of k_verify_half_main
+    int verify_force_redo;   // KB_VERIFY_FORCE_REDO=k (tests): every k-th thread of k_verify_half_main redoes its record with the exact field bodies
     // KB_VERIFY_SPLIT: the preparation of the half-size-scalar verifiers as TWO kernels that share the SMs (capi_verify.cu):
     // a persistent ALU-bound "scalars" kernel (vs_blocks blocks per SM) beside the multiplier-bound "points" kernel
     int verify_split, vs_blocks, vs_pbound;

@@ -848,7 +848,8 @@ KB_FN void fe_reduce512_shift(fe& r, const uint32_t* t)
     uint32_t c = kb_add_small(r.v, w8 * 38u);
     r.v[0] += 38u * c;
 }
-KB_FN void fe_reduce512_mul(fe& r, uint32_t* t)
+// the fold of fe_reduce512_mul: r[0..8) + 2^256 * (returned word, < 2^7) = t[0..16) (mod p)
+KB_FN uint32_t fe_reduce512_fold(fe& r, uint32_t* t)
 {
     // even high words: (t0..t7) += 38 * {t8,t10,t12,t14}, carry into r8
     uint32_t r8;
@@ -870,7 +871,12 @@ KB_FN void fe_reduce512_mul(fe& r, uint32_t* t)
     r.v[0] = t[0];
     KB_UNROLL
     for (int k = 0; k < 7; k++) r.v[k + 1] = hi[k];
-    uint32_t c = kb_add_small(r.v, hi[7] * 38u);
+    return hi[7];
+}
+KB_FN void fe_reduce512_mul(fe& r, uint32_t* t)
+{
+    const uint32_t top = fe_reduce512_fold(r, t);
+    uint32_t c = kb_add_small(r.v, top * 38u);
     // a second wrap leaves a value < 38*2^7, so adding 38 once more cannot carry
     r.v[0] += 38u * c;
 }
@@ -883,10 +889,10 @@ KB_FN void fe_reduce512(fe& r, uint32_t* t)
 #endif
 }
 
-// h = f * g   (fe.rs:299 fe_mul), rows in natural order
-KB_FN void fe_mul_rows(fe& h, const fe& f, const fe& g)
+// ev[0..16) = f * g (ev has room for 17 words), rows in natural order
+KB_FN void fe_mul_rows_wide(uint32_t* ev, const fe& f, const fe& g)
 {
-    uint32_t ev[17], od[16];
+    uint32_t od[16];
     const uint32_t* a = f.v;
     const uint32_t* b = g.v;
     // Operand scanning over b; products a[j]*b[i] with i+j even accumulate in ev (word i+j),
@@ -913,13 +919,19 @@ KB_FN void fe_mul_rows(fe& h, const fe& f, const fe& g)
     kb_cmad4_hi(&ev[8], a[1], a[3], a[5], a[7], b[7]);
     kb_cmad4_top(&od[6], a[0], a[2], a[4], a[6], b[7], od[14]);
     kb_acc15(&ev[1], &od[0]);
+}
+// h = f * g   (fe.rs:299 fe_mul), rows in natural order
+KB_FN void fe_mul_rows(fe& h, const fe& f, const fe& g)
+{
+    uint32_t ev[17];
+    fe_mul_rows_wide(ev, f, g);
     fe_reduce512(h, ev);
 }
 
-// h = f * g, rows ordered so that no register has to be zeroed (see kb_cmad4_new / kb_cmad4_rip)
-KB_FN void fe_mul_rip(fe& h, const fe& f, const fe& g)
+// ev[0..16) = f * g, rows ordered so that no register has to be zeroed (see kb_cmad4_new / kb_cmad4_rip)
+KB_FN void fe_mul_rip_wide(uint32_t* ev, const fe& f, const fe& g)
 {
-    uint32_t ev[16], od[15];
+    uint32_t od[15];
     const uint32_t* a = f.v;
     const uint32_t* b = g.v;
     // Operand scanning over b; products a[j]*b[i] with i+j even accumulate in ev (word i+j),
@@ -946,13 +958,19 @@ KB_FN void fe_mul_rip(fe& h, const fe& f, const fe& g)
     kb_cmad4_rip(&ev[6], a[0], a[2], a[4], a[6], b[6], ev[14], ev[15]);
     kb_cmad4_top(&od[6], a[0], a[2], a[4], a[6], b[7], od[14]);           // words 7..14, carry -> word 15 (a plain word)
     kb_acc15(&ev[1], &od[0]);
+}
+// h = f * g, rows ordered so that no register has to be zeroed
+KB_FN void fe_mul_rip(fe& h, const fe& f, const fe& g)
+{
+    uint32_t ev[16];
+    fe_mul_rip_wide(ev, f, g);
     fe_reduce512(h, ev);
 }
 
-// h = f^2   (fe.rs:544 fe_square), rows in natural order: 28 cross products, doubled, plus 8 squares
-KB_FN void fe_sq_rows(fe& h, const fe& f)
+// ev[0..16) = f^2 (ev has room for 17 words), rows in natural order: 28 cross products, doubled, plus 8 squares
+KB_FN void fe_sq_rows_wide(uint32_t* ev, const fe& f)
 {
-    uint32_t ev[17], od[16];
+    uint32_t od[16];
     const uint32_t* a = f.v;
     // row i: a[j]*a[i] for j > i, word i+j; row 0 lands on fresh words (plain products, no zeroing, no carries)
     kb_cmul4(&od[0], a[1], a[3], a[5], a[7], a[0]);          // words 1,3,5,7
@@ -975,13 +993,19 @@ KB_FN void fe_sq_rows(fe& h, const fe& f)
     kb_acc15(&ev[1], &od[0]);
     kb_dbl16(ev);        // double the cross terms (top bit is clear: sum < 2^511)
     kb_sqr_acc8(ev, a);  // add the squares a[i]^2 on word pairs (2i, 2i+1)
+}
+// h = f^2   (fe.rs:544 fe_square), rows in natural order
+KB_FN void fe_sq_rows(fe& h, const fe& f)
+{
+    uint32_t ev[17];
+    fe_sq_rows_wide(ev, f);
     fe_reduce512(h, ev);
 }
 
-// h = f^2, rows ordered so that no register has to be zeroed: 28 cross products, doubled, plus 8 squares
-KB_FN void fe_sq_rip(fe& h, const fe& f)
+// t[0..16) = f^2, rows ordered so that no register has to be zeroed: 28 cross products, doubled, plus 8 squares
+KB_FN void fe_sq_rip_wide(uint32_t* t, const fe& f)
 {
-    uint32_t ev[16], od[14], t[16];
+    uint32_t ev[16], od[14];
     const uint32_t* a = f.v;
     // row i: a[j]*a[i] for j > i, word i+j; the rows are ordered as in fe_mul_inl — the row that opens a pair first
     // (or a plain product where nothing precedes it), the row below it ripples its carry in.  ev[0], ev[1], ev[14],
@@ -1001,6 +1025,12 @@ KB_FN void fe_sq_rip(fe& h, const fe& f)
     kb_cmad1_rip(&od[10], a[6], a[5], od[12], od[13]);               // word 11, carry -> 13, 14
     kb_sq_merge_dbl(t, ev, od);   // t[1..16) = doubled cross terms (sum < 2^511: the top bit is clear)
     kb_sqr_acc8_fresh0(t, a);     // add the squares a[i]^2 on word pairs (2i, 2i+1)
+}
+// h = f^2, rows ordered so that no register has to be zeroed
+KB_FN void fe_sq_rip(fe& h, const fe& f)
+{
+    uint32_t t[16];
+    fe_sq_rip_wide(t, f);
     fe_reduce512(h, t);
 }
 
@@ -1264,6 +1294,126 @@ KB_FN void fe_cmov(fe& f, const fe& g, uint32_t b)
     for (int i = 0; i < 8; i++) f.v[i] ^= m & (f.v[i] ^ g.v[i]);
 }
 KB_FN void fe_dbl(fe& h, const fe& f) { fe_add(h, f, f); }
+
+// ---------------------------------------------------------------------------------------
+// Short-wrap bodies, for code whose inputs are all public (the verifiers' k_verify_half_prep / k_verify_half_main).
+// Every body above ends by adding a small k (38 * carry, or 38 * the fold's top word < 38 * 2^7) into word 0 and
+// rippling the carry through all eight words, then wrapping a second time: one chain of 9 dependent instructions and
+// a multiply.  The carry leaves word 0 with probability below 2^-19.8 and word 1 below 2^-52, so the bodies below stop
+// the ripple at word 1 and ADD the carry (or borrow) out of word 1 to a per-thread counter `ovf` instead.
+//
+// Invariant: if `ovf` is still 0 after a sequence of short-wrap operations, every output equals the exact body's output
+// bit for bit (the exact ripple stops at word 1 as well, and its second wrap adds 38 * 0).  When it is not 0, the
+// caller recomputes with the exact bodies.  `ovf` counts: a few thousand operations per thread cannot wrap it around.
+// Nothing here is constant-time — the flag depends on the data.
+// ---------------------------------------------------------------------------------------
+// r[0..2) += k; the carry out of word 1 is added to ovf (words 2..7 are not touched)
+KB_FN void kb_add_small2(uint32_t* r, uint32_t k, uint32_t& ovf)
+{
+#if defined(KB_HOST_EMU)
+    uint64_t c = (uint64_t)r[0] + k;
+    r[0] = (uint32_t)c;
+    c = (c >> 32) + r[1];
+    r[1] = (uint32_t)c;
+    ovf += (uint32_t)(c >> 32);
+#else
+    asm("add.cc.u32 %0, %0, %3;\n\t"
+        "addc.cc.u32 %1, %1, 0;\n\t"
+        "addc.u32 %2, %2, 0;"
+        : "+r"(r[0]), "+r"(r[1]), "+r"(ovf)
+        : "r"(k));
+#endif
+}
+// r[0..2) -= k; the borrow out of word 1 is added to ovf (words 2..7 are not touched)
+KB_FN void kb_sub_small2(uint32_t* r, uint32_t k, uint32_t& ovf)
+{
+#if defined(KB_HOST_EMU)
+    uint64_t d = (uint64_t)r[0] - k;
+    r[0] = (uint32_t)d;
+    d = (uint64_t)r[1] - ((d >> 32) & 1u);
+    r[1] = (uint32_t)d;
+    ovf += (uint32_t)((d >> 32) & 1u);
+#else
+    uint32_t m;
+    asm("sub.cc.u32 %0, %0, %3;\n\t"
+        "subc.cc.u32 %1, %1, 0;\n\t"
+        "subc.u32 %2, 0, 0;"
+        : "+r"(r[0]), "+r"(r[1]), "=r"(m)
+        : "r"(k));
+    ovf -= m;   // m = 0 or all ones
+#endif
+}
+KB_FN void fe_reduce512_sw(fe& r, uint32_t* t, uint32_t& ovf)
+{
+#if defined(KB_FE_FOLD_SHIFT)
+    (void)ovf;
+    fe_reduce512_shift(r, t);
+#else
+    const uint32_t top = fe_reduce512_fold(r, t);
+    kb_add_small2(r.v, top * 38u, ovf);
+#endif
+}
+// the row order of fe_mul_inl / fe_sq_inl (KB_FE_MUL_RIP, KB_FE_SQ_RIP), always inlined
+KB_FN void fe_mul_sw(fe& h, const fe& f, const fe& g, uint32_t& ovf)
+{
+    uint32_t t[17];
+#if defined(KB_FE_MUL_RIP)
+    fe_mul_rip_wide(t, f, g);
+#else
+    fe_mul_rows_wide(t, f, g);
+#endif
+    fe_reduce512_sw(h, t, ovf);
+}
+KB_FN void fe_sq_sw(fe& h, const fe& f, uint32_t& ovf)
+{
+    uint32_t t[17];
+#if defined(KB_FE_SQ_RIP)
+    fe_sq_rip_wide(t, f);
+#else
+    fe_sq_rows_wide(t, f);
+#endif
+    fe_reduce512_sw(h, t, ovf);
+}
+KB_FN void fe_add_sw(fe& h, const fe& f, const fe& g, uint32_t& ovf)
+{
+    const uint32_t c = kb_add8(h.v, f.v, g.v);
+    kb_add_small2(h.v, 38u * c, ovf);   // 2^256 = 38
+}
+KB_FN void fe_sub_sw(fe& h, const fe& f, const fe& g, uint32_t& ovf)
+{
+#if defined(KB_FE_SUBMASK)
+    const uint32_t m = kb_sub8m(h.v, f.v, g.v);
+    kb_sub_small2(h.v, m & 38u, ovf);   // -2^256 = -38
+#else
+    const uint32_t b = kb_sub8(h.v, f.v, g.v);
+    kb_sub_small2(h.v, 38u * b, ovf);
+#endif
+}
+KB_FN void fe_dbl_sw(fe& h, const fe& f, uint32_t& ovf) { fe_add_sw(h, f, f, ovf); }
+
+// Two sets of field operations for code written once for both kinds of body (ge.cuh, ops.cuh): the last argument picks
+// the exact bodies (fe_ex) or the short-wrap bodies and their counter (fe_sw).
+struct fe_ex {};
+struct fe_sw {
+    uint32_t ovf;
+};
+KB_FN void fe_mul(fe& h, const fe& f, const fe& g, fe_ex&) { fe_mul(h, f, g); }
+KB_FN void fe_sq(fe& h, const fe& f, fe_ex&) { fe_sq(h, f); }
+KB_FN void fe_add(fe& h, const fe& f, const fe& g, fe_ex&) { fe_add(h, f, g); }
+KB_FN void fe_sub(fe& h, const fe& f, const fe& g, fe_ex&) { fe_sub(h, f, g); }
+KB_FN void fe_dbl(fe& h, const fe& f, fe_ex&) { fe_dbl(h, f); }
+KB_FN void fe_mul(fe& h, const fe& f, const fe& g, fe_sw& s) { fe_mul_sw(h, f, g, s.ovf); }
+KB_FN void fe_sq(fe& h, const fe& f, fe_sw& s) { fe_sq_sw(h, f, s.ovf); }
+KB_FN void fe_add(fe& h, const fe& f, const fe& g, fe_sw& s) { fe_add_sw(h, f, g, s.ovf); }
+KB_FN void fe_sub(fe& h, const fe& f, const fe& g, fe_sw& s) { fe_sub_sw(h, f, g, s.ovf); }
+KB_FN void fe_dbl(fe& h, const fe& f, fe_sw& s) { fe_dbl_sw(h, f, s.ovf); }
+template <class F>
+KB_FN void fe_neg(fe& h, const fe& f, F& fo)
+{
+    fe z;
+    fe_set(z, 0);
+    fe_sub(h, z, f, fo);
+}
 
 // ---------------------------------------------------------------------------------------
 // canonical form and byte I/O (fe.rs:67 fe_from_bytes, :147 fe_to_bytes, :240, :246)

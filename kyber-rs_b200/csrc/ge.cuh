@@ -143,14 +143,22 @@ __device__ __forceinline__ void kb_store_precomp_w128(uint32_t* o, const ge_prec
     kb_store_fe(o + 16, q.xy2d);
 }
 #endif
+// The formulas the verifiers run exist in two forms: with a trailing F& (F = fe_ex or fe_sw, fe.cuh: exact or short-wrap
+// field bodies) and without, which is the exact form every other kernel uses.
 // ge.rs:99 write_cached
-KB_FN void ge_to_cached(ge_cached& r, const ge_p3& p)
+template <class F>
+KB_FN void ge_to_cached(ge_cached& r, const ge_p3& p, F& fo)
 {
     const fe d2 = KB_FE_D2;
-    fe_add(r.YpX, p.Y, p.X);
-    fe_sub(r.YmX, p.Y, p.X);
-    fe_mul(r.T2d, p.T, d2);
+    fe_add(r.YpX, p.Y, p.X, fo);
+    fe_sub(r.YmX, p.Y, p.X, fo);
+    fe_mul(r.T2d, p.T, d2, fo);
     r.Z = p.Z;
+}
+KB_FN void ge_to_cached(ge_cached& r, const ge_p3& p)
+{
+    fe_ex x;
+    ge_to_cached(r, p, x);
 }
 // ExtendedGroupElement::neg (ge.rs:77)
 KB_FN void ge_neg(ge_p3& r, const ge_p3& p)
@@ -161,13 +169,19 @@ KB_FN void ge_neg(ge_p3& r, const ge_p3& p)
     fe_neg(r.T, p.T);
 }
 // -c for a cached operand: swap (Y+X, Y-X), negate 2dT
-KB_FN void ge_cached_cneg(ge_cached& c, uint32_t neg)
+template <class F>
+KB_FN void ge_cached_cneg(ge_cached& c, uint32_t neg, F& fo)
 {
     fe a = c.YpX, n;
     fe_cmov(c.YpX, c.YmX, neg);
     fe_cmov(c.YmX, a, neg);
-    fe_neg(n, c.T2d);
+    fe_neg(n, c.T2d, fo);
     fe_cmov(c.T2d, n, neg);
+}
+KB_FN void ge_cached_cneg(ge_cached& c, uint32_t neg)
+{
+    fe_ex x;
+    ge_cached_cneg(c, neg, x);
 }
 KB_FN void ge_precomp_cneg(ge_precomp& c, uint32_t neg)
 {
@@ -180,24 +194,30 @@ KB_FN void ge_precomp_cneg(ge_precomp& c, uint32_t neg)
 
 // r = p + q   (ge.rs:217 add + :292 to_extended; 8M).  WITH_T=false skips T3 (7M) when the
 // next operation is a doubling.
-KB_FN void ge_add_rt(ge_p3& r, const ge_p3& p, const ge_cached& q, bool WITH_T)
+template <class F>
+KB_FN void ge_add_rt(ge_p3& r, const ge_p3& p, const ge_cached& q, bool WITH_T, F& fo)
 {
     fe a, b, c, d, e, f, g, h;
-    fe_sub(a, p.Y, p.X);
-    fe_add(b, p.Y, p.X);
-    fe_mul(a, a, q.YmX);
-    fe_mul(b, b, q.YpX);
-    fe_mul(c, p.T, q.T2d);
-    fe_mul(d, p.Z, q.Z);
-    fe_dbl(d, d);
-    fe_sub(e, b, a);
-    fe_sub(f, d, c);
-    fe_add(g, d, c);
-    fe_add(h, b, a);
-    fe_mul(r.X, e, f);
-    fe_mul(r.Y, g, h);
-    fe_mul(r.Z, f, g);
-    if (WITH_T) fe_mul(r.T, e, h);
+    fe_sub(a, p.Y, p.X, fo);
+    fe_add(b, p.Y, p.X, fo);
+    fe_mul(a, a, q.YmX, fo);
+    fe_mul(b, b, q.YpX, fo);
+    fe_mul(c, p.T, q.T2d, fo);
+    fe_mul(d, p.Z, q.Z, fo);
+    fe_dbl(d, d, fo);
+    fe_sub(e, b, a, fo);
+    fe_sub(f, d, c, fo);
+    fe_add(g, d, c, fo);
+    fe_add(h, b, a, fo);
+    fe_mul(r.X, e, f, fo);
+    fe_mul(r.Y, g, h, fo);
+    fe_mul(r.Z, f, g, fo);
+    if (WITH_T) fe_mul(r.T, e, h, fo);
+}
+KB_FN void ge_add_rt(ge_p3& r, const ge_p3& p, const ge_cached& q, bool WITH_T)
+{
+    fe_ex x;
+    ge_add_rt(r, p, q, WITH_T, x);
 }
 // r = p + q or p - q (ge.rs:217 add / :236 sub): subtraction swaps the roles of Y+X / Y-X and of
 // the two sums with 2dT.  `sub` is meant to be warp-uniform (public digit of a shared scalar).
@@ -288,42 +308,60 @@ KB_FN void ge_add_front(fe& e, fe& f, fe& g, fe& h, const ge_p3& p, const ge_cac
     fe_add(h, b, a);
 }
 // the same when the operand is known to have Z = 1 in some calls (q_z_one, uniform over the warp): 2 Z1 needs no product
-KB_FN void ge_add_front_z(fe& e, fe& f, fe& g, fe& h, const ge_p3& p, const ge_cached& q, bool q_z_one)
+template <class F>
+KB_FN void ge_add_front_z(fe& e, fe& f, fe& g, fe& h, const ge_p3& p, const ge_cached& q, bool q_z_one, F& fo)
 {
     fe a, b, c, d;
-    fe_sub(a, p.Y, p.X);
-    fe_add(b, p.Y, p.X);
-    fe_mul(a, a, q.YmX);
-    fe_mul(b, b, q.YpX);
-    fe_mul(c, p.T, q.T2d);
+    fe_sub(a, p.Y, p.X, fo);
+    fe_add(b, p.Y, p.X, fo);
+    fe_mul(a, a, q.YmX, fo);
+    fe_mul(b, b, q.YpX, fo);
+    fe_mul(c, p.T, q.T2d, fo);
     if (q_z_one) d = p.Z;
-    else fe_mul(d, p.Z, q.Z);
-    fe_dbl(d, d);
-    fe_sub(e, b, a);
-    fe_sub(f, d, c);
-    fe_add(g, d, c);
-    fe_add(h, b, a);
+    else fe_mul(d, p.Z, q.Z, fo);
+    fe_dbl(d, d, fo);
+    fe_sub(e, b, a, fo);
+    fe_sub(f, d, c, fo);
+    fe_add(g, d, c, fo);
+    fe_add(h, b, a, fo);
+}
+KB_FN void ge_add_front_z(fe& e, fe& f, fe& g, fe& h, const ge_p3& p, const ge_cached& q, bool q_z_one)
+{
+    fe_ex x;
+    ge_add_front_z(e, f, g, h, p, q, q_z_one, x);
+}
+template <class F>
+KB_FN void ge_dbl_front(fe& e, fe& f, fe& g, fe& h, const ge_p3& p, F& fo)
+{
+    fe a, b, c;
+    fe_sq(a, p.X, fo);
+    fe_sq(b, p.Y, fo);
+    fe_sq(c, p.Z, fo);
+    fe_dbl(c, c, fo);
+    fe_add(h, a, b, fo);
+    fe_add(e, p.X, p.Y, fo);
+    fe_sq(e, e, fo);
+    fe_sub(e, h, e, fo);
+    fe_sub(g, a, b, fo);
+    fe_add(f, c, g, fo);
 }
 KB_FN void ge_dbl_front(fe& e, fe& f, fe& g, fe& h, const ge_p3& p)
 {
-    fe a, b, c;
-    fe_sq(a, p.X);
-    fe_sq(b, p.Y);
-    fe_sq(c, p.Z);
-    fe_dbl(c, c);
-    fe_add(h, a, b);
-    fe_add(e, p.X, p.Y);
-    fe_sq(e, e);
-    fe_sub(e, h, e);
-    fe_sub(g, a, b);
-    fe_add(f, c, g);
+    fe_ex x;
+    ge_dbl_front(e, f, g, h, p, x);
+}
+template <class F>
+KB_FN void ge_tail(ge_p3& r, const fe& e, const fe& f, const fe& g, const fe& h, bool WITH_T, F& fo)
+{
+    fe_mul(r.X, e, f, fo);
+    fe_mul(r.Y, g, h, fo);
+    fe_mul(r.Z, f, g, fo);
+    if (WITH_T) fe_mul(r.T, e, h, fo);
 }
 KB_FN void ge_tail(ge_p3& r, const fe& e, const fe& f, const fe& g, const fe& h, bool WITH_T)
 {
-    fe_mul(r.X, e, f);
-    fe_mul(r.Y, g, h);
-    fe_mul(r.Z, f, g);
-    if (WITH_T) fe_mul(r.T, e, h);
+    fe_ex x;
+    ge_tail(r, e, f, g, h, WITH_T, x);
 }
 
 // compile-time flavours (the flag folds away when the call is inlined with a constant)

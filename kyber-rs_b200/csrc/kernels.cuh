@@ -910,8 +910,34 @@ static __global__ void __launch_bounds__(256) k_half_sort_scatter(size_t n, cons
 #ifndef KB_HALF_PREFETCH
 #define KB_HALF_PREFETCH 1   // operands of the additions fetched one step ahead (ops.cuh ge_triple_scalarmult_prefetch)
 #endif
+#if KB_HALF_JOINT
+// k_verify_half_main runs its table build and loop with the short-wrap field bodies (fe.cuh fe_sw): every input is public.
+// A thread whose counter is not 0 at the end recomputes its record with the exact bodies, in a function that holds no
+// barrier; no honest batch is expected to take it (tests/test_verify_short_wrap.py).  `force_redo` = k > 0
+// (KB_VERIFY_FORCE_REDO, tests) starts the counter at 1 on every k-th thread of a block, so that the redo runs for them.
+// k_verify_half_prep keeps the exact bodies: with short-wrap decompressions it was slower (4.89 -> 5.26 ms for 2^20
+// signatures on one B200, DESIGN 7.1).
+__device__ __forceinline__ uint32_t kb_force_redo(int force_redo) { return force_redo > 0 && threadIdx.x % (unsigned)force_redo == 0; }
+// The exact redo of one record of k_verify_half_main: table, loop (the instance without the block barrier) and verdict.
+// Not inlined, so that the cold copy of the loop neither keeps the record live across the hot loop nor adds to the
+// kernel's spills.
 template <bool SCHNORR>
-static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k_verify_half_main(size_t n, const uint32_t* recs, const uint32_t* perm, uint8_t* status, const ge_precomp* comb, int min_windows)
+static __device__ __noinline__ uint32_t kb_verify_half_exact(const uint32_t* o, int nwin, const ge_precomp* comb)
+{
+    kb_half_rec rec;
+    kb_rec_load(rec, o);
+    kb_comb_digit dw[KB_COMB_POS];
+    ge_cached tbl[KB_JOINT_SLOTS];
+    uint32_t uk[8], vk[8];
+    fe_ex ex;
+    sig_half_setup_joint(dw, uk, vk, tbl, rec, ex);
+    ge_p3 W;
+    ge_triple_scalarmult_joint<false>(W, nwin, dw, uk, vk, tbl, comb, ex);
+    return sig_half_finish<SCHNORR>(rec.f, W);
+}
+#endif
+template <bool SCHNORR>
+static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k_verify_half_main(size_t n, const uint32_t* recs, const uint32_t* perm, uint8_t* status, const ge_precomp* comb, int min_windows, int force_redo)
 {
     __shared__ int s_nwin;
 #if KB_HALF_JOINT
@@ -930,7 +956,8 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k
 #if KB_HALF_JOINT
     ge_cached tbl[KB_JOINT_SLOTS];
     uint32_t uk[8], vk[8];
-    sig_half_setup_joint(dw, uk, vk, tbl, rec);
+    fe_sw fo = {kb_force_redo(force_redo)};
+    sig_half_setup_joint(dw, uk, vk, tbl, rec, fo);
 #else
     ge_cached tbl[16];
     int8_t eu[64], ev[64];
@@ -947,7 +974,12 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k
     nwin = s_nwin;
     ge_p3 W;
 #if KB_HALF_JOINT
-    ge_triple_scalarmult_joint(W, nwin, dw, uk, vk, tbl, comb);
+    ge_triple_scalarmult_joint<true>(W, nwin, dw, uk, vk, tbl, comb, fo);
+    if (__any_sync(0xffffffffu, fo.ovf) && fo.ovf) {
+        const uint32_t st = kb_verify_half_exact<SCHNORR>(kb_rec_at(recs, i), nwin, comb);
+        if (live) status[i] = (uint8_t)st;
+        return;
+    }
 #elif KB_HALF_PREFETCH
     ge_triple_scalarmult_prefetch(W, nwin, dw, eu, ev, tbl, comb);
 #else

@@ -608,7 +608,8 @@ KB_FN void kb_operand_fetch(kb_operand& o, int i, int a, const kb_comb_digit* dw
     if (i >= 0) o.c = tbl[8 * a + idx];
     else kb_ld_precomp(o.c, comb + (size_t)(-1 - i) * KB_COMB_HALF + idx);
 }
-KB_FN void kb_operand_use(ge_cached& c, const kb_operand& o, bool is_comb)
+template <class F>
+KB_FN void kb_operand_use(ge_cached& c, const kb_operand& o, bool is_comb, F& fo)
 {
     ge_cached id;
     ge_cached_identity(id);
@@ -618,7 +619,12 @@ KB_FN void kb_operand_use(ge_cached& c, const kb_operand& o, bool is_comb)
     fe_cmov(c.YmX, id.YmX, o.nz ^ 1u);
     fe_cmov(c.T2d, id.T2d, o.nz ^ 1u);
     fe_cmov(c.Z, id.Z, o.nz ^ 1u);
-    ge_cached_cneg(c, o.neg);
+    ge_cached_cneg(c, o.neg, fo);
+}
+KB_FN void kb_operand_use(ge_cached& c, const kb_operand& o, bool is_comb)
+{
+    fe_ex x;
+    kb_operand_use(c, o, is_comb, x);
 }
 KB_FN void ge_triple_scalarmult_prefetch(ge_p3& h, int nwin, const kb_comb_digit* dw, const int8_t* eu, const int8_t* ev, const ge_cached* tbl, const ge_precomp* comb)
 {
@@ -682,14 +688,15 @@ KB_FN int sc_joint4_code(const uint32_t* uk, const uint32_t* vk, int idx)
     return neg ? -code : code;
 }
 // the joint table from A' and R' (affine): nine additions through ONE addition body.  Start points are A', R', the
-// previous sum or -A'; operands are entries already written (A', R', 2R'), possibly negated.
-KB_FN void ge_build_joint_table(ge_cached* tbl, const kb_half_rec& rec)
+// previous sum or -A'; operands are entries already written (A', R', 2R'), possibly negated.  F = fe_ex / fe_sw (fe.cuh).
+template <class F>
+KB_FN void ge_build_joint_table(ge_cached* tbl, const kb_half_rec& rec, F& fo)
 {
     ge_p3 m;
     m.X = rec.ax; m.Y = rec.ay; m.T = rec.at; fe_set(m.Z, 1);
-    ge_to_cached(tbl[0], m);
+    ge_to_cached(tbl[0], m, fo);
     m.X = rec.rx; m.Y = rec.ry; m.T = rec.rt;
-    ge_to_cached(tbl[4], m);
+    ge_to_cached(tbl[4], m, fo);
     ge_cached_identity(tbl[7]);
     //  step        0     1     2     3      4     5      6      7       8
     //  sum        2A'   2R'   R'+A' R'+2A' R'-A' R'-2A' 2R'+A' 2R'+2A' 2R'-A'
@@ -709,20 +716,31 @@ KB_FN void ge_build_joint_table(ge_cached* tbl, const kb_half_rec& rec)
             fe_cmov(b.Y, rec.ry, isr);
             fe_cmov(b.T, rec.rt, isr);
             fe_set(b.Z, 1);
-            if (from == 3) { fe_neg(b.X, b.X); fe_neg(b.T, b.T); }
+            if (from == 3) { fe_neg(b.X, b.X, fo); fe_neg(b.T, b.T, fo); }
         }
         ge_cached c = tbl[opnd];
-        ge_cached_cneg(c, neg);
-        ge_add<true>(m, b, c);
-        ge_to_cached(tbl[dst], m);
+        ge_cached_cneg(c, neg, fo);
+        ge_add_rt(m, b, c, true, fo);
+        ge_to_cached(tbl[dst], m, fo);
     }
 }
-KB_FN void sig_half_setup_joint(kb_comb_digit* dw, uint32_t* uk, uint32_t* vk, ge_cached* tbl, const kb_half_rec& rec)
+KB_FN void ge_build_joint_table(ge_cached* tbl, const kb_half_rec& rec)
+{
+    fe_ex x;
+    ge_build_joint_table(tbl, rec, x);
+}
+template <class F>
+KB_FN void sig_half_setup_joint(kb_comb_digit* dw, uint32_t* uk, uint32_t* vk, ge_cached* tbl, const kb_half_rec& rec, F& fo)
 {
     sc_recode_comb(dw, rec.w);
     sc_joint4_bias(uk, rec.u);
     sc_joint4_bias(vk, rec.v);
-    ge_build_joint_table(tbl, rec);
+    ge_build_joint_table(tbl, rec, fo);
+}
+KB_FN void sig_half_setup_joint(kb_comb_digit* dw, uint32_t* uk, uint32_t* vk, ge_cached* tbl, const kb_half_rec& rec)
+{
+    fe_ex x;
+    sig_half_setup_joint(dw, uk, vk, tbl, rec, x);
 }
 // operand of an addition, one step ahead: a joint-table entry by its code, or comb position p
 KB_FN void kb_operand_fetch_code(kb_operand& o, int d, const ge_cached* tbl)
@@ -749,11 +767,13 @@ KB_FN int sc_joint4_pairs(const uint32_t* u, const uint32_t* v)
 }
 // W = |v|*A' + u*R' + w*B: `npair` steps of (two doublings, one joint addition) — the first one IS its operand —
 // then the comb.  The trip count is uniform over the block (the loop holds the lockstep barrier, every second pair).
-// Operands are fetched one step ahead as in ge_triple_scalarmult_prefetch.
+// Operands are fetched one step ahead as in ge_triple_scalarmult_prefetch.  F = fe_ex / fe_sw (fe.cuh); LOCKSTEP = false
+// drops the block barrier, for a caller that runs the loop in a divergent branch.
 #ifndef KB_JOINT_SYNC
 #define KB_JOINT_SYNC 1   // lockstep barrier when (pair index & KB_JOINT_SYNC) == KB_JOINT_SYNC: every second pair
 #endif
-KB_FN void ge_triple_scalarmult_joint(ge_p3& h, int npair, const kb_comb_digit* dw, const uint32_t* uk, const uint32_t* vk, const ge_cached* tbl, const ge_precomp* comb)
+template <bool LOCKSTEP, class F>
+KB_FN void ge_triple_scalarmult_joint(ge_p3& h, int npair, const kb_comb_digit* dw, const uint32_t* uk, const uint32_t* vk, const ge_cached* tbl, const ge_precomp* comb, F& fo)
 {
     if (npair < 2) npair = 2;   // a leading zero pair costs nothing wrong; it lets the first step below drop T
     kb_operand nx;
@@ -762,35 +782,47 @@ KB_FN void ge_triple_scalarmult_joint(ge_p3& h, int npair, const kb_comb_digit* 
         // the first addition would add to the identity: take the operand itself, (2X : 2Y : 2Z) from (Y+X, Y-X, Z);
         // doublings follow, so T is not needed
         ge_cached c;
-        kb_operand_use(c, nx, false);
-        fe_sub(h.X, c.YpX, c.YmX);
-        fe_add(h.Y, c.YpX, c.YmX);
-        fe_dbl(h.Z, c.Z);
+        kb_operand_use(c, nx, false, fo);
+        fe_sub(h.X, c.YpX, c.YmX, fo);
+        fe_add(h.Y, c.YpX, c.YmX, fo);
+        fe_dbl(h.Z, c.Z, fo);
         fe_set(h.T, 0);
+        // A leading zero pair (a lane whose scalars are shorter than the block's loop) makes that the identity.  It is taken
+        // as (0 : d : d) instead of (0 : 2 : 2): doubling (0 : 2 : 2) gives Y = Z = -16, held as 2^256 - 54, and the squares
+        // of such small negatives carry through every word — the short-wrap bodies would flag the lane.  Any (0 : k : k) is
+        // the identity; with k = d the coordinates look random from the first doubling on.
+        const fe d = KB_FE_D;
+        fe_cmov(h.Y, d, nx.nz ^ 1u);
+        fe_cmov(h.Z, d, nx.nz ^ 1u);
     }
     KB_NOUNROLL
     for (int i = npair - 2; i >= -KB_COMB_POS; i--) {
-        if (i < 0 || (i & KB_JOINT_SYNC) == KB_JOINT_SYNC) KB_LOCKSTEP();
+        if (LOCKSTEP && (i < 0 || (i & KB_JOINT_SYNC) == KB_JOINT_SYNC)) { KB_LOCKSTEP(); }
         const int lead = i >= 0 ? 2 : 0;
         KB_NOUNROLL
         for (int step = 0; step <= lead; step++) {
             fe e, f, g, hh;
             bool with_t;
             if (step < lead) {
-                ge_dbl_front(e, f, g, hh, h);
+                ge_dbl_front(e, f, g, hh, h, fo);
                 with_t = step == lead - 1;   // the addition follows
                 if (with_t) kb_operand_fetch_code(nx, sc_joint4_code(uk, vk, i), tbl);
             } else {
                 ge_cached c;
-                kb_operand_use(c, nx, i < 0);
-                ge_add_front_z(e, f, g, hh, h, c, i < 0);   // comb entries are affine
+                kb_operand_use(c, nx, i < 0, fo);
+                ge_add_front_z(e, f, g, hh, h, c, i < 0, fo);   // comb entries are affine
                 // T is dead when a doubling (or the end) follows: it is needed in front of the comb additions only
                 with_t = i <= 0 && i != -KB_COMB_POS;
                 if (with_t) kb_operand_fetch_comb(nx, -i, dw, comb);   // position -1 - (i - 1)
             }
-            ge_tail(h, e, f, g, hh, with_t);
+            ge_tail(h, e, f, g, hh, with_t, fo);
         }
     }
+}
+KB_FN void ge_triple_scalarmult_joint(ge_p3& h, int npair, const kb_comb_digit* dw, const uint32_t* uk, const uint32_t* vk, const ge_cached* tbl, const ge_precomp* comb)
+{
+    fe_ex x;
+    ge_triple_scalarmult_joint<true>(h, npair, dw, uk, vk, tbl, comb, x);
 }
 // h = a * B for a PUBLIC scalar through the comb: KB_COMB_POS (15) mixed additions instead of 64 (ge_scalarmult_base), no doublings.
 // Any 32-byte scalar gives the reference's result: sc_effective is the integer the reference's digit loop
