@@ -201,6 +201,47 @@ int  kb_dev_keyset_mul(kb_keyset* ks, size_t n, const void* d_key_idx, const voi
  * s = (r + h*a) mod L.  sig[i] = R || s (64 bytes), pk[i] = A (may be NULL).  Deterministic: reproduces the
  * reference's golden signatures.  The secret scalars only meet the constant-time table select. */
 int kb_eddsa_sign_batch(kb_ctx* ctx, size_t n, const uint8_t* seeds, const uint8_t* msg, const uint64_t* msg_off, uint8_t* sig, uint8_t* pk);
+/* schnorr::sign (sign/schnorr/schnorr_sig.rs:25-47) for n (secret x, nonce k, message) triples: A = x*B, R = k*B,
+ * h = Scalar::set_bytes(SHA-512(R || A || M)), s = (k + h*x) mod L; sig[i] = R || s (64 bytes), pk[i] = A (may be NULL).
+ * x and k are raw 32-byte integers, never reduced on entry (clamped keys with bit 254 set are in the domain).  For a
+ * scalar with byte 31 > 127, R and A are the bytes kb_point_mul_base_batch returns for it and the rest of the signature
+ * follows from those bytes.  The nonces are what the reference draws from its random stream, supplied by the caller; the
+ * library cannot detect a reused nonce, and a nonce used twice under one key reveals that key.  Secrets and nonces only
+ * meet the constant-time table select and branch-free scalar code, and the scratch that held them is zeroed before the
+ * call returns.  KB_ERR_ARG for a NULL pointer or decreasing msg_off; n == 0 is KB_OK. */
+int kb_schnorr_sign_batch(kb_ctx* ctx, size_t n, const uint8_t* secrets, const uint8_t* nonces, const uint8_t* msg, const uint64_t* msg_off, uint8_t* sig, uint8_t* pk);
+
+/* ---- signer sets: signing under registered secret keys -------------------------------------------------------------
+ * The participants of a DKG round sign every deal and response with one fixed key each (a round holds 2 n^2 signatures
+ * under n keys).  A signer set derives, once per key and on the device, what signing needs besides the nonce:
+ *   KB_SIGNER_SCHNORR   x and A = x*B                                      (schnorr_sig.rs:25-47)
+ *   KB_SIGNER_EDDSA     a = clamp(SHA-512(seed)[0..32]), prefix = SHA-512(seed)[32..64] and A = a*B
+ *                       (Curve::new_key_and_seed_with_input, curve.rs:74-87; EdDSA::sign, eddsa_sig.rs:120-152)
+ * so that a signature costs one constant-time fixed-base multiplication (r*B) instead of two.  The set holds 64 (Schnorr)
+ * or 96 (EdDSA) bytes per key in an allocation of its own, not in scratch; kb_signerset_destroy zeroes it and waits for
+ * the zeroing before freeing it.  A set belongs to its context (same device, errors in kb_last_error(ctx)) and must be
+ * destroyed before that context. */
+typedef struct kb_signerset kb_signerset;
+#define KB_SIGNER_SCHNORR 0   /* keys are 32-byte secret scalars x (schnorr::sign)                          */
+#define KB_SIGNER_EDDSA   1   /* keys are 32-byte seeds (EdDSA::sign with the curve.rs:74-87 derivation)    */
+/* Registers nkeys keys of one kind; pk_out (may be NULL) receives the nkeys encodings of A, the bytes kb_point_mul_base_batch
+ * returns for x (Schnorr) or a (EdDSA).  KB_ERR_ARG for nkeys == 0, a NULL pointer or an unknown kind. */
+int  kb_signerset_create(kb_ctx* ctx, size_t nkeys, const uint8_t* keys, int kind, uint8_t* pk_out, kb_signerset** out);
+void kb_signerset_destroy(kb_signerset* ss);
+/* sig[i] for key key_idx[i] and message i, byte for byte what kb_schnorr_sign_batch returns for (keys[key_idx[i]],
+ * nonces[i], M_i) (Schnorr set) or kb_eddsa_sign_batch for (keys[key_idx[i]], M_i) (EdDSA set).  A Schnorr set requires
+ * nonces (n x 32 bytes, as kb_schnorr_sign_batch); an EdDSA set derives r = SHA-512(prefix || M) mod L and requires
+ * nonces == NULL; the other combination is KB_ERR_ARG.  KB_ERR_ARG, before anything is launched, for a NULL pointer, a
+ * decreasing msg_off or any key_idx[i] >= nkeys; n == 0 is KB_OK.  The scratch that held nonces is zeroed before the
+ * call returns. */
+int  kb_signerset_sign_batch(kb_signerset* ss, size_t n, const uint32_t* key_idx, const uint8_t* nonces, const uint8_t* msg,
+                             const uint64_t* msg_off, uint8_t* sig);
+/* device buffers + stream, ordered like every kb_dev_* call of the context (d_msg_off as for the other kb_dev_* calls).  An
+ * index >= nkeys gives status 0xFF and 64 zero bytes for that item, and the kernels read nothing of the set for it;
+ * status 0 otherwise (d_status may be NULL).  The nonce / kind rule of the host form holds.  The EdDSA nonces r pass
+ * through scratch, which is zeroed on the stream at the end of the call. */
+int  kb_dev_signerset_sign(kb_signerset* ss, size_t n, const void* d_key_idx, const void* d_nonces, const void* d_msg,
+                           const void* d_msg_off, void* d_sig, void* d_status, void* stream);
 
 /* ---- committed polynomials (share/poly.rs) -------------------------------------------- */
 /* PubPoly::eval (poly.rs:457-469) for npoly polynomials of t commitments each
@@ -323,6 +364,9 @@ int kb_dev_point_sum(kb_ctx* ctx, size_t k, const void* d_partials128, void* d_o
 /* the pure decompress (ExtendedGroupElement::set_bytes -> X, Y, Z, T words) and hash (SHA-512(R || A || M) mod L) stages */
 int kb_dev_point_decompress(kb_ctx* ctx, size_t n, const void* d_in, void* d_out128, void* d_status, void* stream);
 int kb_dev_challenge(kb_ctx* ctx, size_t n, const void* d_r32, const void* d_a32, const void* d_msg, const void* d_msg_off, void* d_out32, void* stream);
+/* kb_schnorr_sign_batch on device buffers (d_pk may be NULL); the caller owns, and wipes, the secret and nonce buffers */
+int kb_dev_schnorr_sign(kb_ctx* ctx, size_t n, const void* d_secrets, const void* d_nonces, const void* d_msg,
+                        const void* d_msg_off, void* d_sig, void* d_pk, void* stream);
 int kb_dev_pripoly_eval(kb_ctx* ctx, size_t npoly, size_t t, const void* d_coeffs, size_t n, void* d_out, void* stream);
 /* kb_dkg_process_round on device buffers for ndealers dealers (arrays start at the first of them) */
 int kb_dev_dkg_process_round(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, int fmt, const void* d_commits, const void* d_shares, void* d_verdict,
@@ -385,6 +429,19 @@ int  kb_mctx_dkg_process_round_keyed(kb_mctx* m, const kb_mkeyset* dealers, cons
                                      const void* commits, const uint8_t* shares, uint8_t* verdict,
                                      const uint8_t* deal_msg, const uint64_t* deal_msg_off, const uint8_t* deal_sig, uint8_t* deal_status,
                                      const uint8_t* resp_msg, const uint64_t* resp_msg_off, const uint8_t* resp_sig, uint8_t* resp_status);
+/* kb_schnorr_sign_batch split by index over all devices (pk may be NULL); msg_off is checked before any device starts */
+int  kb_mctx_schnorr_sign_batch(kb_mctx* m, size_t n, const uint8_t* secrets, const uint8_t* nonces, const uint8_t* msg,
+                                const uint64_t* msg_off, uint8_t* sig, uint8_t* pk);
+/* Signer sets over all devices: one kb_signerset per device, each holding EVERY key (64 or 96 bytes per key on each GPU).
+ * pk_out (may be NULL) receives the public keys once.  If one device fails, the sets already built are destroyed and the
+ * error is in kb_mctx_last_error.  A kb_msignerset must be destroyed before its kb_mctx. */
+typedef struct kb_msignerset kb_msignerset;
+int  kb_mctx_signerset_create(kb_mctx* m, size_t nkeys, const uint8_t* keys, int kind, uint8_t* pk_out, kb_msignerset** out);
+void kb_mctx_signerset_destroy(kb_msignerset* ss);
+/* kb_signerset_sign_batch split by index over all devices.  Every key index, the nonce / kind rule and msg_off are checked
+ * before any device starts (KB_ERR_ARG); each device copies only the message bytes of its own items. */
+int  kb_mctx_signerset_sign_batch(kb_msignerset* ss, size_t n, const uint32_t* key_idx, const uint8_t* nonces, const uint8_t* msg,
+                                  const uint64_t* msg_off, uint8_t* sig);
 /* kb_msm over all devices */
 int kb_mctx_msm(kb_mctx* m, size_t n, const uint8_t* scalars, const uint8_t* points, uint8_t* out32, uint64_t* bad_points);
 

@@ -15,6 +15,10 @@ from .binding import (  # noqa: F401
     KeySet,
     MultiContext,
     MultiKeySet,
+    MultiSignerSet,
+    SignerSet,
+    SIGNER_EDDSA,
+    SIGNER_SCHNORR,
     KBError,
     LIB_PATH,
     SIG_STATUS_NAMES,
@@ -25,4 +29,4 @@ from .binding import (  # noqa: F401
 from . import host  # noqa: F401
 from . import sharding  # noqa: F401
 
-__all__ = ["Context", "KeySet", "MultiContext", "MultiKeySet", "KBError", "LIB_PATH", "SIG_STATUS_NAMES", "FLAG_VARTIME", "FLAG_SHARED_POINT", "load_library", "host", "sharding"]
+__all__ = ["Context", "KeySet", "MultiContext", "MultiKeySet", "SignerSet", "MultiSignerSet", "SIGNER_SCHNORR", "SIGNER_EDDSA", "KBError", "LIB_PATH", "SIG_STATUS_NAMES", "FLAG_VARTIME", "FLAG_SHARED_POINT", "load_library", "host", "sharding"]

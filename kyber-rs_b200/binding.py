@@ -12,6 +12,9 @@ LIB_PATH = os.environ.get("KYBER_B200_LIB") or os.path.join(os.path.dirname(os.p
 FLAG_VARTIME = 1
 FLAG_SHARED_POINT = 2
 
+SIGNER_SCHNORR = 0   # signer-set keys are secret scalars x (schnorr::sign)
+SIGNER_EDDSA = 1     # signer-set keys are 32-byte seeds (EdDSA::sign)
+
 # kb_sig_status -> the reference's SignatureError display strings (sign/error.rs:6-25)
 SIG_STATUS_NAMES = {
     0: "ok",
@@ -48,6 +51,9 @@ EXPORTS = [
     "kb_dkg_process_round_keyed", "kb_dev_dkg_process_round_keyed",
     "kb_mctx_keyset_create", "kb_mctx_keyset_destroy", "kb_mctx_keyset_verify_batch", "kb_mctx_dkg_process_round_keyed",
     "kb_keyset_mul_batch", "kb_dev_keyset_mul", "kb_mctx_keyset_mul_batch",
+    "kb_schnorr_sign_batch", "kb_dev_schnorr_sign", "kb_mctx_schnorr_sign_batch",
+    "kb_signerset_create", "kb_signerset_destroy", "kb_signerset_sign_batch", "kb_dev_signerset_sign",
+    "kb_mctx_signerset_create", "kb_mctx_signerset_destroy", "kb_mctx_signerset_sign_batch",
 ]
 
 
@@ -150,6 +156,18 @@ def load_library(path: str = LIB_PATH):
     L.kb_mctx_keyset_verify_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32]
     L.kb_mctx_keyset_mul_batch.argtypes = [vp, sz, vp, vp, vp, vp, u32]
     L.kb_mctx_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8
+    L.kb_schnorr_sign_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp]
+    L.kb_dev_schnorr_sign.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp, vp]
+    L.kb_mctx_schnorr_sign_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp]
+    L.kb_signerset_create.argtypes = [vp, sz, vp, i32, vp, ctypes.POINTER(vp)]
+    L.kb_signerset_destroy.argtypes = [vp]
+    L.kb_signerset_destroy.restype = None
+    L.kb_signerset_sign_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp]
+    L.kb_dev_signerset_sign.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp, vp]
+    L.kb_mctx_signerset_create.argtypes = [vp, sz, vp, i32, vp, ctypes.POINTER(vp)]
+    L.kb_mctx_signerset_destroy.argtypes = [vp]
+    L.kb_mctx_signerset_destroy.restype = None
+    L.kb_mctx_signerset_sign_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp]
     _LIB = L
     return L
 
@@ -344,6 +362,19 @@ class Context:
         sig = np.empty((n, 64), dtype=np.uint8)
         pk = np.empty((n, 32), dtype=np.uint8)
         self._check(self.L.kb_eddsa_sign_batch(self.h, n, _ptr(seeds), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(pk)), "kb_eddsa_sign_batch")
+        return sig, pk
+
+    def schnorr_sign_batch(self, secrets, nonces, msg, msg_off):
+        """schnorr::sign for n (secret x, nonce k, message) triples in one call -> (sig[n,64], pk[n,32])."""
+        x, k = _u8(secrets, (-1, 32)), _u8(nonces, (-1, 32))
+        msg = _u8(msg)
+        msg_off = np.ascontiguousarray(msg_off, dtype=np.uint64)
+        n = x.shape[0]
+        if k.shape[0] != n or msg_off.shape[0] != n + 1:
+            raise ValueError("schnorr_sign_batch: one nonce per secret, n+1 message offsets")
+        sig = np.empty((n, 64), dtype=np.uint8)
+        pk = np.empty((n, 32), dtype=np.uint8)
+        self._check(self.L.kb_schnorr_sign_batch(self.h, n, _ptr(x), _ptr(k), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(pk)), "kb_schnorr_sign_batch")
         return sig, pk
 
     def pubpoly_eval_batch(self, commits, t, poly_id, idx):
@@ -585,6 +616,11 @@ class Context:
         """Registers the public keys pk (nkeys x 32 encodings) for verification by key index (KeySet)."""
         return KeySet(self, pk)
 
+    def signerset(self, keys, kind=SIGNER_SCHNORR):
+        """Registers secret keys (nkeys x 32: scalars x for SIGNER_SCHNORR, seeds for SIGNER_EDDSA) for signing by key index
+        (SignerSet); its .pk holds the public keys."""
+        return SignerSet(self, keys, kind)
+
     # ---- device-pointer API (torch CUDA tensors; enqueues on torch's current stream) --------
     @staticmethod
     def _dp(t):
@@ -645,6 +681,10 @@ class Context:
 
     def dev_point_sum(self, k, partials, out32):
         self._check(self.L.kb_dev_point_sum(self.h, k, self._dp(partials), self._dp(out32), self._stream()), "kb_dev_point_sum")
+
+    def dev_schnorr_sign(self, n, secrets, nonces, msg, msg_off, sig, pk=None):
+        self._check(self.L.kb_dev_schnorr_sign(self.h, n, self._dp(secrets), self._dp(nonces), self._dp(msg), self._dp(msg_off), self._dp(sig), self._dp(pk), self._stream()),
+                    "kb_dev_schnorr_sign")
 
 
 class KeySet:
@@ -711,6 +751,58 @@ class KeySet:
         current stream; an index outside the set gives status 0xFF and 32 zero bytes."""
         dp = Context._dp
         self.ctx._check(self.L.kb_dev_keyset_mul(self.h, n, dp(key_idx), dp(scalars), dp(out), dp(status), flags, Context._stream()), "kb_dev_keyset_mul")
+
+
+def _sign_args(what, n, key_idx, nonces, msg, msg_off):
+    key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+    k = _u8(nonces, (-1, 32)) if nonces is not None else None
+    msg = _u8(msg)
+    msg_off = np.ascontiguousarray(msg_off, dtype=np.uint64)
+    if (k is not None and k.shape[0] != n) or msg_off.shape[0] != n + 1:
+        raise ValueError(f"{what}: one key index (and nonce) per item, n+1 message offsets")
+    return key_idx, k, msg, msg_off
+
+
+class SignerSet:
+    """One kb_signerset: secret keys registered with a Context (x, or a and prefix, and A per key, on the device).
+    sign_batch(key_idx, msg, msg_off, nonces) equals Context.schnorr_sign_batch(keys[key_idx], nonces) (SIGNER_SCHNORR) or
+    Context.eddsa_sign_batch(keys[key_idx]) (SIGNER_EDDSA, nonces=None) byte for byte."""
+
+    def __init__(self, ctx: Context, keys, kind=SIGNER_SCHNORR):
+        self.ctx = ctx   # the signer set belongs to its context and must go before it
+        self.L = ctx.L
+        self.h = None
+        k = _u8(keys, (-1, 32))
+        self.nkeys = k.shape[0]
+        self.kind = kind
+        self.pk = np.empty((self.nkeys, 32), dtype=np.uint8)
+        h = ctypes.c_void_p()
+        ctx._check(self.L.kb_signerset_create(ctx.h, self.nkeys, _ptr(k), int(kind), _ptr(self.pk), ctypes.byref(h)), "kb_signerset_create")
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.kb_signerset_destroy(self.h)
+            self.h = None
+
+    def __del__(self):  # pragma: no cover
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def sign_batch(self, key_idx, msg, msg_off, nonces=None):
+        n = np.asarray(key_idx).shape[0]
+        key_idx, k, msg, msg_off = _sign_args("SignerSet.sign_batch", n, key_idx, nonces, msg, msg_off)
+        sig = np.empty((n, 64), dtype=np.uint8)
+        self.ctx._check(self.L.kb_signerset_sign_batch(self.h, n, _ptr(key_idx), _ptr(k), _ptr(msg), _ptr(msg_off), _ptr(sig)), "kb_signerset_sign_batch")
+        return sig
+
+    def dev_sign(self, n, key_idx, nonces, msg, msg_off, sig, status=None):
+        """key_idx: n uint32 (torch int32 tensor), nonces n x 32 (None for SIGNER_EDDSA), sig n x 64, status n bytes (or None), on
+        torch's current stream; an index outside the set gives status 0xFF and 64 zero bytes."""
+        dp = Context._dp
+        self.ctx._check(self.L.kb_dev_signerset_sign(self.h, n, dp(key_idx), dp(nonces), dp(msg), dp(msg_off), dp(sig), dp(status), Context._stream()), "kb_dev_signerset_sign")
 
 
 class MultiContext:
@@ -820,6 +912,23 @@ class MultiContext:
                     "kb_mctx_dkg_process_round_keyed")
         return verdict, outs[0], outs[1]
 
+    def schnorr_sign_batch(self, secrets, nonces, msg, msg_off):
+        """Context.schnorr_sign_batch split by index over the devices -> (sig[n,64], pk[n,32])."""
+        x, k = _u8(secrets, (-1, 32)), _u8(nonces, (-1, 32))
+        msg = _u8(msg)
+        msg_off = np.ascontiguousarray(msg_off, dtype=np.uint64)
+        n = x.shape[0]
+        if k.shape[0] != n or msg_off.shape[0] != n + 1:
+            raise ValueError("schnorr_sign_batch: one nonce per secret, n+1 message offsets")
+        sig = np.empty((n, 64), dtype=np.uint8)
+        pk = np.empty((n, 32), dtype=np.uint8)
+        self._check(self.L.kb_mctx_schnorr_sign_batch(self.h, n, _ptr(x), _ptr(k), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(pk)), "kb_mctx_schnorr_sign_batch")
+        return sig, pk
+
+    def signerset(self, keys, kind=SIGNER_SCHNORR):
+        """Registers secret keys on every device of this context (MultiSignerSet)."""
+        return MultiSignerSet(self, keys, kind)
+
     def msm(self, scalars, points):
         s, p = _u8(scalars, (-1, 32)), _u8(points, (-1, 32))
         assert s.shape == p.shape
@@ -877,3 +986,37 @@ class MultiKeySet:
         st = np.empty(n, dtype=np.uint8)
         self.mctx._check(self.L.kb_mctx_keyset_mul_batch(self.h, n, _ptr(key_idx), _ptr(s), _ptr(out), _ptr(st), flags), "kb_mctx_keyset_mul_batch")
         return out, st
+
+
+class MultiSignerSet:
+    """One kb_msignerset: secret keys registered on every device of a MultiContext; sign_batch splits a batch by index."""
+
+    def __init__(self, mctx: MultiContext, keys, kind=SIGNER_SCHNORR):
+        self.mctx = mctx   # the signer set belongs to its context and must go before it
+        self.L = mctx.L
+        self.h = None
+        k = _u8(keys, (-1, 32))
+        self.nkeys = k.shape[0]
+        self.kind = kind
+        self.pk = np.empty((self.nkeys, 32), dtype=np.uint8)
+        h = ctypes.c_void_p()
+        mctx._check(self.L.kb_mctx_signerset_create(mctx.h, self.nkeys, _ptr(k), int(kind), _ptr(self.pk), ctypes.byref(h)), "kb_mctx_signerset_create")
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.kb_mctx_signerset_destroy(self.h)
+            self.h = None
+
+    def __del__(self):  # pragma: no cover
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def sign_batch(self, key_idx, msg, msg_off, nonces=None):
+        n = np.asarray(key_idx).shape[0]
+        key_idx, k, msg, msg_off = _sign_args("MultiSignerSet.sign_batch", n, key_idx, nonces, msg, msg_off)
+        sig = np.empty((n, 64), dtype=np.uint8)
+        self.mctx._check(self.L.kb_mctx_signerset_sign_batch(self.h, n, _ptr(key_idx), _ptr(k), _ptr(msg), _ptr(msg_off), _ptr(sig)), "kb_mctx_signerset_sign_batch")
+        return sig

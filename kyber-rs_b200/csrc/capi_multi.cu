@@ -287,6 +287,84 @@ int kb_mctx_dkg_process_round_keyed(kb_mctx* m, const kb_mkeyset* dealers, const
     });
 }
 
+// ---- signing, split by index ------------------------------------------------------------------------------------------
+// the message offsets of items [lo, hi) made relative to the first of their bytes (malloc'ed; NULL when out of memory)
+static uint64_t* kb_rel_offsets(const uint64_t* msg_off, size_t lo, size_t hi)
+{
+    uint64_t* off = (uint64_t*)malloc(8 * (hi - lo + 1));
+    if (off)
+        for (size_t j = 0; j <= hi - lo; j++) off[j] = msg_off[lo + j] - msg_off[lo];
+    return off;
+}
+int kb_mctx_schnorr_sign_batch(kb_mctx* m, size_t n, const uint8_t* secrets, const uint8_t* nonces, const uint8_t* msg, const uint64_t* msg_off, uint8_t* sig, uint8_t* pk)
+{
+    if (!m || (n && (!secrets || !nonces || !msg_off || !sig))) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    if (!kb_msg_off_ok(n, msg_off) || (msg_off[n] != msg_off[0] && !msg)) return KB_ERR_ARG;
+    return kb_on_all(m, [&](int i) {
+        size_t lo, hi;
+        kb_shard(n, i, m->ndev, &lo, &hi);
+        if (hi == lo) return (int)KB_OK;
+        uint64_t* off = kb_rel_offsets(msg_off, lo, hi);
+        if (!off) return (int)KB_ERR_NOMEM;
+        const int rc = kb_schnorr_sign_batch(m->ctx[i], hi - lo, secrets + 32 * lo, nonces + 32 * lo, msg ? msg + msg_off[lo] : nullptr, off, sig + 64 * lo, pk ? pk + 32 * lo : nullptr);
+        free(off);
+        return rc;
+    });
+}
+
+struct kb_msignerset {
+    kb_mctx* m;
+    size_t nkeys;
+    int kind;
+    kb_signerset* ss[KB_MAX_DEVICES];   // ss[i] belongs to m->ctx[i] and holds every key
+};
+
+int kb_mctx_signerset_create(kb_mctx* m, size_t nkeys, const uint8_t* keys, int kind, uint8_t* pk_out, kb_msignerset** out)
+{
+    if (!out) return KB_ERR_ARG;
+    *out = nullptr;
+    if (!m || nkeys == 0 || !keys || (kind != KB_SIGNER_SCHNORR && kind != KB_SIGNER_EDDSA)) return KB_ERR_ARG;
+    kb_msignerset* ms = (kb_msignerset*)calloc(1, sizeof(kb_msignerset));
+    if (!ms) return KB_ERR_NOMEM;
+    ms->m = m;
+    ms->nkeys = nkeys;
+    ms->kind = kind;
+    const int rc = kb_on_all(m, [&](int i) { return kb_signerset_create(m->ctx[i], nkeys, keys, kind, i == 0 ? pk_out : nullptr, &ms->ss[i]); });
+    if (rc != KB_OK) {
+        kb_mctx_signerset_destroy(ms);
+        return rc;
+    }
+    *out = ms;
+    return KB_OK;
+}
+void kb_mctx_signerset_destroy(kb_msignerset* ms)
+{
+    if (!ms) return;
+    for (int i = 0; i < ms->m->ndev; i++) kb_signerset_destroy(ms->ss[i]);
+    free(ms);
+}
+int kb_mctx_signerset_sign_batch(kb_msignerset* ms, size_t n, const uint32_t* key_idx, const uint8_t* nonces, const uint8_t* msg, const uint64_t* msg_off, uint8_t* sig)
+{
+    if (!ms || (ms->kind == KB_SIGNER_SCHNORR) != (nonces != nullptr)) return KB_ERR_ARG;
+    if (n && (!key_idx || !msg_off || !sig)) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    uint32_t over = 0;
+    for (size_t i = 0; i < n; i++) over |= (uint32_t)(key_idx[i] >= ms->nkeys);
+    if (over || !kb_msg_off_ok(n, msg_off) || (msg_off[n] != msg_off[0] && !msg)) return KB_ERR_ARG;
+    kb_mctx* m = ms->m;
+    return kb_on_all(m, [&](int i) {
+        size_t lo, hi;
+        kb_shard(n, i, m->ndev, &lo, &hi);
+        if (hi == lo) return (int)KB_OK;
+        uint64_t* off = kb_rel_offsets(msg_off, lo, hi);
+        if (!off) return (int)KB_ERR_NOMEM;
+        const int rc = kb_signerset_sign_batch(ms->ss[i], hi - lo, key_idx + lo, nonces ? nonces + 32 * lo : nullptr, msg ? msg + msg_off[lo] : nullptr, off, sig + 64 * lo);
+        free(off);
+        return rc;
+    });
+}
+
 // ---- sharded by points, one collective ---------------------------------------------------------------------------------
 int kb_mctx_msm(kb_mctx* m, size_t n, const uint8_t* scalars, const uint8_t* points, uint8_t* out32, uint64_t* bad_points)
 {

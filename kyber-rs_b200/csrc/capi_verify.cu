@@ -1,4 +1,4 @@
-// capi_verify.cu — eddsa::verify_with_checks / schnorr::verify_with_checks and EdDSA::sign entry points
+// capi_verify.cu — eddsa::verify_with_checks / schnorr::verify_with_checks, EdDSA::sign and schnorr::sign entry points
 #define KB_K_SIGN
 // Field-arithmetic bodies of THIS translation unit (fe.cuh): the zero-free row order of fe_mul / fe_sq and the borrow-mask
 // wrap of fe_sub.  All bodies are bit-exact; which one is faster depends on the kernel (the balance ptxas strikes between
@@ -267,6 +267,69 @@ int kb_eddsa_sign_batch(kb_ctx* ctx, size_t n, const uint8_t* seeds, const uint8
     cudaMemsetAsync(d_a, 0, 32 * n, ctx->stream);
     cudaMemsetAsync(d_r, 0, 32 * n, ctx->stream);
     cudaMemsetAsync(d_seed, 0, 32 * n, ctx->stream);
+    if (rc != KB_OK) {
+        cudaStreamSynchronize(ctx->stream);
+        return rc;
+    }
+    KB_SYNC();
+    return KB_OK;
+}
+
+// ---- schnorr::sign: k_schnorr_sign_stage1, k_compress_batch on the 2n points, k_sign_finish with a = x and r = k
+int kb_dev_schnorr_sign(kb_ctx* ctx, size_t n, const void* d_secrets, const void* d_nonces, const void* d_msg, const void* d_msg_off, void* d_sig, void* d_pk, void* stream)
+{
+    if (!ctx || (n && (!d_secrets || !d_nonces || !d_msg_off || !d_sig))) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    KB_DEV_ENTER(st);
+    uint8_t* d_ra;
+    uint32_t* xyz;
+    KB_SCRATCH(8, 64 * n, d_ra);
+    KB_SCRATCH(KB_SLOT_XYZ, 96 * 2 * n, xyz);
+    const uint8_t *x = (const uint8_t*)d_secrets, *k = (const uint8_t*)d_nonces;
+    k_schnorr_sign_stage1<<<kb_blocks(n, KB_THREADS), KB_THREADS, 64 * 8 * 96, st>>>(n, x, k, xyz, ctx->base_table);
+    KB_LAUNCHED();
+    k_compress_batch<<<kb_blocks((2 * n + KB_INV_K - 1) / KB_INV_K, KB_THREADS), KB_THREADS, 0, st>>>(2 * n, xyz, nullptr, d_ra);
+    KB_LAUNCHED();
+    k_sign_finish<<<kb_blocks(n, KB_THREADS), KB_THREADS, 0, st>>>(n, d_ra, (const uint8_t*)d_msg, (const uint64_t*)d_msg_off, x, k, (uint8_t*)d_sig, (uint8_t*)d_pk);
+    KB_LAUNCHED();
+    KB_DEV_RETURN(st, KB_OK);
+}
+// staging of kb_schnorr_sign_batch; the caller wipes the secret scratch whatever this returns
+static int kb_schnorr_sign_run(kb_ctx* ctx, size_t n, const uint8_t* secrets, const uint8_t* nonces, const uint8_t* msg, const uint64_t* msg_off, size_t mbytes, uint8_t* sig, uint8_t* pk,
+                               uint8_t* d_x, uint8_t* d_k)
+{
+    uint8_t *d_m, *d_sig, *d_pk;
+    uint64_t* d_off;
+    KB_SCRATCH(4, mbytes, d_m);
+    KB_SCRATCH(5, 8 * (n + 1), d_off);
+    KB_SCRATCH(2, 64 * n, d_sig);
+    KB_SCRATCH(1, 32 * n, d_pk);
+    KB_H2D(d_x, secrets, 32 * n);
+    KB_H2D(d_k, nonces, 32 * n);
+    if (mbytes) KB_H2D(d_m, msg, mbytes);
+    KB_H2D(d_off, msg_off, 8 * (n + 1));
+    const int rc = kb_dev_schnorr_sign(ctx, n, d_x, d_k, d_m, d_off, d_sig, pk ? d_pk : nullptr, ctx->stream);
+    if (rc != KB_OK) return rc;
+    KB_D2H(sig, d_sig, 64 * n);
+    if (pk) KB_D2H(pk, d_pk, 32 * n);
+    return KB_OK;
+}
+int kb_schnorr_sign_batch(kb_ctx* ctx, size_t n, const uint8_t* secrets, const uint8_t* nonces, const uint8_t* msg, const uint64_t* msg_off, uint8_t* sig, uint8_t* pk)
+{
+    KB_ENTER();
+    if (n && (!secrets || !nonces || !msg_off || !sig)) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    if (!kb_msg_off_ok(n, msg_off)) return KB_ERR_ARG;
+    const size_t mbytes = (size_t)msg_off[n];
+    if (mbytes && !msg) return KB_ERR_ARG;
+    uint8_t *d_x, *d_k;
+    KB_SCRATCH(0, 32 * n, d_x);
+    KB_SCRATCH(6, 32 * n, d_k);
+    const int rc = kb_schnorr_sign_run(ctx, n, secrets, nonces, msg, msg_off, mbytes, sig, pk, d_x, d_k);
+    // the secrets and nonces do not outlive the call, on the error paths either
+    cudaMemsetAsync(d_x, 0, 32 * n, ctx->stream);
+    cudaMemsetAsync(d_k, 0, 32 * n, ctx->stream);
     if (rc != KB_OK) {
         cudaStreamSynchronize(ctx->stream);
         return rc;

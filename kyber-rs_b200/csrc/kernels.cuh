@@ -46,7 +46,7 @@ __device__ __forceinline__ void kb_stage(uint32_t* dst, const uint32_t* src, int
     __syncthreads();
 }
 
-// Kernel groups: a translation unit defines KB_K_POINT / KB_K_SIGN / KB_K_POLY / KB_K_MSM / KB_K_KEYSET for the non-template kernels it
+// Kernel groups: a translation unit defines KB_K_POINT / KB_K_SIGN / KB_K_SIGNER / KB_K_POLY / KB_K_MSM / KB_K_KEYSET for the non-template kernels it
 // launches (nvcc compiles every __global__ function it sees, used or not).
 #if defined(KB_K_POINT)
 // ---- base-point table: table[w*8 + j] = (j+1) * 16^w * B, w = 0..63 (replaces constants.rs:89 BASE)
@@ -416,62 +416,175 @@ static __global__ void __launch_bounds__(KB_THREADS) k_challenge(size_t n, const
 }
 
 #endif  // KB_K_POINT
-#if defined(KB_K_SIGN)
+#if defined(KB_K_SIGN) || defined(KB_K_SIGNER)
 // ---- EdDSA::sign (sign/eddsa/eddsa_sig.rs:120-152) with the key derivation of
 // Curve::new_key_and_seed_with_input (group/edwards25519/curve.rs:74-87), three launches:
 //   k_sign_stage1   (a, prefix) = clamp(SHA-512(seed)); r = SHA-512(prefix || M) mod L; r*B and a*B (constant-time comb)
 //   k_compress_batch on the 2n points  ->  R and A encodings
 //   k_sign_finish   h = SHA-512(R || A || M) mod L; s = (r + h*a) mod L; sig = R || s
 // The secret scalars a and r only ever meet the constant-time select (no secret-dependent address or branch).
+//
+// schnorr::sign (sign/schnorr/schnorr_sig.rs:25-47) is the same chain without the derivation: k_schnorr_sign_stage1 computes
+// k*B and x*B from the caller's nonce and secret, and k_sign_finish reads x and k where the caller's buffers hold them.
+//
+// Signer sets (capi_signer.cu) hold x or (a, prefix) and A per key, so a signature pays one comb instead of two:
+//   k_signer_stage1<EDDSA>   r = SHA-512(prefix || M) mod L (EdDSA) or r = the caller's nonce (Schnorr); r*B
+//   k_compress_batch on the n points  ->  R encodings (zero where the key index is outside the set)
+//   k_signer_finish          h = SHA-512(R || A || M) mod L; s = (r + h*a) mod L from the set's a and A
+__device__ __forceinline__ void kb_sign_stage_base(ge_precomp* base, const ge_precomp* table)
+{
+    kb_stage(reinterpret_cast<uint32_t*>(base), reinterpret_cast<const uint32_t*>(table), 64 * 8 * 24);
+}
+// s*B through the constant-time select of the 48 KiB table staged in shared memory, into item i of xyz
+__device__ __forceinline__ void kb_sign_comb(uint32_t* xyz, size_t i, const uint32_t* s, const ge_precomp* base)
+{
+    int8_t e[64];
+    ge_p3 h;
+    sc_recode16(e, s);
+    ge_scalarmult_base<true>(h, e, base);
+    kb_store_xyz(xyz, i, h);
+}
+// Curve::new_key_and_seed_with_input (curve.rs:74-87): a = clamp(SHA-512(seed)[0..32]), prefix = SHA-512(seed)[32..64]
+__device__ __forceinline__ void kb_eddsa_derive(uint32_t* a, uint32_t* prefix, const uint32_t* seed)
+{
+    uint32_t d[16];
+    sha512_prefixed<8>(d, seed, nullptr, 0);
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+        a[k] = d[k];
+        prefix[k] = d[8 + k];
+    }
+    a[0] &= 0xfffffff8u;                     // digest[0] &= 0xf8
+    a[7] = (a[7] & 0x7fffffffu) | 0x40000000u;  // digest[31] &= 0x7f; |= 0x40   (unreduced scalar, SURVEY §A3)
+}
+// sig[i] = R || (r + h*a) mod L with h = SHA-512(R || A || M) mod L (eddsa_sig.rs:120-152, schnorr_sig.rs:25-47)
+__device__ __forceinline__ void kb_sign_close(uint8_t* sig, size_t i, const uint32_t* rw, const uint32_t* aw, const uint8_t* m, uint64_t mlen, const uint32_t* a, const uint32_t* r)
+{
+    uint32_t d[16], h[8], s[8];
+    sha512_ram(d, rw, aw, m, mlen);
+    sc_reduce512(h, d);
+    sc_muladd(s, h, a, r);
+    kb_store32(sig, 2 * i, rw);
+    kb_store32(sig, 2 * i + 1, s);
+}
+#endif  // KB_K_SIGN || KB_K_SIGNER
+#if defined(KB_K_SIGN)
 static __global__ void __launch_bounds__(KB_THREADS) k_sign_stage1(size_t n, const uint8_t* seeds, const uint8_t* msg, const uint64_t* msg_off, uint32_t* xyz, uint8_t* a_out, uint8_t* r_out,
                                                             const ge_precomp* table)
 {
     extern __shared__ uint4 smem4[];
     ge_precomp* base = reinterpret_cast<ge_precomp*>(smem4);
-    kb_stage(reinterpret_cast<uint32_t*>(base), reinterpret_cast<const uint32_t*>(table), 64 * 8 * 24);
+    kb_sign_stage_base(base, table);
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    uint32_t seed[8], d[16], a[8], r[8];
+    uint32_t seed[8], prefix[8], a[8], r[8];
     kb_load32(seed, seeds, i);
-    sha512_prefixed<8>(d, seed, nullptr, 0);
-#pragma unroll
-    for (int k = 0; k < 8; k++) a[k] = d[k];
-    a[0] &= 0xfffffff8u;                     // digest[0] &= 0xf8
-    a[7] = (a[7] & 0x7fffffffu) | 0x40000000u;  // digest[31] &= 0x7f; |= 0x40   (unreduced scalar, SURVEY §A3)
+    kb_eddsa_derive(a, prefix, seed);
     const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
     uint32_t d2[16];
-    sha512_prefixed<8>(d2, d + 8, msg + lo, hi - lo);   // prefix = digest[32..64]
+    sha512_prefixed<8>(d2, prefix, msg + lo, hi - lo);
     sc_reduce512(r, d2);
-    int8_t e[64];
-    ge_p3 h;
-    sc_recode16(e, r);
-    ge_scalarmult_base<true>(h, e, base);
-    kb_store_xyz(xyz, 2 * i, h);
-    sc_recode16(e, a);
-    ge_scalarmult_base<true>(h, e, base);
-    kb_store_xyz(xyz, 2 * i + 1, h);
+    kb_sign_comb(xyz, 2 * i, r, base);
+    kb_sign_comb(xyz, 2 * i + 1, a, base);
     kb_store32(a_out, i, a);
     kb_store32(r_out, i, r);
+}
+// (k*B, x*B) as items (2i, 2i + 1) of xyz; the scalars are used raw, as kb_point_mul_base_batch uses them
+static __global__ void __launch_bounds__(KB_THREADS) k_schnorr_sign_stage1(size_t n, const uint8_t* secrets, const uint8_t* nonces, uint32_t* xyz, const ge_precomp* table)
+{
+    extern __shared__ uint4 smem4[];
+    ge_precomp* base = reinterpret_cast<ge_precomp*>(smem4);
+    kb_sign_stage_base(base, table);
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint32_t s[8];
+    kb_load32(s, nonces, i);
+    kb_sign_comb(xyz, 2 * i, s, base);
+    kb_load32(s, secrets, i);
+    kb_sign_comb(xyz, 2 * i + 1, s, base);
 }
 static __global__ void __launch_bounds__(KB_THREADS) k_sign_finish(size_t n, const uint8_t* ra, const uint8_t* msg, const uint64_t* msg_off, const uint8_t* a_in, const uint8_t* r_in, uint8_t* sig, uint8_t* pk)
 {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    uint32_t rw[8], aw[8], d[16], h[8], a[8], r[8], s[8];
+    uint32_t rw[8], aw[8], a[8], r[8];
     kb_load32(rw, ra, 2 * i);
     kb_load32(aw, ra, 2 * i + 1);
-    const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
-    sha512_ram(d, rw, aw, msg + lo, hi - lo);
-    sc_reduce512(h, d);
     kb_load32(a, a_in, i);
     kb_load32(r, r_in, i);
-    sc_muladd(s, h, a, r);
-    kb_store32(sig, 2 * i, rw);
-    kb_store32(sig, 2 * i + 1, s);
+    const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
+    kb_sign_close(sig, i, rw, aw, msg + lo, hi - lo, a, r);
     if (pk) kb_store32(pk, i, aw);
 }
 
 #endif  // KB_K_SIGN
+#if defined(KB_K_SIGNER)
+// ---- signer sets: per key, sec = x (Schnorr) or a (EdDSA), prefix (EdDSA only) and A, 32 bytes each
+static __global__ void __launch_bounds__(KB_THREADS) k_signer_derive(size_t nkeys, const uint8_t* seeds, uint8_t* sec, uint8_t* prefix)
+{
+    const size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= nkeys) return;
+    uint32_t seed[8], a[8], p[8];
+    kb_load32(seed, seeds, k);
+    kb_eddsa_derive(a, p, seed);
+    kb_store32(sec, k, a);
+    kb_store32(prefix, k, p);
+}
+// R = r*B for item i under key key_idx[i]: r = SHA-512(prefix || M_i) mod L, kept in r_out for the finish (EDDSA), or r =
+// nonces[i] (Schnorr).  An index outside the set reads nothing of it and gives the identity with status 0xFF.
+template <bool EDDSA>
+static __global__ void __launch_bounds__(KB_THREADS) k_signer_stage1(size_t n, const uint32_t* key_idx, size_t nkeys, const uint8_t* prefix, const uint8_t* nonces, const uint8_t* msg,
+                                                                     const uint64_t* msg_off, uint32_t* xyz, uint8_t* r_out, uint8_t* status, const ge_precomp* table)
+{
+    extern __shared__ uint4 smem4[];
+    ge_precomp* base = reinterpret_cast<ge_precomp*>(smem4);
+    kb_sign_stage_base(base, table);
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t k = __ldg(key_idx + i);
+    status[i] = k < nkeys ? 0 : 0xFF;
+    if (k >= nkeys) {
+        ge_p3 h;
+        ge_identity(h);
+        kb_store_xyz(xyz, i, h);
+        return;
+    }
+    uint32_t r[8];
+    if (EDDSA) {
+        uint32_t p[8], d[16];
+        kb_load32(p, prefix, k);
+        const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
+        sha512_prefixed<8>(d, p, msg + lo, hi - lo);
+        sc_reduce512(r, d);
+        kb_store32(r_out, i, r);
+    } else {
+        kb_load32(r, nonces, i);
+    }
+    kb_sign_comb(xyz, i, r, base);
+}
+// sig[i] from R (k_compress_batch), the set's a and A, and r (r_in: the EdDSA scratch or the Schnorr nonces); 64 zero bytes
+// where the key index is outside the set
+static __global__ void __launch_bounds__(KB_THREADS) k_signer_finish(size_t n, const uint32_t* key_idx, size_t nkeys, const uint8_t* sec, const uint8_t* kpk, const uint8_t* r_enc,
+                                                                     const uint8_t* msg, const uint64_t* msg_off, const uint8_t* r_in, uint8_t* sig)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t k = __ldg(key_idx + i);
+    if (k >= nkeys) {
+        const uint32_t z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+        kb_store32(sig, 2 * i, z);
+        kb_store32(sig, 2 * i + 1, z);
+        return;
+    }
+    uint32_t rw[8], aw[8], a[8], r[8];
+    kb_load32(rw, r_enc, i);
+    kb_load32(aw, kpk, k);
+    kb_load32(a, sec, k);
+    kb_load32(r, r_in, i);
+    const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
+    kb_sign_close(sig, i, rw, aw, msg + lo, hi - lo, a, r);
+}
+#endif  // KB_K_SIGNER
 // ---- eddsa::verify_with_checks / schnorr::verify_with_checks, two launches (ops.cuh: sig_stage1 / sig_finish)
 #ifndef KB_VERIFY_MINBLOCKS
 #define KB_VERIFY_MINBLOCKS 3

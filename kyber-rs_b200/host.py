@@ -362,16 +362,13 @@ def find_pub(points, to_find: Point, ctx: Context | None = None):
 def schnorr_sign_batch(privates, msgs, nonces, ctx: Context | None = None):
     """schnorr::sign (sign/schnorr/schnorr_sig.rs:25-47) for n (private scalar, message) pairs with the
     nonces k supplied by the caller (the reference draws them from its RNG): R = k*B, h = H(R || A || M),
-    s = k + x*h.  Returns (signatures[n,64], public keys[n,32]).  The fixed-base mults run constant-time."""
+    s = k + x*h.  Returns (signatures[n,64], public keys[n,32]).  One C-ABI call (kb_schnorr_sign_batch): both
+    fixed-base multiplications run constant-time, and the secrets and nonces are wiped from device scratch."""
     ctx = ctx or default_context()
     x = np.frombuffer(b"".join(s.v if isinstance(s, Scalar) else bytes(s) for s in privates), np.uint8).reshape(-1, 32)
     k = np.frombuffer(b"".join(s.v if isinstance(s, Scalar) else bytes(s) for s in nonces), np.uint8).reshape(-1, 32)
     flat, off = pack_messages(list(msgs))
-    pub = ctx.point_mul_base_batch(x)
-    r = ctx.point_mul_base_batch(k)
-    h = ctx.challenge_batch(r, pub, flat, off)
-    s = ctx.sc_muladd_batch(x, h, k)
-    return np.concatenate([r, s], axis=1), pub
+    return ctx.schnorr_sign_batch(x, k, flat, off)
 
 
 def _xy_commit(shares, t: int):

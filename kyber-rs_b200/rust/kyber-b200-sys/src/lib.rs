@@ -24,6 +24,19 @@ pub struct kb_mkeyset {
     _private: [u8; 0],
 }
 
+#[repr(C)]
+pub struct kb_signerset {
+    _private: [u8; 0],
+}
+
+#[repr(C)]
+pub struct kb_msignerset {
+    _private: [u8; 0],
+}
+
+pub const KB_SIGNER_SCHNORR: c_int = 0;
+pub const KB_SIGNER_EDDSA: c_int = 1;
+
 pub const KB_OK: c_int = 0;
 pub const KB_ERR_NCCL: c_int = -4;
 pub const KB_ERR_ARG: c_int = -1;
@@ -70,6 +83,13 @@ extern "C" {
     pub fn kb_dev_keyset_mul(ks: *mut kb_keyset, n: usize, d_key_idx: *const c_void, d_scalars: *const c_void, d_out: *mut c_void, d_status: *mut c_void, flags: u32, stream: *mut c_void) -> c_int;
 
     pub fn kb_eddsa_sign_batch(ctx: *mut kb_ctx, n: usize, seeds: *const u8, msg: *const u8, msg_off: *const u64, sig: *mut u8, pk: *mut u8) -> c_int;
+    pub fn kb_schnorr_sign_batch(ctx: *mut kb_ctx, n: usize, secrets: *const u8, nonces: *const u8, msg: *const u8, msg_off: *const u64, sig: *mut u8, pk: *mut u8) -> c_int;
+    pub fn kb_dev_schnorr_sign(ctx: *mut kb_ctx, n: usize, d_secrets: *const c_void, d_nonces: *const c_void, d_msg: *const c_void, d_msg_off: *const c_void, d_sig: *mut c_void, d_pk: *mut c_void, stream: *mut c_void) -> c_int;
+    // signer sets: signing under registered secret keys (kind: KB_SIGNER_SCHNORR or KB_SIGNER_EDDSA)
+    pub fn kb_signerset_create(ctx: *mut kb_ctx, nkeys: usize, keys: *const u8, kind: c_int, pk_out: *mut u8, out: *mut *mut kb_signerset) -> c_int;
+    pub fn kb_signerset_destroy(ss: *mut kb_signerset);
+    pub fn kb_signerset_sign_batch(ss: *mut kb_signerset, n: usize, key_idx: *const u32, nonces: *const u8, msg: *const u8, msg_off: *const u64, sig: *mut u8) -> c_int;
+    pub fn kb_dev_signerset_sign(ss: *mut kb_signerset, n: usize, d_key_idx: *const c_void, d_nonces: *const c_void, d_msg: *const c_void, d_msg_off: *const c_void, d_sig: *mut c_void, d_status: *mut c_void, stream: *mut c_void) -> c_int;
 
     pub fn kb_pubpoly_eval_batch(ctx: *mut kb_ctx, npoly: usize, t: usize, commits: *const u8, m: usize, poly_id: *const u32, idx: *const u32, out: *mut u8, status: *mut u8) -> c_int;
     pub fn kb_vss_verify_deals_batch(ctx: *mut kb_ctx, npoly: usize, t: usize, commits: *const u8, m: usize, poly_id: *const u32, idx: *const u32, shares: *const u8, verdict: *mut u8) -> c_int;
@@ -140,6 +160,10 @@ extern "C" {
         commits: *const c_void, shares: *const u8, verdict: *mut u8,
         deal_msg: *const u8, deal_msg_off: *const u64, deal_sig: *const u8, deal_status: *mut u8,
         resp_msg: *const u8, resp_msg_off: *const u64, resp_sig: *const u8, resp_status: *mut u8) -> c_int;
+    pub fn kb_mctx_schnorr_sign_batch(m: *mut kb_mctx, n: usize, secrets: *const u8, nonces: *const u8, msg: *const u8, msg_off: *const u64, sig: *mut u8, pk: *mut u8) -> c_int;
+    pub fn kb_mctx_signerset_create(m: *mut kb_mctx, nkeys: usize, keys: *const u8, kind: c_int, pk_out: *mut u8, out: *mut *mut kb_msignerset) -> c_int;
+    pub fn kb_mctx_signerset_destroy(ss: *mut kb_msignerset);
+    pub fn kb_mctx_signerset_sign_batch(ss: *mut kb_msignerset, n: usize, key_idx: *const u32, nonces: *const u8, msg: *const u8, msg_off: *const u64, sig: *mut u8) -> c_int;
     pub fn kb_mctx_msm(m: *mut kb_mctx, n: usize, scalars: *const u8, points: *const u8, out32: *mut u8, bad_points: *mut u64) -> c_int;
 
     pub fn kb_probe_imad(ctx: *mut kb_ctx, kind: c_int, iters: c_int, macs_per_sec: *mut c_double, elapsed_ms: *mut c_double) -> c_int;

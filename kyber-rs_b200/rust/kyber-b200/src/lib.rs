@@ -220,6 +220,87 @@ impl Drop for KeySet<'_> {
     }
 }
 
+/// Batch companion of `schnorr::sign` (sign/schnorr/schnorr_sig.rs:25-47).  Items are (secret x, nonce k, message); the
+/// reference draws k from its random stream, here the caller supplies it (the library cannot detect a reused nonce, and
+/// a nonce used twice under one key reveals that key).  Returns the 64-byte signatures R || s and the public keys x*B.
+pub fn schnorr_sign_batch(gpu: &Gpu, items: &[(EdScalar, EdScalar, &[u8])]) -> Result<(Vec<[u8; 64]>, Vec<EdPoint>), GpuError> {
+    let n = items.len();
+    let x = pack_scalars(&items.iter().map(|(x, _, _)| x.clone()).collect::<Vec<_>>());
+    let k = pack_scalars(&items.iter().map(|(_, k, _)| k.clone()).collect::<Vec<_>>());
+    let (msg, off) = pack_messages(items.iter().map(|(_, _, m)| *m));
+    let mut sig = vec![0u8; 64 * n];
+    let mut pk = vec![0u8; 32 * n];
+    gpu.check(unsafe { sys::kb_schnorr_sign_batch(gpu.ctx, n, x.as_ptr(), k.as_ptr(), msg.as_ptr(), off.as_ptr(), sig.as_mut_ptr(), pk.as_mut_ptr()) })?;
+    Ok((unpack_sigs(&sig), unpack_points(&pk)))
+}
+
+fn pack_messages<'m>(msgs: impl Iterator<Item = &'m [u8]>) -> (Vec<u8>, Vec<u64>) {
+    let (mut msg, mut off) = (vec![], vec![0u64]);
+    for m in msgs {
+        msg.extend_from_slice(m);
+        off.push(msg.len() as u64);
+    }
+    (msg, off)
+}
+fn unpack_sigs(b: &[u8]) -> Vec<[u8; 64]> {
+    b.chunks(64).map(|c| c.try_into().expect("64 bytes")).collect()
+}
+
+/// Which signing function a `SignerSet` serves.
+#[derive(Clone, Copy, PartialEq, Eq, Debug)]
+pub enum SignerKind {
+    /// keys are secret scalars x; `schnorr::sign` (schnorr_sig.rs:25-47), nonces from the caller
+    Schnorr,
+    /// keys are 32-byte seeds; `EdDSA::sign` (eddsa_sig.rs:120-152) with the key derivation of curve.rs:74-87,
+    /// deterministic nonces
+    EdDSA,
+}
+
+/// Secret keys registered once with a `Gpu` — the key each participant of a DKG round signs its deals and responses
+/// with — so that a signature pays one constant-time fixed-base multiplication instead of two.  Signatures are byte for
+/// byte those of `schnorr_sign_batch` / `kb_eddsa_sign_batch` under the same key.  Borrows the `Gpu`: a signer set is
+/// dropped before its context; dropping it zeroes the keys on the device.
+pub struct SignerSet<'a> {
+    gpu: &'a Gpu,
+    ss: *mut sys::kb_signerset,
+    nkeys: usize,
+    kind: SignerKind,
+    /// the public key of each registered key (x*B or a*B)
+    pub public: Vec<EdPoint>,
+}
+
+impl<'a> SignerSet<'a> {
+    /// Registers `keys`: secret scalars (`SignerKind::Schnorr`, their raw 32 bytes) or seeds (`SignerKind::EdDSA`).
+    pub fn new(gpu: &'a Gpu, keys: &[[u8; 32]], kind: SignerKind) -> Result<Self, GpuError> {
+        let flat: Vec<u8> = keys.iter().flat_map(|k| k.iter().copied()).collect();
+        let mut pk = vec![0u8; 32 * keys.len()];
+        let mut ss = std::ptr::null_mut();
+        let k = if kind == SignerKind::EdDSA { sys::KB_SIGNER_EDDSA } else { sys::KB_SIGNER_SCHNORR };
+        gpu.check(unsafe { sys::kb_signerset_create(gpu.ctx, keys.len(), flat.as_ptr(), k, pk.as_mut_ptr(), &mut ss) })?;
+        Ok(SignerSet { gpu, ss, nkeys: keys.len(), kind, public: unpack_points(&pk) })
+    }
+    /// Items are (key index, message); `nonces` holds one nonce per item for a Schnorr set and must be `None` for an
+    /// EdDSA set.  A key index outside the set or the other nonce / kind combination is `GpuError::Arg`.
+    pub fn sign_batch(&self, items: &[(u32, &[u8])], nonces: Option<&[EdScalar]>) -> Result<Vec<[u8; 64]>, GpuError> {
+        let n = items.len();
+        if items.iter().any(|(k, _)| *k as usize >= self.nkeys) || (self.kind == SignerKind::Schnorr) != nonces.is_some() || nonces.map_or(false, |k| k.len() != n) {
+            return Err(GpuError::Arg);
+        }
+        let key_idx: Vec<u32> = items.iter().map(|(k, _)| *k).collect();
+        let (msg, off) = pack_messages(items.iter().map(|(_, m)| *m));
+        let k = nonces.map(pack_scalars);
+        let mut sig = vec![0u8; 64 * n];
+        let kp = k.as_ref().map_or(std::ptr::null(), |v| v.as_ptr());
+        self.gpu.check(unsafe { sys::kb_signerset_sign_batch(self.ss, n, key_idx.as_ptr(), kp, msg.as_ptr(), off.as_ptr(), sig.as_mut_ptr()) })?;
+        Ok(unpack_sigs(&sig))
+    }
+}
+impl Drop for SignerSet<'_> {
+    fn drop(&mut self) {
+        unsafe { sys::kb_signerset_destroy(self.ss) }
+    }
+}
+
 /// Batch companion of `PubPoly::eval` / `PubPoly::check` (share/poly.rs:457-469, :526-530) — the
 /// group math of `Aggregator::verify_deal` (share/vss/pedersen/vss.rs:899-912).
 pub trait PubPolyBatch {
