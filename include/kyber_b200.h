@@ -178,6 +178,24 @@ int  kb_keyset_verify_batch(kb_keyset* ks, size_t n, const uint32_t* key_idx, co
  * for that item, and the kernel reads nothing of the key set for it. */
 int  kb_dev_keyset_verify(kb_keyset* ks, size_t n, const void* d_key_idx, const void* d_msg, const void* d_msg_off,
                           const void* d_sig, void* d_status, int schnorr, void* stream);
+/* eddsa::verify_with_checks / schnorr::verify_with_checks x n, with the 32 pk bytes of every item given, under a key set:
+ * an item whose pk bytes equal a registered key's bytes is verified from that key's comb, every other item by the
+ * general verifier.  status[i] equals what kb_eddsa_verify_batch / kb_schnorr_verify_batch returns for item i.
+ * hits (may be NULL) receives the number of items that took the comb path.
+ * The match is on the bytes, not on the point: a registered key that is small-order, not canonical or undecodable is a
+ * hit (and gets the status the general verifier gives it), another encoding of a registered point is a miss.  Keys
+ * registered twice match the lowest index.  The lookup is a table built by kb_keyset_create under a seed drawn per set,
+ * and reads at most as many slots as the longest run of the registered keys.  The general verifier here is always the
+ * default half-size-scalar path, whatever KB_VERIFY_FULL / KB_VERIFY_SPLIT say (the statuses are the same).
+ * Arguments as kb_eddsa_verify_batch, plus KB_ERR_ARG for a NULL key set or n >= 2^32; n == 0 returns KB_OK and writes
+ * nothing.  An unknown key is not an error: there is no 0xFF status.  The host form stages the whole batch in one copy
+ * (no pipelined chunks as kb_eddsa_verify_batch has). */
+int  kb_keyset_verify_pk_batch(kb_keyset* ks, size_t n, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off,
+                               const uint8_t* sig, uint8_t* status, int schnorr, uint64_t* hits);
+/* device buffers + stream, ordered like every kb_dev_* call of the context; d_hits (may be NULL) is one uint64 on the
+ * device.  Only enqueues work: the split into the two sub-batches and their counts stay on the device. */
+int  kb_dev_keyset_verify_pk(kb_keyset* ks, size_t n, const void* d_pk, const void* d_msg, const void* d_msg_off,
+                             const void* d_sig, void* d_status, int schnorr, void* d_hits, void* stream);
 /* out[i] = compress(scalars[i] * keys[key_idx[i]]): Point::mul(s, Some(p)) with a registered p (point.rs:207,
  * ge.rs:508), the Diffie-Hellman step dh_exchange(secret, remote_public) (dh/dh_impl.rs:74-80) of encrypted_deal and
  * ECIES.  out and status are byte for byte what kb_point_mul_batch(ctx, n, scalars, keys[key_idx], out, status, flags)
@@ -419,6 +437,10 @@ void kb_mctx_keyset_destroy(kb_mkeyset* ks);
  * (KB_ERR_ARG); each device copies only the message bytes of its own items. */
 int  kb_mctx_keyset_verify_batch(kb_mkeyset* ks, size_t n, const uint32_t* key_idx, const uint8_t* msg, const uint64_t* msg_off,
                                  const uint8_t* sig, uint8_t* status, int schnorr);
+/* kb_keyset_verify_pk_batch split by index over all devices.  The arguments are checked before any device starts
+ * (KB_ERR_ARG); each device copies only the message bytes of its own items.  hits (may be NULL) is the sum over devices. */
+int  kb_mctx_keyset_verify_pk_batch(kb_mkeyset* ks, size_t n, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off,
+                                    const uint8_t* sig, uint8_t* status, int schnorr, uint64_t* hits);
 /* kb_keyset_mul_batch split by index over all devices, each against its own copy of the key set.  Flags and every key
  * index are checked before any device starts (KB_ERR_ARG). */
 int  kb_mctx_keyset_mul_batch(kb_mkeyset* ks, size_t n, const uint32_t* key_idx, const uint8_t* scalars, uint8_t* out,

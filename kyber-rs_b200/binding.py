@@ -51,6 +51,7 @@ EXPORTS = [
     "kb_dkg_process_round_keyed", "kb_dev_dkg_process_round_keyed",
     "kb_mctx_keyset_create", "kb_mctx_keyset_destroy", "kb_mctx_keyset_verify_batch", "kb_mctx_dkg_process_round_keyed",
     "kb_keyset_mul_batch", "kb_dev_keyset_mul", "kb_mctx_keyset_mul_batch",
+    "kb_keyset_verify_pk_batch", "kb_dev_keyset_verify_pk", "kb_mctx_keyset_verify_pk_batch",
     "kb_schnorr_sign_batch", "kb_dev_schnorr_sign", "kb_mctx_schnorr_sign_batch",
     "kb_signerset_create", "kb_signerset_destroy", "kb_signerset_sign_batch", "kb_dev_signerset_sign",
     "kb_mctx_signerset_create", "kb_mctx_signerset_destroy", "kb_mctx_signerset_sign_batch",
@@ -146,6 +147,8 @@ def load_library(path: str = LIB_PATH):
     L.kb_keyset_destroy.restype = None
     L.kb_keyset_verify_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32]
     L.kb_dev_keyset_verify.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32, vp]
+    L.kb_keyset_verify_pk_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32, vp]
+    L.kb_dev_keyset_verify_pk.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32, vp, vp]
     L.kb_keyset_mul_batch.argtypes = [vp, sz, vp, vp, vp, vp, u32]
     L.kb_dev_keyset_mul.argtypes = [vp, sz, vp, vp, vp, vp, u32, vp]
     L.kb_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8
@@ -154,6 +157,7 @@ def load_library(path: str = LIB_PATH):
     L.kb_mctx_keyset_destroy.argtypes = [vp]
     L.kb_mctx_keyset_destroy.restype = None
     L.kb_mctx_keyset_verify_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32]
+    L.kb_mctx_keyset_verify_pk_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, i32, vp]
     L.kb_mctx_keyset_mul_batch.argtypes = [vp, sz, vp, vp, vp, vp, u32]
     L.kb_mctx_dkg_process_round_keyed.argtypes = [vp, vp, vp, sz, sz, sz, i32, vp, vp, vp] + [vp] * 8
     L.kb_schnorr_sign_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp]
@@ -733,6 +737,21 @@ class KeySet:
         dp = Context._dp
         self.ctx._check(self.L.kb_dev_keyset_verify(self.h, n, dp(key_idx), dp(msg), dp(msg_off), dp(sig), dp(status), int(schnorr), Context._stream()), "kb_dev_keyset_verify")
 
+    def verify_pk_batch(self, pk, msg, msg_off, sig, schnorr=False, out=None, return_hits=False):
+        """Context.verify_batch(pk, msg, msg_off, sig, schnorr) status for status: items whose 32 pk bytes equal a registered
+        key's take that key's comb, every other item the general verifier.  With return_hits, (status, number of comb items)."""
+        n, pk, msg, msg_off, sig, st, hits = _verify_pk_args("KeySet.verify_pk_batch", pk, msg, msg_off, sig, out)
+        self.ctx._check(self.L.kb_keyset_verify_pk_batch(self.h, n, _ptr(pk), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(st), int(schnorr), _ptr(hits)),
+                        "kb_keyset_verify_pk_batch")
+        return (st, int(hits[0])) if return_hits else st
+
+    def dev_verify_pk(self, n, pk, msg, msg_off, sig, status, schnorr=False, hits=None):
+        """verify_pk_batch on CUDA tensors as Context.dev_verify takes them, on torch's current stream; hits: one int64 on the
+        device (or None) receives the number of comb items."""
+        dp = Context._dp
+        self.ctx._check(self.L.kb_dev_keyset_verify_pk(self.h, n, dp(pk), dp(msg), dp(msg_off), dp(sig), dp(status), int(schnorr), dp(hits), Context._stream()),
+                        "kb_dev_keyset_verify_pk")
+
     def mul_batch(self, key_idx, scalars, flags=0):
         """(out, status) = Context.point_mul_batch(scalars, keys[key_idx], flags) byte for byte, from the keys' combs:
         Point::mul(s, Some(pk)) of dh_exchange.  flags: 0 or FLAG_VARTIME."""
@@ -751,6 +770,17 @@ class KeySet:
         current stream; an index outside the set gives status 0xFF and 32 zero bytes."""
         dp = Context._dp
         self.ctx._check(self.L.kb_dev_keyset_mul(self.h, n, dp(key_idx), dp(scalars), dp(out), dp(status), flags, Context._stream()), "kb_dev_keyset_mul")
+
+
+def _verify_pk_args(what, pk, msg, msg_off, sig, out):
+    pk, sig = _u8(pk, (-1, 32)), _u8(sig, (-1, 64))
+    msg = _u8(msg)
+    msg_off = np.ascontiguousarray(msg_off, dtype=np.uint64)
+    n = pk.shape[0]
+    if sig.shape[0] != n or msg_off.shape[0] != n + 1:
+        raise ValueError(f"{what}: one pk and one signature per item, n+1 message offsets")
+    st = out if out is not None else np.empty(n, dtype=np.uint8)
+    return n, pk, msg, msg_off, sig, st, np.zeros(1, dtype=np.uint64)
 
 
 def _sign_args(what, n, key_idx, nonces, msg, msg_off):
@@ -974,6 +1004,13 @@ class MultiKeySet:
         st = out if out is not None else np.empty(n, dtype=np.uint8)
         self.mctx._check(self.L.kb_mctx_keyset_verify_batch(self.h, n, _ptr(key_idx), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(st), int(schnorr)), "kb_mctx_keyset_verify_batch")
         return st
+
+    def verify_pk_batch(self, pk, msg, msg_off, sig, schnorr=False, out=None, return_hits=False):
+        """KeySet.verify_pk_batch split by index over the devices; hits summed over them."""
+        n, pk, msg, msg_off, sig, st, hits = _verify_pk_args("MultiKeySet.verify_pk_batch", pk, msg, msg_off, sig, out)
+        self.mctx._check(self.L.kb_mctx_keyset_verify_pk_batch(self.h, n, _ptr(pk), _ptr(msg), _ptr(msg_off), _ptr(sig), _ptr(st), int(schnorr), _ptr(hits)),
+                         "kb_mctx_keyset_verify_pk_batch")
+        return (st, int(hits[0])) if return_hits else st
 
     def mul_batch(self, key_idx, scalars, flags=0):
         """KeySet.mul_batch split by index over the devices."""

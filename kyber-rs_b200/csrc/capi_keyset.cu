@@ -4,11 +4,18 @@
 #define KB_FE_MUL_RIP
 #define KB_FE_SQ_RIP
 #define KB_FE_SUBMASK
+#include <random>
+#include <vector>
+
 #include "ctx.cuh"
 #include "kernels.cuh"
 
 // One allocation per key set: the combs (KB_KEY_ENTRIES affine entries per key), then the 32-byte keys, then one byte of
 // facts per key.  It is not part of the context's scratch, so kb_ctx_wipe leaves it alone.
+// A second, small allocation holds the lookup table of kb_dev_keyset_verify_pk: open addressing with linear probing, one
+// key index per slot (KB_PK_MISS: empty), hmask + 1 >= 2 nkeys slots, hashed with kb_pk_hash under a seed drawn for this
+// set (a fixed hash would let whoever chooses the queried pks aim them at long runs).  hprobe is the longest run any
+// registered key needed; a lookup reads at most that many slots.
 struct kb_keyset {
     kb_ctx* ctx;
     size_t nkeys;
@@ -16,6 +23,9 @@ struct kb_keyset {
     ge_precomp* table;
     uint8_t* pk;
     uint8_t* facts;
+    uint32_t* htab;
+    uint32_t hmask, hprobe;
+    uint64_t hseed[2];
 };
 #define KB_KEY_TABLE_BYTES (sizeof(ge_precomp) * (size_t)KB_KEY_ENTRIES)
 static_assert(KB_KEY_TABLE_BYTES == 393216, "384 KiB of comb per key");
@@ -33,6 +43,103 @@ static int kb_keyset_launch(kb_keyset* ks, size_t n, const uint32_t* d_key_idx, 
     else k_verify_stage2<false><<<g2, KB_THREADS, 0, st>>>(n, xyz, fl, d_sig, d_status);
     KB_LAUNCHED();
     k_keyset_bad_index<<<kb_blocks(n, 256), 256, 0, st>>>(n, d_key_idx, ks->nkeys, d_status);
+    KB_LAUNCHED();
+    return KB_OK;
+}
+
+// the lookup table of the host keys pk[0 .. nkeys) (see kb_keyset), copied to ks->htab; a key whose bytes repeat an
+// earlier key's is not inserted, so a lookup finds the lowest index of equal bytes
+static int kb_keyset_build_lookup(kb_keyset* ks, const uint8_t* pk)
+{
+    kb_ctx* ctx = ks->ctx;
+    const size_t nkeys = ks->nkeys;
+    if (nkeys > ((size_t)1 << 31)) return KB_ERR_NOMEM;
+    size_t cap = 2;
+    while (cap < 2 * nkeys) cap <<= 1;
+    std::random_device rd;
+    for (int k = 0; k < 2; k++) ks->hseed[k] = ((uint64_t)rd() << 32) ^ (uint64_t)rd();
+    ks->hmask = (uint32_t)(cap - 1);
+    ks->hprobe = 0;
+    std::vector<uint32_t> tab(cap, KB_PK_MISS);
+    for (size_t k = 0; k < nkeys; k++) {
+        uint32_t w[8];
+        memcpy(w, pk + 32 * k, 32);   // little-endian words, as kb_load32 reads them on the device
+        const uint64_t h = kb_pk_hash(w, ks->hseed[0], ks->hseed[1]);
+        for (uint32_t p = 0;; p++) {
+            uint32_t& e = tab[kb_pk_slot(h, p, ks->hmask)];
+            if (e == KB_PK_MISS) {
+                e = (uint32_t)k;
+                if (p + 1 > ks->hprobe) ks->hprobe = p + 1;
+                break;
+            }
+            if (memcmp(pk + 32 * (size_t)e, pk + 32 * k, 32) == 0) break;
+        }
+    }
+    cudaError_t e = cudaMalloc(&ks->htab, 4 * cap);
+    if (e != cudaSuccess) {
+        kb_fail(ctx, e, "kb_keyset_create: cudaMalloc of the lookup table");
+        return KB_ERR_NOMEM;
+    }
+    e = cudaMemcpy(ks->htab, tab.data(), 4 * cap, cudaMemcpyHostToDevice);
+    return e == cudaSuccess ? KB_OK : kb_fail(ctx, e, "kb_keyset_create: copy of the lookup table");
+}
+
+// Scratch of kb_dev_keyset_verify_pk: kidx[n], hit_item[n], hit_key[n], miss_item[n], the per-block counts, then
+// {hits, misses}
+#define KB_SLOT_PK_PART 54
+// the launches of kb_dev_keyset_verify_pk; every grid is sized for n and every kernel after the scan reads its count from
+// the device, so nothing waits for the host
+static int kb_keyset_pk_launch(kb_keyset* ks, size_t n, const uint8_t* d_pk, const uint8_t* d_msg, const uint64_t* d_msg_off, const uint8_t* d_sig, uint8_t* d_status, int schnorr,
+                               unsigned long long* d_hits, cudaStream_t st)
+{
+    kb_ctx* ctx = ks->ctx;
+    const uint32_t nblk = kb_blocks(n, KB_PK_BLOCK);
+    uint32_t *part, *xyz;
+    uint8_t* fl;
+    KB_SCRATCH(KB_SLOT_PK_PART, 4 * (4 * n + nblk + 2), part);
+    KB_SCRATCH(KB_SLOT_XYZ, KB_VERIFY_SCRATCH_BYTES * n, xyz);
+    KB_SCRATCH(KB_SLOT_FLAGS, KB_VERIFY_FLAG_BYTES(n), fl);
+    uint32_t *kidx = part, *hit_item = part + n, *hit_key = part + 2 * n, *miss_item = part + 3 * n, *blk = part + 4 * n, *cnt = blk + nblk;
+    k_pk_lookup<<<nblk, KB_PK_BLOCK, 0, st>>>(n, d_pk, ks->htab, ks->hmask, ks->hprobe, ks->hseed[0], ks->hseed[1], ks->pk, kidx, blk);
+    KB_LAUNCHED();
+    k_pk_scan<<<1, 1024, 0, st>>>(n, nblk, blk, cnt, d_hits);
+    KB_LAUNCHED();
+    k_pk_scatter<<<nblk, KB_PK_BLOCK, 0, st>>>(n, kidx, blk, hit_item, hit_key, miss_item);
+    KB_LAUNCHED();
+    // hits: the comb path of kb_dev_keyset_verify, 96 bytes of xyz and one flag byte per slot
+    const unsigned g1 = kb_blocks(n, KB_THREADS), g2 = kb_blocks((n + KB_INV_K - 1) / KB_INV_K, KB_THREADS);
+    if (schnorr) k_keyset_verify_pk<true><<<g1, KB_THREADS, 0, st>>>(cnt, hit_item, hit_key, ks->pk, ks->facts, ks->table, d_msg, d_msg_off, d_sig, ctx->comb, xyz, fl);
+    else k_keyset_verify_pk<false><<<g1, KB_THREADS, 0, st>>>(cnt, hit_item, hit_key, ks->pk, ks->facts, ks->table, d_msg, d_msg_off, d_sig, ctx->comb, xyz, fl);
+    KB_LAUNCHED();
+    if (schnorr) k_verify_stage2_list<true><<<g2, KB_THREADS, 0, st>>>(cnt, hit_item, xyz, fl, d_sig, d_status);
+    else k_verify_stage2_list<false><<<g2, KB_THREADS, 0, st>>>(cnt, hit_item, xyz, fl, d_sig, d_status);
+    KB_LAUNCHED();
+    // misses: the default half-size-scalar path of kb_verify_launch (whatever KB_VERIFY_FULL / KB_VERIFY_SPLIT say: the
+    // statuses are the same), its records in xyz after the hits are done with it
+    const uint32_t* mcnt = cnt + 1;
+    const unsigned th = kb_item_threads(ctx, n);
+    if (schnorr) k_verify_half_prep_list<true><<<g1, KB_THREADS, 0, st>>>(n, mcnt, miss_item, d_pk, d_msg, d_msg_off, d_sig, xyz);
+    else k_verify_half_prep_list<false><<<g1, KB_THREADS, 0, st>>>(n, mcnt, miss_item, d_pk, d_msg, d_msg_off, d_sig, xyz);
+    KB_LAUNCHED();
+    const uint32_t* perm = nullptr;
+#if KB_HALF_JOINT
+    // sorted or not by the rule of kb_verify_launch, applied to the upper bound n
+    if (ctx->verify_sort && (n >= 16384 || ctx->verify_sort == 2)) {
+        uint32_t* pm = reinterpret_cast<uint32_t*>(fl);
+        uint8_t* keys = fl + 4 * n;
+        uint32_t* hist = reinterpret_cast<uint32_t*>(fl + ((5 * n + 255) & ~(size_t)255));
+        KB_CUDA(cudaMemsetAsync(hist, 0, 4 * KB_SORT_BINS, st));
+        k_half_sort_count_list<<<kb_blocks(n, 256), 256, 0, st>>>(mcnt, xyz, keys, hist);
+        KB_LAUNCHED();
+        k_half_sort_scan<<<1, 32, 0, st>>>(hist, hist + KB_SORT_BINS);
+        KB_LAUNCHED();
+        k_half_sort_scatter_list<<<kb_blocks(n, 256), 256, 0, st>>>(mcnt, keys, hist + KB_SORT_BINS, pm);
+        KB_LAUNCHED();
+        perm = pm;
+    }
+#endif
+    if (schnorr) k_verify_half_main_list<true><<<kb_blocks(n, th), th, 0, st>>>(n, mcnt, miss_item, xyz, perm, d_status, ctx->comb, ctx->verify_min_windows, ctx->verify_force_redo);
+    else k_verify_half_main_list<false><<<kb_blocks(n, th), th, 0, st>>>(n, mcnt, miss_item, xyz, perm, d_status, ctx->comb, ctx->verify_min_windows, ctx->verify_force_redo);
     KB_LAUNCHED();
     return KB_OK;
 }
@@ -128,6 +235,7 @@ int kb_keyset_create(kb_ctx* ctx, size_t nkeys, const uint8_t* pk, kb_keyset** o
         if (le == cudaSuccess) le = cudaStreamSynchronize(ctx->stream);
         if (le != cudaSuccess) rc = kb_fail(ctx, le, "kb_keyset_create: k_keyset_build");
     }
+    if (rc == KB_OK) rc = kb_keyset_build_lookup(ks, pk);
     if (rc != KB_OK) {
         kb_keyset_destroy(ks);
         return rc;
@@ -141,6 +249,7 @@ void kb_keyset_destroy(kb_keyset* ks)
     cudaSetDevice(ks->ctx->device);
     cudaDeviceSynchronize();   // verify calls on any stream may still read the combs
     if (ks->mem) cudaFree(ks->mem);
+    if (ks->htab) cudaFree(ks->htab);
     free(ks);
 }
 int kb_dev_keyset_verify(kb_keyset* ks, size_t n, const void* d_key_idx, const void* d_msg, const void* d_msg_off, const void* d_sig, void* d_status, int schnorr, void* stream)
@@ -190,6 +299,55 @@ int kb_keyset_verify_batch(kb_keyset* ks, size_t n, const uint32_t* key_idx, con
     }
     KB_D2H(status, d_st, n);
     KB_SYNC();
+    return KB_OK;
+}
+
+// ---- verification by public-key bytes: registered keys on the comb path, every other key on the general verifier
+int kb_dev_keyset_verify_pk(kb_keyset* ks, size_t n, const void* d_pk, const void* d_msg, const void* d_msg_off, const void* d_sig, void* d_status, int schnorr, void* d_hits, void* stream)
+{
+    if (!ks) return KB_ERR_ARG;
+    kb_ctx* ctx = ks->ctx;
+    if (n && (!d_pk || !d_msg_off || !d_sig || !d_status)) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    if (n > UINT32_MAX) return KB_ERR_ARG;   // item numbers are 32-bit in the sub-batch lists
+    cudaStream_t st = (cudaStream_t)stream;
+    KB_DEV_ENTER(st);
+    KB_DEV_RETURN(st, kb_keyset_pk_launch(ks, n, (const uint8_t*)d_pk, (const uint8_t*)d_msg, (const uint64_t*)d_msg_off, (const uint8_t*)d_sig, (uint8_t*)d_status, schnorr,
+                                          (unsigned long long*)d_hits, st));
+}
+// plain staging: copy in, the device form, copy out, all on the context's stream
+int kb_keyset_verify_pk_batch(kb_keyset* ks, size_t n, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off, const uint8_t* sig, uint8_t* status, int schnorr, uint64_t* hits)
+{
+    if (!ks) return KB_ERR_ARG;
+    kb_ctx* ctx = ks->ctx;
+    KB_ENTER();
+    if (n && (!pk || !msg_off || !sig || !status)) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    if (n > UINT32_MAX || !kb_msg_off_ok(n, msg_off)) return KB_ERR_ARG;
+    const size_t mbytes = (size_t)msg_off[n];
+    if (mbytes && !msg) return KB_ERR_ARG;
+    uint8_t *d_pk, *d_sig, *d_m, *d_st;
+    uint64_t *d_off, *d_hits;
+    KB_SCRATCH(0, 32 * n, d_pk);
+    KB_SCRATCH(1, 64 * n, d_sig);
+    KB_SCRATCH(2, mbytes, d_m);
+    KB_SCRATCH(3, 8 * (n + 1), d_off);
+    KB_SCRATCH(4, n, d_st);
+    KB_SCRATCH(5, 8, d_hits);
+    KB_H2D(d_pk, pk, 32 * n);
+    KB_H2D(d_sig, sig, 64 * n);
+    if (mbytes) KB_H2D(d_m, msg, mbytes);
+    KB_H2D(d_off, msg_off, 8 * (n + 1));
+    const int rc = kb_dev_keyset_verify_pk(ks, n, d_pk, d_m, d_off, d_sig, d_st, schnorr, d_hits, ctx->stream);
+    if (rc != KB_OK) {
+        cudaStreamSynchronize(ctx->stream);
+        return rc;
+    }
+    uint64_t h = 0;
+    KB_D2H(status, d_st, n);
+    KB_D2H(&h, d_hits, 8);
+    KB_SYNC();
+    if (hits) *hits = h;
     return KB_OK;
 }
 

@@ -249,6 +249,36 @@ int kb_mctx_keyset_verify_batch(kb_mkeyset* mk, size_t n, const uint32_t* key_id
         return rc;
     });
 }
+int kb_mctx_keyset_verify_pk_batch(kb_mkeyset* mk, size_t n, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off, const uint8_t* sig, uint8_t* status, int schnorr,
+                                   uint64_t* hits)
+{
+    if (!mk || (n && (!pk || !msg_off || !sig || !status))) return KB_ERR_ARG;
+    if (n == 0) return KB_OK;
+    kb_mctx* m = mk->m;
+    if ((n + m->ndev - 1) / m->ndev > UINT32_MAX) return KB_ERR_ARG;
+    if (!kb_msg_off_ok(n, msg_off) || (msg_off[n] != msg_off[0] && !msg)) return KB_ERR_ARG;
+    uint64_t h[KB_MAX_DEVICES] = {};
+    const int rc = kb_on_all(m, [&](int i) {
+        size_t lo, hi;
+        kb_shard(n, i, m->ndev, &lo, &hi);
+        if (hi == lo) return (int)KB_OK;
+        // the device is handed its own message bytes, with offsets made relative to the first of them
+        const size_t cn = hi - lo;
+        const uint64_t m0 = msg_off[lo];
+        uint64_t* off = (uint64_t*)malloc(8 * (cn + 1));
+        if (!off) return (int)KB_ERR_NOMEM;
+        for (size_t j = 0; j <= cn; j++) off[j] = msg_off[lo + j] - m0;
+        const int r = kb_keyset_verify_pk_batch(mk->ks[i], cn, pk + 32 * lo, msg ? msg + m0 : nullptr, off, sig + 64 * lo, status + lo, schnorr, &h[i]);
+        free(off);
+        return r;
+    });
+    if (rc == KB_OK && hits) {
+        uint64_t s = 0;
+        for (int i = 0; i < m->ndev; i++) s += h[i];
+        *hits = s;
+    }
+    return rc;
+}
 int kb_mctx_keyset_mul_batch(kb_mkeyset* mk, size_t n, const uint32_t* key_idx, const uint8_t* scalars, uint8_t* out, uint8_t* status, uint32_t flags)
 {
     if (!mk || (flags & ~KB_FLAG_VARTIME) || (n && (!key_idx || !scalars || !out))) return KB_ERR_ARG;

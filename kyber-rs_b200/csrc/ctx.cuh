@@ -140,6 +140,7 @@ int kb_dev_end(kb_ctx* ctx, cudaStream_t st);
 //   30, 31  forward-difference arrays B / decoded commitments
 //   32..45  two lanes of the pipelined host-buffer verify
 //   46..63  protocol-level entry points (capi_proto.cu) and the multi-device context
+//   54      the partition of kb_dev_keyset_verify_pk (capi_keyset.cu)
 
 // ---- drivers shared between translation units (each defined in the file named) -------------------------------------
 // capi_verify.cu: the two launches of a signature-verification batch on device buffers

@@ -719,6 +719,143 @@ static __global__ void __launch_bounds__(KB_THREADS) k_keyset_mul(size_t n, cons
     kb_store_xyz(xyz, i, h);
     status[i] = (uint8_t)st;
 }
+// ---- verification by public-key bytes (kb_dev_keyset_verify_pk): the pk of every item is looked up in the key set's
+// open-addressing table, the batch is split stably into the items whose 32 bytes equal a registered key's (hits: comb
+// path) and all others (misses: the general verifier), and both sub-batches run with their counts in device memory.
+#define KB_PK_MISS 0xffffffffu   // an empty table slot, and the key index of an item that is not registered
+#define KB_PK_BLOCK 256
+// the table's hash of 32 key bytes under the key set's seed (s0, s1); the host builds the table with the same function
+__host__ __device__ __forceinline__ uint64_t kb_pk_hash(const uint32_t* w, uint64_t s0, uint64_t s1)
+{
+    uint64_t h = s0;
+    for (int k = 0; k < 4; k++) {
+        h ^= ((uint64_t)w[2 * k + 1] << 32) | w[2 * k];
+        h *= 0x9e3779b97f4a7c15ull;
+        h ^= h >> 32;
+    }
+    h ^= s1;
+    h *= 0xbf58476d1ce4e5b9ull;
+    return h ^ (h >> 31);
+}
+__host__ __device__ __forceinline__ uint32_t kb_pk_slot(uint64_t h, uint32_t p, uint32_t mask) { return ((uint32_t)h + p) & mask; }
+// kidx[i] = the lowest index of a key whose bytes equal pk[i], or KB_PK_MISS; at most `probe` slots (the longest run of
+// the registered keys) are read whatever the query.  blk_hits[b] = the hits of block b.
+static __global__ void __launch_bounds__(KB_PK_BLOCK) k_pk_lookup(size_t n, const uint8_t* pk, const uint32_t* htab, uint32_t mask, uint32_t probe, uint64_t s0, uint64_t s1, const uint8_t* kpk,
+                                                                  uint32_t* kidx, uint32_t* blk_hits)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t k = KB_PK_MISS;
+    if (i < n) {
+        uint32_t w[8];
+        kb_load32(w, pk, i);
+        const uint64_t h = kb_pk_hash(w, s0, s1);
+        for (uint32_t p = 0; p < probe; p++) {
+            const uint32_t e = __ldg(htab + kb_pk_slot(h, p, mask));
+            if (e == KB_PK_MISS) break;
+            uint32_t kw[8], d = 0;
+            kb_load32(kw, kpk, e);
+#pragma unroll
+            for (int q = 0; q < 8; q++) d |= kw[q] ^ w[q];
+            if (d == 0) {
+                k = e;
+                break;
+            }
+        }
+        kidx[i] = k;
+    }
+    const int c = __syncthreads_count(k != KB_PK_MISS);
+    if (threadIdx.x == 0) blk_hits[blockIdx.x] = (uint32_t)c;
+}
+// one block of 1024: blk[b] becomes the hits before block b; counts = {hits, n - hits}; *hits_out = hits (if given)
+static __global__ void __launch_bounds__(1024) k_pk_scan(size_t n, uint32_t nblk, uint32_t* blk, uint32_t* counts, unsigned long long* hits_out)
+{
+    __shared__ uint32_t s_warp[32];
+    const uint32_t t = threadIdx.x, lane = t & 31, per = (nblk + blockDim.x - 1) / blockDim.x;
+    const uint32_t lo = min(t * per, nblk), hi = min(lo + per, nblk);
+    uint32_t sum = 0;
+    for (uint32_t b = lo; b < hi; b++) sum += blk[b];
+    uint32_t x = sum;   // inclusive scan over the threads
+#pragma unroll
+    for (int off = 1; off < 32; off <<= 1) {
+        const uint32_t y = __shfl_up_sync(0xffffffffu, x, off);
+        if (lane >= (uint32_t)off) x += y;
+    }
+    if (lane == 31) s_warp[t >> 5] = x;
+    __syncthreads();
+    if (t < 32) {
+        uint32_t w = s_warp[t];
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+            const uint32_t y = __shfl_up_sync(0xffffffffu, w, off);
+            if (lane >= (uint32_t)off) w += y;
+        }
+        s_warp[t] = w;
+    }
+    __syncthreads();
+    uint32_t excl = x - sum + (t >= 32 ? s_warp[(t >> 5) - 1] : 0u);
+    for (uint32_t b = lo; b < hi; b++) {
+        const uint32_t c = blk[b];
+        blk[b] = excl;
+        excl += c;
+    }
+    if (t == blockDim.x - 1) {
+        counts[0] = excl;
+        counts[1] = (uint32_t)(n - excl);
+        if (hits_out) *hits_out = excl;
+    }
+}
+// the stable partition: hit j = (hit_item[j], hit_key[j]), miss j = miss_item[j], both in item order
+static __global__ void __launch_bounds__(KB_PK_BLOCK) k_pk_scatter(size_t n, const uint32_t* kidx, const uint32_t* blk_off, uint32_t* hit_item, uint32_t* hit_key, uint32_t* miss_item)
+{
+    __shared__ uint32_t s_warp[KB_PK_BLOCK / 32];
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint32_t k = i < n ? __ldg(kidx + i) : KB_PK_MISS;
+    const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const uint32_t bal = __ballot_sync(0xffffffffu, k != KB_PK_MISS);
+    if (lane == 0) s_warp[wid] = __popc(bal);
+    __syncthreads();
+    uint32_t r = __popc(bal & ((1u << lane) - 1u));   // hits before this thread in the block
+    for (uint32_t w = 0; w < wid; w++) r += s_warp[w];
+    if (i >= n) return;
+    const uint32_t off = blk_off[blockIdx.x];
+    if (k != KB_PK_MISS) {
+        hit_item[off + r] = (uint32_t)i;
+        hit_key[off + r] = k;
+    } else {
+        miss_item[(size_t)blockIdx.x * KB_PK_BLOCK - off + (threadIdx.x - r)] = (uint32_t)i;   // every earlier block is full
+    }
+}
+// k_keyset_verify for hit j < *cnt: item hit_item[j] under key hit_key[j]; (X, Y, Z) and the flag byte go to slot j
+template <bool SCHNORR>
+static __global__ void __launch_bounds__(KB_THREADS) k_keyset_verify_pk(const uint32_t* cnt, const uint32_t* hit_item, const uint32_t* hit_key, const uint8_t* kpk, const uint8_t* facts,
+                                                                        const ge_precomp* ktab, const uint8_t* msg, const uint64_t* msg_off, const uint8_t* sig, const ge_precomp* comb,
+                                                                        uint32_t* xyz, uint8_t* flags)
+{
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= *cnt) return;
+    const size_t i = __ldg(hit_item + j), k = __ldg(hit_key + j);
+    uint32_t pw[8], sw[16];
+    kb_load32(pw, kpk, k);
+    const uint32_t kf = __ldg(facts + k);
+    kb_load32(sw, sig, 2 * i);
+    kb_load32(sw + 8, sig, 2 * i + 1);
+    const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
+    ge_p3 Q;
+    const uint32_t f = sig_keyset_stage1<SCHNORR>(Q, kf, pw, sw, msg + lo, hi - lo, comb, ktab + k * KB_KEY_ENTRIES);
+    kb_store_xyz(xyz, j, Q);
+    flags[j] = (uint8_t)f;
+}
+// k_verify_stage2 over the *cnt slots of k_keyset_verify_pk: the status of slot j goes to status[item[j]]
+template <bool SCHNORR>
+static __global__ void __launch_bounds__(KB_THREADS) k_verify_stage2_list(const uint32_t* cnt, const uint32_t* item, const uint32_t* xyz, const uint8_t* flags, const uint8_t* sig, uint8_t* status)
+{
+    kb_batch_compress(*cnt, xyz, [&](size_t j, uint32_t* enc) {
+        const size_t i = __ldg(item + j);
+        uint32_t rw[8];
+        kb_load32(rw, sig, 2 * i);
+        status[i] = (uint8_t)sig_finish<SCHNORR>(flags[j], enc, rw);
+    });
+}
 #endif  // KB_K_KEYSET
 
 // ---- the same verifiers with half-size scalars (ops.cuh sig_half_*, half.cuh): 128 doublings per signature,
@@ -835,9 +972,16 @@ __device__ __forceinline__ void kb_rec_load(kb_half_rec& rec, const uint32_t* o)
 #if KB_PREP_ROLES
 static __device__ unsigned int kb_prep_role_counter[1024];
 #endif
-template <bool SCHNORR>
-static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_PREP_MINBLOCKS) k_verify_half_prep(size_t n, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off, uint64_t msg_base, const uint8_t* sig, uint32_t* recs)
+// LIST (the sub-batches of kb_dev_keyset_verify_pk): the launch is sized for an upper bound, the real count is *cnt in device
+// memory, and record j is the preparation of the caller's item[j].  Without LIST, cnt and item are not read.
+template <bool SCHNORR, bool LIST>
+__device__ __forceinline__ void kb_verify_half_prep_run(size_t n, const uint32_t* cnt, const uint32_t* item, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off, uint64_t msg_base,
+                                                        const uint8_t* sig, uint32_t* recs)
 {
+    if constexpr (LIST) {
+        n = *cnt;
+        if ((size_t)blockIdx.x * blockDim.x >= n) return;   // whole blocks past the count (all of them when it is 0)
+    }
     int role = 0;
 #if KB_PREP_ROLES
     __shared__ unsigned int s_role;
@@ -855,10 +999,12 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_PREP_MINBLOCKS) k
 #else
     if (i >= n) return;
 #endif
+    size_t src = i;
+    if constexpr (LIST) src = __ldg(item + i);
     uint32_t pw[8], sw[16];
-    kb_load32(pw, pk, i);
-    kb_load32(sw, sig, 2 * i);
-    kb_load32(sw + 8, sig, 2 * i + 1);
+    kb_load32(pw, pk, src);
+    kb_load32(sw, sig, 2 * src);
+    kb_load32(sw + 8, sig, 2 * src + 1);
     uint32_t* o = kb_rec_at(recs, i);
     uint32_t dec = 0, f = 0, vneg = 0;
     int nwin = 0;
@@ -880,7 +1026,7 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_PREP_MINBLOCKS) k
             }
         } else {
             // msg_off holds offsets into the caller's whole message array; `msg` points at byte msg_base of it
-            const uint64_t lo = msg_off[i], hi = msg_off[i + 1];
+            const uint64_t lo = msg_off[src], hi = msg_off[src + 1];
             kb_half_sc sc;
             sig_half_scalars<SCHNORR>(sc, pw, sw, msg + (lo - msg_base), hi - lo);
             kb_rec_store_scalars(o, sc);
@@ -897,6 +1043,19 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_PREP_MINBLOCKS) k
     }
     kb_rec_store72_clear73(o, kb_rec_pack72(f, nwin, vneg));
 }
+template <bool SCHNORR>
+static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_PREP_MINBLOCKS) k_verify_half_prep(size_t n, const uint8_t* pk, const uint8_t* msg, const uint64_t* msg_off, uint64_t msg_base, const uint8_t* sig, uint32_t* recs)
+{
+    kb_verify_half_prep_run<SCHNORR, false>(n, nullptr, nullptr, pk, msg, msg_off, msg_base, sig, recs);
+}
+#if defined(KB_K_KEYSET)
+template <bool SCHNORR>
+static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_PREP_MINBLOCKS) k_verify_half_prep_list(size_t n, const uint32_t* cnt, const uint32_t* item, const uint8_t* pk, const uint8_t* msg,
+                                                                                                        const uint64_t* msg_off, const uint8_t* sig, uint32_t* recs)
+{
+    kb_verify_half_prep_run<SCHNORR, true>(n, cnt, item, pk, msg, msg_off, 0, sig, recs);
+}
+#endif
 // ---- the preparation as TWO kernels that share the SMs (KB_VERIFY_SPLIT=1, capi_verify.cu).  The phases of
 // k_verify_half_prep load different pipes and run one after the other in every block; here the "scalars" phase is a
 // PERSISTENT kernel of a few blocks per SM (work drawn from a counter) that is launched first on a side stream, and the
@@ -969,7 +1128,7 @@ static __global__ void __launch_bounds__(256) k_verify_half_fix(size_t n, uint32
 // pairs, 64.6 on average; a block of 128 random ones runs the maximum of its members, 66.4 on average.
 #define KB_SORT_BINS 129
 #if KB_HALF_JOINT
-static __global__ void __launch_bounds__(256) k_half_sort_count(size_t n, const uint32_t* recs, uint8_t* keys, uint32_t* hist)
+__device__ __forceinline__ void kb_half_sort_count_run(size_t n, const uint32_t* recs, uint8_t* keys, uint32_t* hist)
 {
     __shared__ uint32_t s_hist[KB_SORT_BINS];
     for (int k = threadIdx.x; k < KB_SORT_BINS; k += blockDim.x) s_hist[k] = 0;
@@ -986,6 +1145,7 @@ static __global__ void __launch_bounds__(256) k_half_sort_count(size_t n, const 
     for (int k = threadIdx.x; k < KB_SORT_BINS; k += blockDim.x)
         if (s_hist[k]) atomicAdd(&hist[k], s_hist[k]);
 }
+static __global__ void __launch_bounds__(256) k_half_sort_count(size_t n, const uint32_t* recs, uint8_t* keys, uint32_t* hist) { kb_half_sort_count_run(n, recs, keys, hist); }
 // first position of every bin, longest records first
 static __global__ void k_half_sort_scan(const uint32_t* hist, uint32_t* cursor)
 {
@@ -996,7 +1156,7 @@ static __global__ void k_half_sort_scan(const uint32_t* hist, uint32_t* cursor)
         pos += hist[k];
     }
 }
-static __global__ void __launch_bounds__(256) k_half_sort_scatter(size_t n, const uint8_t* keys, uint32_t* cursor, uint32_t* perm)
+__device__ __forceinline__ void kb_half_sort_scatter_run(size_t n, const uint8_t* keys, uint32_t* cursor, uint32_t* perm)
 {
     __shared__ uint32_t s_cnt[KB_SORT_BINS], s_base[KB_SORT_BINS];
     for (int k = threadIdx.x; k < KB_SORT_BINS; k += blockDim.x) s_cnt[k] = 0;
@@ -1013,6 +1173,12 @@ static __global__ void __launch_bounds__(256) k_half_sort_scatter(size_t n, cons
     __syncthreads();
     if (i < n) perm[s_base[key] + rank] = (uint32_t)i;
 }
+static __global__ void __launch_bounds__(256) k_half_sort_scatter(size_t n, const uint8_t* keys, uint32_t* cursor, uint32_t* perm) { kb_half_sort_scatter_run(n, keys, cursor, perm); }
+#if defined(KB_K_KEYSET)
+// the same over the *cnt records of a sub-batch (kb_dev_keyset_verify_pk)
+static __global__ void __launch_bounds__(256) k_half_sort_count_list(const uint32_t* cnt, const uint32_t* recs, uint8_t* keys, uint32_t* hist) { kb_half_sort_count_run(*cnt, recs, keys, hist); }
+static __global__ void __launch_bounds__(256) k_half_sort_scatter_list(const uint32_t* cnt, const uint8_t* keys, uint32_t* cursor, uint32_t* perm) { kb_half_sort_scatter_run(*cnt, keys, cursor, perm); }
+#endif
 #endif
 // Resident blocks per SM of the main kernel.  3 (168 registers, no spills) was the best setting while two radix-16 tables
 // sat in local memory (2 blocks: +5 %, 4: slower in round 1); with the joint table (1.7 KB per thread, a third of the DRAM
@@ -1049,9 +1215,15 @@ static __device__ __noinline__ uint32_t kb_verify_half_exact(const uint32_t* o, 
     return sig_half_finish<SCHNORR>(rec.f, W);
 }
 #endif
-template <bool SCHNORR>
-static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k_verify_half_main(size_t n, const uint32_t* recs, const uint32_t* perm, uint8_t* status, const ge_precomp* comb, int min_windows, int force_redo)
+// LIST: as kb_verify_half_prep_run — *cnt records, and the status of record j goes to status[item[j]]
+template <bool SCHNORR, bool LIST>
+__device__ __forceinline__ void kb_verify_half_main_run(size_t n, const uint32_t* cnt, const uint32_t* item, const uint32_t* recs, const uint32_t* perm, uint8_t* status, const ge_precomp* comb,
+                                                        int min_windows, int force_redo)
 {
+    if constexpr (LIST) {
+        n = *cnt;
+        if ((size_t)blockIdx.x * blockDim.x >= n) return;   // whole blocks past the count, before the first barrier
+    }
     __shared__ int s_nwin;
 #if KB_HALF_JOINT
     if (threadIdx.x == 0) s_nwin = 2 * min_windows;   // the joint loop counts radix-4 digit pairs
@@ -1090,7 +1262,7 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k
     ge_triple_scalarmult_joint<true>(W, nwin, dw, uk, vk, tbl, comb, fo);
     if (__any_sync(0xffffffffu, fo.ovf) && fo.ovf) {
         const uint32_t st = kb_verify_half_exact<SCHNORR>(kb_rec_at(recs, i), nwin, comb);
-        if (live) status[i] = (uint8_t)st;
+        if (live) status[LIST ? __ldg(item + i) : i] = (uint8_t)st;
         return;
     }
 #elif KB_HALF_PREFETCH
@@ -1098,8 +1270,21 @@ static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k
 #else
     ge_triple_scalarmult_vartime(W, nwin, dw, eu, ev, tbl, comb);
 #endif
-    if (live) status[i] = (uint8_t)sig_half_finish<SCHNORR>(rec.f, W);
+    if (live) status[LIST ? __ldg(item + i) : i] = (uint8_t)sig_half_finish<SCHNORR>(rec.f, W);
 }
+template <bool SCHNORR>
+static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k_verify_half_main(size_t n, const uint32_t* recs, const uint32_t* perm, uint8_t* status, const ge_precomp* comb, int min_windows, int force_redo)
+{
+    kb_verify_half_main_run<SCHNORR, false>(n, nullptr, nullptr, recs, perm, status, comb, min_windows, force_redo);
+}
+#if defined(KB_K_KEYSET)
+template <bool SCHNORR>
+static __global__ void __launch_bounds__(KB_THREADS, KB_VERIFY_HALF_MINBLOCKS) k_verify_half_main_list(size_t n, const uint32_t* cnt, const uint32_t* item, const uint32_t* recs, const uint32_t* perm,
+                                                                                                         uint8_t* status, const ge_precomp* comb, int min_windows, int force_redo)
+{
+    kb_verify_half_main_run<SCHNORR, true>(n, cnt, item, recs, perm, status, comb, min_windows, force_redo);
+}
+#endif
 
 #if defined(KB_K_POLY)
 // ---- committed polynomials

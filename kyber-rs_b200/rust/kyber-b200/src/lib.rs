@@ -192,6 +192,36 @@ impl<'a> KeySet<'a> {
         }
         Ok(res.into_iter().map(|r| r.unwrap()).collect())
     }
+    /// Items are (public key bytes, message, signature), as `verify_batch` takes them, with the same result item by item:
+    /// an item whose 32 key bytes equal a registered key's is verified from that key's comb, every other item by the
+    /// general verifier, in one call.  Also returns how many items took the comb path.
+    pub fn verify_pk_batch(&self, items: &[(&[u8], &[u8], &[u8])], schnorr: bool) -> Result<(Vec<Result<(), SignatureError>>, u64), GpuError> {
+        let mut res: Vec<Option<Result<(), SignatureError>>> = vec![None; items.len()];
+        let (mut pk, mut sig, mut msg, mut off, mut idx) = (vec![], vec![], vec![], vec![0u64], vec![]);
+        for (i, (p, m, s)) in items.iter().enumerate() {
+            if s.len() != 64 {
+                res[i] = Some(status_to_result(1)); // eddsa_sig.rs:161 / schnorr_sig.rs:68
+                continue;
+            }
+            if p.len() != 32 {
+                res[i] = Some(status_to_result(5)); // as verify_batch: the reference cannot build such a key
+                continue;
+            }
+            pk.extend_from_slice(p);
+            sig.extend_from_slice(s);
+            msg.extend_from_slice(m);
+            off.push(msg.len() as u64);
+            idx.push(i);
+        }
+        let n = idx.len();
+        let mut st = vec![0u8; n];
+        let mut hits = 0u64;
+        self.gpu.check(unsafe { sys::kb_keyset_verify_pk_batch(self.ks, n, pk.as_ptr(), msg.as_ptr(), off.as_ptr(), sig.as_ptr(), st.as_mut_ptr(), schnorr as i32, &mut hits) })?;
+        for (k, i) in idx.into_iter().enumerate() {
+            res[i] = Some(status_to_result(st[k]));
+        }
+        Ok((res.into_iter().map(|r| r.unwrap()).collect(), hits))
+    }
     /// Batch companion of `Point::mul(s, Some(pk))` for registered keys — the `dh_exchange(secret, remote_public)` step
     /// (dh/dh_impl.rs:74-80) of `encrypted_deal` and ECIES.  Items are (key index, scalar); the result is what
     /// `BatchPoint::mul_batch` returns for the same key bytes, from the keys' combs.  The scalars are secret: the table
