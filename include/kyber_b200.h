@@ -56,7 +56,9 @@ extern "C" {
  *   KB_FD_GRAPH=0             forward-difference round: launch the conversion chain kernel by kernel instead of as a CUDA graph
  *   KB_FD_CHECK_Q4_MAX=c      forward-difference round: the final check uses four lanes per item up to c items (default 8192, 0 = never)
  *   KB_FD_Q4_MAX=c            forward-difference round: conversion launches of up to c cells use four lanes per cell (default 8192, 0 = never)
- *   KB_MSM_C=c                Pippenger window bits (default floor(log2 n) - 3 within 4..16) */
+ *   KB_MSM_C=c                Pippenger window bits (default floor(log2 n) - 3 within 4..16)
+ *   KB_RC_CHUNKS=c            batched round check (KB_ROUND_CHECK_BATCHED): chunks per window of the shared-scalar
+ *                             multi-scalar multiplication, 1..16 (default: by the number of dealers) */
 typedef struct kb_ctx kb_ctx;
 
 typedef enum kb_err {
@@ -282,6 +284,26 @@ int kb_dkg_verify_round(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_
  * share/vss/pedersen/vss.rs:155-159); here a dealer with an element that is not a consistent representation of a curve
  * point (Z = 0, T Z != X Y, or off the curve) gets verdict 0 throughout. */
 int kb_dkg_verify_round_limbs(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_t dealer_hi, const int32_t* commit_limbs, const uint8_t* shares, uint8_t* verdict);
+/* How the rounds of a context check their shares: kb_dkg_verify_round[_limbs], kb_dkg_process_round[_keyed], their kb_dev_
+ * forms and, per device (set it on each kb_mctx_ctx(m, i)), the kb_mctx_ forms.  kb_vss_verify_deals_batch is always exact.
+ *   EXACT    every share is evaluated (forward differences or Horner).  The default of a new context.
+ *   BATCHED  each dealer's n checks are tested at once as one random linear combination, with weights of 128 bits drawn
+ *            from the OS per call (DESIGN.md section 3.10), plus an exact test of the small-order parts of its commitments.
+ *            A dealer that fails it, or that sent a share with byte 31 > 127, is checked share by share.  The verdicts are
+ *            those of EXACT except with probability at most 2^-128 for each dealer that has a wrong share.
+ *            Measured on one B200 at 1 000 W, n = 1 024, t = 683 (profiles/r9_bench_round_batched.json): 5.2 ms for the
+ *            share checks of a round of honest dealers, against 143 ms EXACT; a dealer that fails costs about 0.5 ms more,
+ *            plus about 27 ms for the first (the latency of its per-share checks), so BATCHED is slower than EXACT from
+ *            about 210 failing dealers on. */
+typedef enum kb_round_check {
+    KB_ROUND_CHECK_EXACT = 0,
+    KB_ROUND_CHECK_BATCHED = 1
+} kb_round_check;
+/* KB_ERR_ARG for any other mode.  kb_ctx_wipe leaves the mode as it is. */
+int kb_ctx_set_round_check(kb_ctx* ctx, int mode);
+/* *dealers = the number of dealers the last round call of this context checked share by share (0 after an EXACT round);
+ * waits for that call's stream. */
+int kb_ctx_round_fallbacks(kb_ctx* ctx, uint64_t* dealers);
 /* PriPoly::eval (poly.rs:133-141) for npoly private polynomials of t coefficients at the indices 0..n-1:
  * out[d*n + i] = poly[d].eval(i) — the shares a dealer hands out (new_dealer, share/vss/pedersen/vss.rs:313). */
 int kb_pripoly_eval_batch(kb_ctx* ctx, size_t npoly, size_t t, const uint8_t* coeffs, size_t n, uint8_t* out);

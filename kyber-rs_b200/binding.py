@@ -55,7 +55,11 @@ EXPORTS = [
     "kb_schnorr_sign_batch", "kb_dev_schnorr_sign", "kb_mctx_schnorr_sign_batch",
     "kb_signerset_create", "kb_signerset_destroy", "kb_signerset_sign_batch", "kb_dev_signerset_sign",
     "kb_mctx_signerset_create", "kb_mctx_signerset_destroy", "kb_mctx_signerset_sign_batch",
+    "kb_ctx_set_round_check", "kb_ctx_round_fallbacks",
 ]
+
+# kb_round_check: how the DKG rounds of a context check their shares
+ROUND_CHECK = {"exact": 0, "batched": 1}
 
 
 def load_library(path: str = LIB_PATH):
@@ -172,6 +176,8 @@ def load_library(path: str = LIB_PATH):
     L.kb_mctx_signerset_destroy.argtypes = [vp]
     L.kb_mctx_signerset_destroy.restype = None
     L.kb_mctx_signerset_sign_batch.argtypes = [vp, sz, vp, vp, vp, vp, vp]
+    L.kb_ctx_set_round_check.argtypes = [vp, i32]
+    L.kb_ctx_round_fallbacks.argtypes = [vp, ctypes.POINTER(ctypes.c_uint64)]
     _LIB = L
     return L
 
@@ -244,6 +250,17 @@ class Context:
 
     def wipe(self):
         self._check(self.L.kb_ctx_wipe(self.h), "kb_ctx_wipe")
+
+    def set_round_check(self, mode):
+        """"exact" (every share evaluated, the default) or "batched" (one random linear combination per dealer, dealers
+        that fail it checked share by share) for every DKG round of this context."""
+        self._check(self.L.kb_ctx_set_round_check(self.h, ROUND_CHECK[mode]), "kb_ctx_set_round_check")
+
+    def round_fallbacks(self):
+        """Dealers the last round call checked share by share (0 after an exact round); waits for that call's stream."""
+        v = ctypes.c_uint64()
+        self._check(self.L.kb_ctx_round_fallbacks(self.h, ctypes.byref(v)), "kb_ctx_round_fallbacks")
+        return int(v.value)
 
     @property
     def sm_count(self):
@@ -866,6 +883,13 @@ class MultiContext:
     @property
     def launches(self):
         return int(self.L.kb_mctx_launch_count(self.h))
+
+    def set_round_check(self, mode):
+        """Context.set_round_check on the context of every device."""
+        for k in range(len(self.devices)):
+            rc = self.L.kb_ctx_set_round_check(self.L.kb_mctx_ctx(self.h, k), ROUND_CHECK[mode])
+            if rc != 0:
+                raise KBError(f"kb_ctx_set_round_check failed with {rc}")
 
     def verify_batch(self, pk, msg, msg_off, sig, schnorr=False, out=None):
         pk, sig = _u8(pk, (-1, 32)), _u8(sig, (-1, 64))

@@ -57,6 +57,8 @@ int kb_ctx_create(int device, kb_ctx** out)
     ok = ok && cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&ctx->order_ev, cudaEventDisableTiming) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&ctx->fd_pw_ev, cudaEventDisableTiming) == cudaSuccess;
+    ok = ok && cudaEventCreateWithFlags(&ctx->rc_ev, cudaEventDisableTiming) == cudaSuccess;
+    ok = ok && cudaMallocHost(&ctx->rc_host, sizeof(uint32_t)) == cudaSuccess;   // here, so that the kb_dev_ rounds only enqueue
     ok = ok && cudaEventCreateWithFlags(&ctx->fork_ev, cudaEventDisableTiming) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&ctx->join_ev, cudaEventDisableTiming) == cudaSuccess;
     for (int k = 0; k < 2; k++) {
@@ -113,6 +115,9 @@ int kb_ctx_create(int device, kb_ctx** out)
         ctx->fd_steps_wide = fw ? atoi(fw) : 0;
         const char* fm = getenv("KB_FD_STEPS_MINB");
         ctx->fd_steps_minb = fm ? atoi(fm) : 0;
+        const char* rcc = getenv("KB_RC_CHUNKS");
+        const int rccn = rcc ? atoi(rcc) : 0;
+        ctx->rc_chunks = (rccn >= 1 && rccn <= 16) ? rccn : 0;
         const char* mc = getenv("KB_MSM_C");
         const int mcv = mc ? atoi(mc) : 0;
         ctx->msm_c = (mcv >= 4 && mcv <= 16) ? mcv : 0;
@@ -146,6 +151,8 @@ void kb_ctx_destroy(kb_ctx* ctx)
     if (ctx->base128) cudaFree(ctx->base128);
     if (ctx->comb) cudaFree(ctx->comb);
     if (ctx->fd_pw_host) cudaFreeHost(ctx->fd_pw_host);
+    if (ctx->rc_host) cudaFreeHost(ctx->rc_host);
+    if (ctx->rc_ev) cudaEventDestroy(ctx->rc_ev);
     if (ctx->fd_graph_exec) cudaGraphExecDestroy((cudaGraphExec_t)ctx->fd_graph_exec);
     for (int k = 0; k < 3; k++)
         if (ctx->tev[k]) cudaEventDestroy(ctx->tev[k]);
@@ -166,6 +173,22 @@ void kb_ctx_destroy(kb_ctx* ctx)
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
     free(ctx);
+}
+int kb_ctx_set_round_check(kb_ctx* ctx, int mode)
+{
+    if (!ctx || (mode != KB_ROUND_CHECK_EXACT && mode != KB_ROUND_CHECK_BATCHED)) return KB_ERR_ARG;
+    ctx->round_check = mode;
+    return KB_OK;
+}
+int kb_ctx_round_fallbacks(kb_ctx* ctx, uint64_t* dealers)
+{
+    KB_ENTER();
+    if (!dealers) return KB_ERR_ARG;
+    *dealers = 0;
+    if (!ctx->rc_valid) return KB_OK;
+    KB_CUDA(cudaEventSynchronize(ctx->rc_ev));
+    *dealers = *ctx->rc_host;
+    return KB_OK;
 }
 const char* kb_last_error(const kb_ctx* ctx) { return ctx ? ctx->err : "no context"; }
 int kb_device_sm_count(const kb_ctx* ctx) { return ctx ? ctx->sm_count : 0; }

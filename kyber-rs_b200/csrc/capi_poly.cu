@@ -4,6 +4,8 @@
 #include "kernels.cuh"
 #include "msm.cuh"
 #include "dkgfd.cuh"
+#include "dkgrlc.cuh"
+#include <random>
 // commitments -> cached form into scratch slots 8 (cached) / 9 (bad flags); then the eval kernel.
 //   d_shares != 0           verdicts of the share checks into d_out (one byte per item)
 //   d_shares == 0, d_out    encodings of the evaluations into d_out, per-item status into d_status
@@ -222,8 +224,97 @@ static size_t kb_dkg_plan(const kb_ctx* ctx, size_t n, size_t t, size_t nd)
     // measured, n = 256, t = 171: 32 / 64 / 128 / 256 dealers -> Horner 4.2 ms at 32 dealers, forward differences 2.5 / 3.5 / 5.8 ms
     return (nd * t >= 1024 && best_time * 1.15 < horner) ? best_h : 0;
 }
+// KB_ROUND_CHECK_BATCHED (dkgrlc.cuh): weights, decode, the shared-scalar multi-scalar multiplication, the torsion images and
+// the share sums, one launch per dealer to decide, then the share-by-share checks of the dealers that failed, on a list
+// whose length stays on the device.  Everything is enqueued on st; the fallback count is copied to rc_host at the end.
+static int kb_dkg_rc_run(kb_ctx* ctx, size_t n, size_t t, size_t nd, const void* d_commits, int limbs, const uint8_t* d_shares, uint8_t* d_verdict, cudaStream_t st)
+{
+    ctx->rc_valid = 0;   // until this call has enqueued the copy of its own count
+    if (nd >= ((size_t)1 << 32)) return KB_ERR_ARG;
+    const size_t nd32 = (nd + 31) & ~(size_t)31, n32 = (n + 31) & ~(size_t)31;
+    const size_t sms = (size_t)(ctx->sm_count > 0 ? ctx->sm_count : 1);
+    // chunks per window: about 512 dealer-chunks per window, at most 2.  Measured on a B200 at 1 000 W (KB_RC_CHUNKS sweep of
+    // tools/bench_round_batched.py, honest cfg4 round): 1 024 dealers 6.23 / 6.31 / 6.35 / 6.64 / 6.97 / 6.81 ms at 1 / 2 / 4 /
+    // 5 / 8 / 16 chunks; the 128 dealers of one GPU of eight 3.19 / 2.47 / 2.64 / 2.89 / 3.21 / 3.80 ms.  More chunks fill the
+    // GPU better in k_rc_msm but lengthen the fold in k_rc_dealer, a serial chain of one thread per dealer.
+    size_t nch = ctx->rc_chunks ? (size_t)ctx->rc_chunks : (512 + nd32 - 1) / nd32;   // KB_RC_CHUNKS: 1..16
+    if (!ctx->rc_chunks && nch > 2) nch = 2;
+    if (nch > t) nch = t;
+    if (nch < 1) nch = 1;
+    // share sums: parts per dealer so that about four threads per SM-lane run, at most 32 and at most n
+    size_t sparts = (4 * sms * 128 + nd - 1) / nd;
+    if (sparts > 32) sparts = 32;
+    if (sparts > n) sparts = n;
+    if (sparts < 1) sparts = 1;
+    uint32_t *dec, *dbad, *z, *ent, *cnt, *parts, *tor, *spart, *sflag, *stw, *list;
+    unsigned long long* wacc;
+    int16_t* dig;
+    uint8_t* bkt;
+    KB_SCRATCH(31, 128 * nd * t, dec);
+    KB_SCRATCH(9, 4 * nd, dbad);
+    KB_SCRATCH(55, 64 * t, wacc);
+    KB_SCRATCH(56, 16 * n32, z);
+    KB_SCRATCH(57, 2 * KB_RC_WINDOWS * t, dig);
+    KB_SCRATCH(58, 4 * KB_RC_WINDOWS * t, ent);
+    KB_SCRATCH(59, KB_RC_WINDOWS * t, bkt);
+    KB_SCRATCH(60, 4 * (KB_RC_WINDOWS + 1 + 3 * nd), cnt);   // window counts, fallback count, state words, fallback list
+    KB_SCRATCH(61, 128 * KB_RC_WINDOWS * nch * nd, parts);
+    KB_SCRATCH(62, 128 * 5 * nd, tor);
+    KB_SCRATCH(63, (32 + 4) * sparts * nd, spart);
+    sflag = spart + 8 * sparts * nd;
+    stw = cnt + KB_RC_WINDOWS + 1;
+    list = stw + nd;
+    // the weights are drawn after the inputs are in place, from the OS, for this call only
+    kb_rc_seed seed;
+    {
+        std::random_device rd;
+        for (int k = 0; k < 8; k++) seed.w[k] = (uint32_t)rd();
+    }
+    KB_CUDA(cudaMemsetAsync(wacc, 0, 64 * t, st));
+    KB_CUDA(cudaMemsetAsync(dbad, 0, 4 * nd, st));
+    const size_t jchunks = (t + KB_RC_POW_J - 1) / KB_RC_POW_J;
+    k_rc_weights<<<kb_blocks(jchunks * n32, KB_THREADS), KB_THREADS, 0, st>>>(n, t, seed, z, wacc);
+    KB_LAUNCHED();
+    memset(&seed, 0, sizeof(seed));
+    k_rc_digits<<<kb_blocks(t, KB_THREADS), KB_THREADS, 0, st>>>(t, wacc, dig);
+    KB_LAUNCHED();
+    k_rc_sort<<<KB_RC_WINDOWS, 256, 0, st>>>(t, dig, ent, bkt, cnt);
+    KB_LAUNCHED();
+    if (limbs) k_fd_decode_limbs<<<kb_blocks(nd * t, KB_THREADS), KB_THREADS, 0, st>>>(nd, t, (const int32_t*)d_commits, dec, dbad);
+    else k_fd_decode<<<kb_blocks(nd * t, KB_THREADS), KB_THREADS, 0, st>>>(nd, t, (const uint8_t*)d_commits, dec, dbad);
+    KB_LAUNCHED();
+    // k_rc_torsion is a few blocks of long serial chains (t / 2 additions, then [L]): it runs on a second stream beside the
+    // multi-scalar multiplication and the share sums, which fill the GPU
+    cudaStream_t side = (st == ctx->stream2) ? ctx->stream : ctx->stream2;
+    KB_CUDA(cudaEventRecord(ctx->fork_ev, st));
+    KB_CUDA(cudaStreamWaitEvent(side, ctx->fork_ev, 0));
+    k_rc_torsion<<<kb_blocks(5 * nd, KB_THREADS), KB_THREADS, 0, side>>>(nd, t, dec, tor);
+    KB_LAUNCHED();
+    KB_CUDA(cudaEventRecord(ctx->join_ev, side));
+    k_rc_msm<<<kb_blocks(KB_RC_WINDOWS * nch * nd32, KB_THREADS), KB_THREADS, 0, st>>>(nd, t, nch, dec, ent, bkt, cnt, parts);
+    KB_LAUNCHED();
+    k_rc_shares<<<kb_blocks(sparts * nd, KB_THREADS), KB_THREADS, 0, st>>>(nd, n, sparts, z, d_shares, spart, sflag);
+    KB_LAUNCHED();
+    KB_CUDA(cudaStreamWaitEvent(st, ctx->join_ev, 0));
+    k_rc_dealer<<<kb_blocks(nd, KB_THREADS), KB_THREADS, 64 * 8 * 96, st>>>(nd, nch, sparts, parts, tor, spart, sflag, dbad, ctx->base_table, stw);
+    KB_LAUNCHED();
+    // the sums of z_i s_(d,i) are combinations of the verifiers' secrets: they do not stay in device scratch
+    KB_CUDA(cudaMemsetAsync(spart, 0, 32 * sparts * nd, st));
+    k_rc_verdict<<<kb_blocks(nd * n, KB_THREADS), KB_THREADS, 0, st>>>(nd, n, stw, d_verdict);
+    KB_LAUNCHED();
+    k_rc_compact<<<1, 1024, 0, st>>>(nd, stw, list, cnt + KB_RC_WINDOWS);
+    KB_LAUNCHED();
+    k_poly_eval_list<<<kb_blocks(nd * n, KB_THREADS), KB_THREADS, 64 * 8 * 96, st>>>(nd, t, dec, dbad, list, cnt + KB_RC_WINDOWS, n, d_shares, d_verdict, ctx->base_table);
+    KB_LAUNCHED();
+    KB_CUDA(cudaMemcpyAsync(ctx->rc_host, cnt + KB_RC_WINDOWS, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    KB_CUDA(cudaEventRecord(ctx->rc_ev, st));
+    ctx->rc_valid = 1;
+    return KB_OK;
+}
 int kb_dkg_round_run(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, const void* d_commits, int limbs, const uint8_t* d_shares, uint8_t* d_verdict, cudaStream_t st)
 {
+    if (ctx->round_check == KB_ROUND_CHECK_BATCHED) return kb_dkg_rc_run(ctx, n, t, ndealers, d_commits, limbs, d_shares, d_verdict, st);
+    ctx->rc_valid = 0;
     const size_t h = kb_dkg_plan(ctx, n, t, ndealers);
     if (h) return kb_dkg_fd_run(ctx, n, t, ndealers, h, d_commits, limbs, d_shares, d_verdict, st);
     return kb_poly_run(ctx, ndealers, t, d_commits, limbs, n * ndealers, nullptr, nullptr, n, d_shares, d_verdict, nullptr, nullptr, st);

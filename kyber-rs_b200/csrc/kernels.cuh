@@ -1338,17 +1338,31 @@ static __global__ void __launch_bounds__(KB_THREADS) k_pripoly_eval(size_t npoly
 // items enumerate a DKG round: k = i * npoly + d (verifier-major), so the 32 lanes of a warp
 // hold 32 different dealers and the SAME evaluation point x = i + 1 — the double-and-add over
 // the bits of x is then branch-uniform across the warp.
-static __global__ void __launch_bounds__(KB_THREADS) k_poly_eval(size_t m, size_t npoly, size_t t, const uint32_t* cached, const uint8_t* bad, const uint32_t* poly_id,
-                                                          const uint32_t* idx, size_t n_verifiers, const uint8_t* shares, uint32_t* xyz, uint8_t* status, uint8_t* verdict, const ge_precomp* table)
+// LIST = true (k_poly_eval_list): the items are those of the *cnt dealers list[0 ..) of a DKG round, k = i * (*cnt) + f for
+// dealer list[f]; the commitments are the extended points dec[j * npoly + d] and dealer_bad[d] of k_fd_decode.
+template <bool LIST>
+__device__ __forceinline__ void kb_poly_eval_run(size_t m, size_t npoly, size_t t, const uint32_t* cached, const uint8_t* bad, const uint32_t* poly_id, const uint32_t* idx,
+                                                 size_t n_verifiers, const uint8_t* shares, uint32_t* xyz, uint8_t* status, uint8_t* verdict, const ge_precomp* table,
+                                                 const uint32_t* dec, const uint32_t* dealer_bad, const uint32_t* list, const uint32_t* cnt)
 {
     extern __shared__ uint4 smem4[];
     ge_precomp* base = reinterpret_cast<ge_precomp*>(smem4);
+    size_t nl = 0;
+    if constexpr (LIST) {
+        nl = *cnt;
+        m = nl * n_verifiers;
+        if ((size_t)blockIdx.x * blockDim.x >= m) return;   // the grid is sized for every dealer: whole blocks leave here
+    }
     if (shares) kb_stage(reinterpret_cast<uint32_t*>(base), reinterpret_cast<const uint32_t*>(table), 64 * 8 * 24);
     size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool live = k < m;   // the coefficient loop holds a block barrier: tail threads redo the last item
     if (!live) k = m - 1;
     size_t d, i, slot;
-    if (poly_id) {
+    if constexpr (LIST) {
+        d = list[k % nl];
+        i = k / nl;
+        slot = d * n_verifiers + i;
+    } else if (poly_id) {
         d = poly_id[k];
         i = idx[k];
         slot = k;
@@ -1357,18 +1371,25 @@ static __global__ void __launch_bounds__(KB_THREADS) k_poly_eval(size_t m, size_
         i = k / npoly;
         slot = d * n_verifiers + i;
     }
-    const uint32_t* cp = cached + 32 * (d * t);
-    const uint8_t* bp = bad + d * t;
+    const uint32_t* cp = LIST ? nullptr : cached + 32 * (d * t);
+    const uint8_t* bp = LIST ? nullptr : bad + d * t;
     ge_p3 v;
     ge_identity(v);
     uint32_t anybad = 0;
+    if constexpr (LIST) anybad = dealer_bad[d] ? 1u : 0u;
     kb_naf xn;
     kb_naf_from(xn, (uint64_t)i + 1);
     for (size_t j = t; j-- > 0;) {
         __syncthreads();   // keeps the block's warps on the same instructions (see KB_LOCKSTEP in ops.cuh)
         ge_cached c;
-        kb_load_cached_w128(c, cp + 32 * j);
-        anybad |= bp[j];
+        if constexpr (LIST) {
+            ge_p3 P;
+            kb_load_p3_w128(P, dec + (j * npoly + d) * 32);
+            ge_to_cached(c, P);
+        } else {
+            kb_load_cached_w128(c, cp + 32 * j);
+            anybad |= bp[j];
+        }
         kb_horner_step(v, xn, c);
     }
     if (!shares) {
@@ -1396,6 +1417,18 @@ static __global__ void __launch_bounds__(KB_THREADS) k_poly_eval(size_t m, size_
     fe_sub(df, l, r);
     same &= fe_is_zero(df);
     if (live) verdict[slot] = (uint8_t)(same & (anybad ^ 1u));
+}
+static __global__ void __launch_bounds__(KB_THREADS) k_poly_eval(size_t m, size_t npoly, size_t t, const uint32_t* cached, const uint8_t* bad, const uint32_t* poly_id,
+                                                          const uint32_t* idx, size_t n_verifiers, const uint8_t* shares, uint32_t* xyz, uint8_t* status, uint8_t* verdict, const ge_precomp* table)
+{
+    kb_poly_eval_run<false>(m, npoly, t, cached, bad, poly_id, idx, n_verifiers, shares, xyz, status, verdict, table, nullptr, nullptr, nullptr, nullptr);
+}
+// the share checks of the dealers list[0 .. *cnt) of a round of npoly dealers and n_verifiers verifiers (the fallback of
+// KB_ROUND_CHECK_BATCHED, dkgrlc.cuh); the grid covers every dealer, the count is read on the device
+static __global__ void __launch_bounds__(KB_THREADS) k_poly_eval_list(size_t npoly, size_t t, const uint32_t* dec, const uint32_t* dealer_bad, const uint32_t* list, const uint32_t* cnt,
+                                                               size_t n_verifiers, const uint8_t* shares, uint8_t* verdict, const ge_precomp* table)
+{
+    kb_poly_eval_run<true>(0, npoly, t, nullptr, nullptr, nullptr, nullptr, n_verifiers, shares, nullptr, nullptr, verdict, table, dec, dealer_bad, list, cnt);
 }
 
 #endif  // KB_K_POLY

@@ -97,6 +97,8 @@ extern "C" {
     pub fn kb_vss_verify_deals_batch(ctx: *mut kb_ctx, npoly: usize, t: usize, commits: *const u8, m: usize, poly_id: *const u32, idx: *const u32, shares: *const u8, verdict: *mut u8) -> c_int;
     pub fn kb_dkg_verify_round(ctx: *mut kb_ctx, n: usize, t: usize, dealer_lo: usize, dealer_hi: usize, commits: *const u8, shares: *const u8, verdict: *mut u8) -> c_int;
     pub fn kb_dkg_verify_round_limbs(ctx: *mut kb_ctx, n: usize, t: usize, dealer_lo: usize, dealer_hi: usize, commit_limbs: *const i32, shares: *const u8, verdict: *mut u8) -> c_int;
+    pub fn kb_ctx_set_round_check(ctx: *mut kb_ctx, mode: c_int) -> c_int;
+    pub fn kb_ctx_round_fallbacks(ctx: *mut kb_ctx, dealers: *mut u64) -> c_int;
 
     pub fn kb_pubpoly_sum(ctx: *mut kb_ctx, npoly: usize, t: usize, commits: *const u8, out: *mut u8, status: *mut u8) -> c_int;
 

@@ -21,6 +21,16 @@ pub enum GpuError {
     InvalidPoint(usize),
 }
 
+/// How a DKG round checks its shares (`kb_round_check`).
+#[derive(Clone, Copy, PartialEq, Eq, Debug)]
+pub enum RoundCheck {
+    /// every share is evaluated (the default)
+    Exact,
+    /// one random linear combination per dealer; dealers that fail it are checked share by share.  The verdicts are the
+    /// exact ones except with probability at most 2^-128 per dealer with a wrong share.
+    Batched,
+}
+
 /// One CUDA device, one host thread — kyber-rs itself is single-threaded (SURVEY §8b).
 pub struct Gpu {
     ctx: *mut sys::kb_ctx,
@@ -34,6 +44,20 @@ impl Gpu {
             sys::KB_ERR_NOMEM => Err(GpuError::NoMem),
             _ => Err(GpuError::Cuda("no usable CUDA device (there is no CPU fallback)".into())),
         }
+    }
+    /// How the DKG rounds of this context check their shares (`kb_ctx_set_round_check`); a new context is `Exact`.
+    pub fn set_round_check(&self, mode: RoundCheck) -> Result<(), GpuError> {
+        let m = match mode {
+            RoundCheck::Exact => 0,
+            RoundCheck::Batched => 1,
+        };
+        self.check(unsafe { sys::kb_ctx_set_round_check(self.ctx, m) })
+    }
+    /// Dealers the last round call checked share by share (0 after an `Exact` round).
+    pub fn round_fallbacks(&self) -> Result<u64, GpuError> {
+        let mut d = 0u64;
+        self.check(unsafe { sys::kb_ctx_round_fallbacks(self.ctx, &mut d) })?;
+        Ok(d)
     }
     fn check(&self, rc: i32) -> Result<(), GpuError> {
         match rc {
