@@ -58,7 +58,10 @@ extern "C" {
  *   KB_FD_Q4_MAX=c            forward-difference round: conversion launches of up to c cells use four lanes per cell (default 8192, 0 = never)
  *   KB_MSM_C=c                Pippenger window bits (default floor(log2 n) - 3 within 4..16)
  *   KB_RC_CHUNKS=c            batched round check (KB_ROUND_CHECK_BATCHED): chunks per window of the shared-scalar
- *                             multi-scalar multiplication, 1..16 (default: by the number of dealers) */
+ *                             multi-scalar multiplication, 1..16 (default: by the number of dealers); the same for the
+ *                             column kernel of kb_dkg_verify_columns
+ *   KB_DKG_COLUMNS=0|1        kb_dkg_verify_columns on a partial verifier range: never / always by the column kernel
+ *                             (default: by size) */
 typedef struct kb_ctx kb_ctx;
 
 typedef enum kb_err {
@@ -284,6 +287,17 @@ int kb_dkg_verify_round(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_
  * share/vss/pedersen/vss.rs:155-159); here a dealer with an element that is not a consistent representation of a curve
  * point (Z = 0, T Z != X Y, or off the curve) gets verdict 0 throughout. */
 int kb_dkg_verify_round_limbs(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_t dealer_hi, const int32_t* commit_limbs, const uint8_t* shares, uint8_t* verdict);
+/* The share checks of a Pedersen-DKG round restricted to verifiers [ver_lo, ver_hi): what participants ver_lo..ver_hi-1 run in
+ * process_deal (dkg.rs:513-597) for the deals of dealers [dealer_lo, dealer_hi).  commits as in kb_dkg_process_round (fmt,
+ * whole array indexed by absolute dealer); shares[(d - dealer_lo)*k + (i - ver_lo)], k = ver_hi - ver_lo, is the share dealer
+ * d sent to verifier i; verdict in the same layout, equal byte for byte to kb_vss_verify_deals_batch on the same items
+ * (poly_id = d, idx = i) and, for ver_lo = 0 and ver_hi = n, to kb_dkg_verify_round.
+ * The whole range is kb_dkg_verify_round itself (its round-check mode and fallback count).  A partial range is checked
+ * exactly in both modes, one multi-scalar multiplication per column with the exponents (i + 1)^j mod 8L (DESIGN.md section
+ * 3.11), and kb_ctx_round_fallbacks then reports 0.  KB_ERR_ARG when ver_lo >= ver_hi, ver_hi > n, dealer_hi < dealer_lo or
+ * n > 2^32; an empty dealer range returns KB_OK.  The shares do not stay in device scratch. */
+int kb_dkg_verify_columns(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_t dealer_hi, size_t ver_lo, size_t ver_hi,
+                          int fmt, const void* commits, const uint8_t* shares, uint8_t* verdict);
 /* How the rounds of a context check their shares: kb_dkg_verify_round[_limbs], kb_dkg_process_round[_keyed], their kb_dev_
  * forms and, per device (set it on each kb_mctx_ctx(m, i)), the kb_mctx_ forms.  kb_vss_verify_deals_batch is always exact.
  *   EXACT    every share is evaluated (forward differences or Horner).  The default of a new context.
@@ -400,6 +414,9 @@ int kb_dev_msm(kb_ctx* ctx, size_t n, const void* d_scalars, const void* d_point
 int kb_dev_msm_ext(kb_ctx* ctx, size_t n, const void* d_scalars, const void* d_points128, void* d_out32, void* d_partial128, void* d_bad_points, void* stream);
 int kb_dev_dkg_verify_round(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, const void* d_commits, const void* d_shares, void* d_verdict, void* stream);
 int kb_dev_dkg_verify_round_limbs(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, const void* d_commit_limbs, const void* d_shares, void* d_verdict, void* stream);
+/* kb_dkg_verify_columns on device buffers for ndealers dealers (commitments, shares and verdicts start at the first of them) */
+int kb_dev_dkg_verify_columns(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, size_t ver_lo, size_t ver_hi, int fmt,
+                              const void* d_commits, const void* d_shares, void* d_verdict, void* stream);
 int kb_dev_point_sum(kb_ctx* ctx, size_t k, const void* d_partials128, void* d_out32, void* stream);
 /* the pure decompress (ExtendedGroupElement::set_bytes -> X, Y, Z, T words) and hash (SHA-512(R || A || M) mod L) stages */
 int kb_dev_point_decompress(kb_ctx* ctx, size_t n, const void* d_in, void* d_out128, void* d_status, void* stream);

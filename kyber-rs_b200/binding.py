@@ -56,6 +56,7 @@ EXPORTS = [
     "kb_signerset_create", "kb_signerset_destroy", "kb_signerset_sign_batch", "kb_dev_signerset_sign",
     "kb_mctx_signerset_create", "kb_mctx_signerset_destroy", "kb_mctx_signerset_sign_batch",
     "kb_ctx_set_round_check", "kb_ctx_round_fallbacks",
+    "kb_dkg_verify_columns", "kb_dev_dkg_verify_columns",
 ]
 
 # kb_round_check: how the DKG rounds of a context check their shares
@@ -123,6 +124,8 @@ def load_library(path: str = LIB_PATH):
     L.kb_dev_msm_ext.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp]
     L.kb_dev_dkg_verify_round.argtypes = [vp, sz, sz, sz, vp, vp, vp, vp]
     L.kb_dev_dkg_verify_round_limbs.argtypes = [vp, sz, sz, sz, vp, vp, vp, vp]
+    L.kb_dkg_verify_columns.argtypes = [vp, sz, sz, sz, sz, sz, sz, i32, vp, vp, vp]
+    L.kb_dev_dkg_verify_columns.argtypes = [vp, sz, sz, sz, sz, sz, i32, vp, vp, vp, vp]
     L.kb_dev_point_sum.argtypes = [vp, sz, vp, vp, vp]
     L.kb_pripoly_eval_batch.argtypes = [vp, sz, sz, vp, sz, vp]
     L.kb_dev_pripoly_eval.argtypes = [vp, sz, sz, vp, sz, vp, vp]
@@ -445,6 +448,25 @@ class Context:
         self._check(fn(self.h, n, t, dealer_lo, dealer_hi, _ptr(c), _ptr(sh), _ptr(verdict)), "kb_dkg_verify_round")
         return verdict
 
+    def dkg_verify_columns(self, n, t, commits, shares, ver_lo, ver_hi, dealer_lo=0, dealer_hi=None, fmt=0):
+        """The share checks of verifiers [ver_lo, ver_hi) for dealers [dealer_lo, dealer_hi): what those participants run in
+        process_deal.  commits: the whole round's (ndealers*t, 32) encodings (fmt 0) or (ndealers*t, 40) int32 limbs (fmt 1);
+        shares: ((dealer_hi - dealer_lo) * k, 32), row (d - dealer_lo) * k + (i - ver_lo), k = ver_hi - ver_lo.  Returns the
+        verdicts in the layout of the shares."""
+        c = self._points(commits, fmt == 1)
+        sh = _u8(shares, (-1, 32))
+        ndealers = c.shape[0] // t if t else 0
+        if dealer_hi is None:
+            dealer_hi = ndealers
+        if not t or ndealers * t != c.shape[0] or not (0 <= dealer_lo <= dealer_hi <= ndealers):
+            raise ValueError("dkg_verify_columns: commits must hold ndealers*t points and the dealer range lie inside them")
+        k = max(ver_hi - ver_lo, 0)
+        if sh.shape[0] != (dealer_hi - dealer_lo) * k:
+            raise ValueError("dkg_verify_columns: shares must hold (dealer_hi - dealer_lo) * (ver_hi - ver_lo) scalars")
+        verdict = np.zeros(sh.shape[0], dtype=np.uint8)
+        self._check(self.L.kb_dkg_verify_columns(self.h, n, t, dealer_lo, dealer_hi, ver_lo, ver_hi, int(fmt), _ptr(c), _ptr(sh), _ptr(verdict)), "kb_dkg_verify_columns")
+        return verdict
+
     def pripoly_eval_batch(self, coeffs, t, n):
         """PriPoly::eval for every polynomial at indices 0..n-1: (npoly*n, 32) shares, polynomial-major."""
         c = _u8(coeffs, (-1, 32))
@@ -672,6 +694,11 @@ class Context:
     def dev_dkg_verify_round(self, n, t, ndealers, commits, shares, verdict, limbs=False):
         fn = self.L.kb_dev_dkg_verify_round_limbs if limbs else self.L.kb_dev_dkg_verify_round
         self._check(fn(self.h, n, t, ndealers, self._dp(commits), self._dp(shares), self._dp(verdict), self._stream()), "kb_dev_dkg_verify_round")
+
+    def dev_dkg_verify_columns(self, n, t, ndealers, commits, shares, verdict, ver_lo, ver_hi, fmt=0):
+        """dkg_verify_columns on CUDA tensors for ndealers dealers (commits, shares and verdict start at the first of them)."""
+        self._check(self.L.kb_dev_dkg_verify_columns(self.h, n, t, ndealers, ver_lo, ver_hi, int(fmt), self._dp(commits), self._dp(shares), self._dp(verdict), self._stream()),
+                    "kb_dev_dkg_verify_columns")
 
     def dev_dkg_process_round(self, n, t, ndealers, commits, shares, verdict, deal=None, resp=None, limbs=False):
         """deal / resp = (pk, msg, msg_off, sig, status) CUDA tensors or None."""

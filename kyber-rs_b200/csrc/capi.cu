@@ -118,6 +118,8 @@ int kb_ctx_create(int device, kb_ctx** out)
         const char* rcc = getenv("KB_RC_CHUNKS");
         const int rccn = rcc ? atoi(rcc) : 0;
         ctx->rc_chunks = (rccn >= 1 && rccn <= 16) ? rccn : 0;
+        const char* dcol = getenv("KB_DKG_COLUMNS");
+        ctx->dkg_columns = dcol ? atoi(dcol) : -1;
         const char* mc = getenv("KB_MSM_C");
         const int mcv = mc ? atoi(mc) : 0;
         ctx->msm_c = (mcv >= 4 && mcv <= 16) ? mcv : 0;

@@ -5,6 +5,7 @@
 #include "msm.cuh"
 #include "dkgfd.cuh"
 #include "dkgrlc.cuh"
+#include "dkgcol.cuh"
 #include <random>
 // commitments -> cached form into scratch slots 8 (cached) / 9 (bad flags); then the eval kernel.
 //   d_shares != 0           verdicts of the share checks into d_out (one byte per item)
@@ -319,6 +320,82 @@ int kb_dkg_round_run(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, const voi
     if (h) return kb_dkg_fd_run(ctx, n, t, ndealers, h, d_commits, limbs, d_shares, d_verdict, st);
     return kb_poly_run(ctx, ndealers, t, d_commits, limbs, n * ndealers, nullptr, nullptr, n, d_shares, d_verdict, nullptr, nullptr, st);
 }
+// (column, dealer) pairs per pass of the column kernel: its window sums take 128 * KB_COL_WINDOWS * chunks bytes per pair
+// (138 MB per pass at one chunk), and 2^15 pairs are 33 windows x 2^15 threads, several times what the GPU holds
+#define KB_COL_PAIRS ((size_t)1 << 15)
+// How a partial verifier range is checked: the column kernel or the per-share Horner kernel on its items.  The column
+// kernel costs about the same per (column, dealer) pair at any size, and 2.6 times a Horner walk once the GPU is full; the
+// per-share kernel is bound by the latency of its walks (t dependent steps) until it has several items per lane.  Measured on
+// a B200 at 1 000 W (tools/bench_dkg_columns.py, 1 024 dealers, t = 683, from ver_lo = 333): k = 1 / 4 / 6 / 8 / 16 / 64
+// columns 4.9 / 12.8 / 18.5 / 22.5 / 42.9 / 166.0 ms by the column kernel, 15.4 / 17.4 / 19.3 / 19.4 / 24.0 / 82.8 ms per
+// share; the two meet between 6 and 8 columns.  That was at x < 2^10: a Horner step is about one doubling per bit of x, so for larger x the crossover lies higher.
+#define KB_COL_MAX_PAIRS ((size_t)6144)
+static bool kb_dkg_columns_plan(const kb_ctx* ctx, size_t nd, size_t kc)
+{
+    if (ctx->dkg_columns >= 0) return ctx->dkg_columns != 0;   // KB_DKG_COLUMNS
+    return nd * kc <= KB_COL_MAX_PAIRS;
+}
+// The share checks of verifiers [ver_lo, ver_hi) for nd dealers: shares and verdicts [d][kc], kc = ver_hi - ver_lo.  The
+// whole range is the round itself.  A partial one runs the column kernel (dkgcol.cuh): one shared-exponent multi-scalar
+// multiplication per column, in passes of at most KB_COL_PAIRS (column, dealer) pairs; or k_poly_eval on its items.
+static int kb_dkg_columns_run(kb_ctx* ctx, size_t n, size_t t, size_t nd, size_t ver_lo, size_t ver_hi, const void* d_commits, int limbs, const uint8_t* d_shares, uint8_t* d_verdict,
+                              cudaStream_t st)
+{
+    if (ver_lo == 0 && ver_hi == n) return kb_dkg_round_run(ctx, n, t, nd, d_commits, limbs, d_shares, d_verdict, st);
+    ctx->rc_valid = 0;   // no share is checked twice: the fallback count of this call is 0
+    const size_t kc = ver_hi - ver_lo;
+    if (!kb_dkg_columns_plan(ctx, nd, kc)) {
+        const size_t m = nd * kc;
+        uint32_t *pid, *idx;
+        KB_SCRATCH(55, 4 * m, pid);
+        KB_SCRATCH(56, 4 * m, idx);
+        k_col_items<<<kb_blocks(m, KB_THREADS), KB_THREADS, 0, st>>>(m, kc, ver_lo, pid, idx);
+        KB_LAUNCHED();
+        return kb_poly_run(ctx, nd, t, d_commits, limbs, m, pid, idx, 0, d_shares, d_verdict, nullptr, nullptr, st);
+    }
+    const size_t nd32 = (nd + 31) & ~(size_t)31;
+    size_t group = KB_COL_PAIRS / nd;
+    if (group < 1) group = 1;
+    if (group > kc) group = kc;
+    // chunks per window as kb_dkg_rc_run chooses them, counting the lanes of all the pass's columns
+    size_t nch = ctx->rc_chunks ? (size_t)ctx->rc_chunks : (512 + group * nd32 - 1) / (group * nd32);   // KB_RC_CHUNKS: 1..16
+    if (!ctx->rc_chunks && nch > 2) nch = 2;
+    if (nch > t) nch = t;
+    if (nch < 1) nch = 1;
+    const size_t nwin = group * KB_COL_WINDOWS;
+    uint32_t *dec, *dbad, *ent, *cnt, *parts;
+    int16_t* dig;
+    uint8_t* bkt;
+    KB_SCRATCH(31, 128 * nd * t, dec);
+    KB_SCRATCH(9, 4 * nd, dbad);
+    KB_SCRATCH(57, 2 * nwin * t, dig);
+    KB_SCRATCH(58, 4 * nwin * t, ent);
+    KB_SCRATCH(59, nwin * t, bkt);
+    KB_SCRATCH(60, 4 * nwin, cnt);
+    KB_SCRATCH(61, 128 * nwin * nch * nd, parts);
+    KB_CUDA(cudaMemsetAsync(dbad, 0, 4 * nd, st));
+    if (limbs) k_fd_decode_limbs<<<kb_blocks(nd * t, KB_THREADS), KB_THREADS, 0, st>>>(nd, t, (const int32_t*)d_commits, dec, dbad);
+    else k_fd_decode<<<kb_blocks(nd * t, KB_THREADS), KB_THREADS, 0, st>>>(nd, t, (const uint8_t*)d_commits, dec, dbad);
+    KB_LAUNCHED();
+    const size_t jchunks = (t + KB_RC_POW_J - 1) / KB_RC_POW_J;
+    for (size_t c0 = 0; c0 < kc; c0 += group) {
+        const size_t g = kc - c0 < group ? kc - c0 : group;
+        k_col_digits<<<kb_blocks(g * jchunks, KB_THREADS), KB_THREADS, 0, st>>>(g, t, (uint64_t)(ver_lo + c0) + 1, dig);
+        KB_LAUNCHED();
+        k_rc_sort<<<(unsigned)(g * KB_COL_WINDOWS), 256, 0, st>>>(t, dig, ent, bkt, cnt);
+        KB_LAUNCHED();
+        k_col_msm<<<kb_blocks(g * KB_COL_WINDOWS * nch * nd32, KB_THREADS), KB_THREADS, 0, st>>>(nd, t, g * KB_COL_WINDOWS, nch, dec, ent, bkt, cnt, parts);
+        KB_LAUNCHED();
+        k_col_check<<<kb_blocks(g * nd, KB_THREADS), KB_THREADS, 64 * 8 * 96, st>>>(nd, g, kc, c0, nch, parts, dbad, d_shares, ctx->base_table, d_verdict);
+        KB_LAUNCHED();
+    }
+    return KB_OK;
+}
+static bool kb_columns_args_ok(size_t n, size_t t, size_t nd_lo, size_t nd_hi, size_t ver_lo, size_t ver_hi, int fmt)
+{
+    return t && nd_lo <= nd_hi && ver_lo < ver_hi && ver_hi <= n && n <= ((size_t)1 << 32) && nd_hi - nd_lo < ((size_t)1 << 32) && t < ((size_t)1 << 31) &&
+           (fmt == KB_POINT_ENC32 || fmt == KB_POINT_LIMBS40);
+}
 
 extern "C" {
 int kb_dev_dkg_verify_round(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, const void* d_commits, const void* d_shares, void* d_verdict, void* stream)
@@ -407,6 +484,43 @@ int kb_dkg_verify_round(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_
 int kb_dkg_verify_round_limbs(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_t dealer_hi, const int32_t* commit_limbs, const uint8_t* shares, uint8_t* verdict)
 {
     return kb_dkg_round_host(ctx, n, t, dealer_lo, dealer_hi, commit_limbs, 1, shares, verdict);
+}
+int kb_dkg_verify_columns(kb_ctx* ctx, size_t n, size_t t, size_t dealer_lo, size_t dealer_hi, size_t ver_lo, size_t ver_hi, int fmt, const void* commits, const uint8_t* shares,
+                          uint8_t* verdict)
+{
+    KB_ENTER();
+    if (!kb_columns_args_ok(n, t, dealer_lo, dealer_hi, ver_lo, ver_hi, fmt)) return KB_ERR_ARG;
+    const size_t nd = dealer_hi - dealer_lo, kc = ver_hi - ver_lo;
+    if (nd == 0) return KB_OK;
+    if (!commits || !shares || !verdict) return KB_ERR_ARG;
+    const int limbs = fmt == KB_POINT_LIMBS40;
+    const size_t cbytes = limbs ? 160 : 32;   // per commitment
+    uint8_t *d_c, *d_sh, *d_v;
+    KB_SCRATCH(0, cbytes * nd * t, d_c);
+    KB_SCRATCH(2, 32 * nd * kc, d_sh);
+    KB_SCRATCH(1, nd * kc, d_v);
+    KB_H2D(d_c, (const uint8_t*)commits + cbytes * dealer_lo * t, cbytes * nd * t);
+    KB_H2D(d_sh, shares, 32 * nd * kc);
+    int rc = kb_dkg_columns_run(ctx, n, t, nd, ver_lo, ver_hi, d_c, limbs, d_sh, d_v, ctx->stream);
+    // the shares are secrets of the verifiers: they do not stay in device scratch
+    cudaMemsetAsync(d_sh, 0, 32 * nd * kc, ctx->stream);
+    if (rc != KB_OK) {
+        cudaStreamSynchronize(ctx->stream);
+        return rc;
+    }
+    KB_D2H(verdict, d_v, nd * kc);
+    KB_SYNC();
+    return KB_OK;
+}
+int kb_dev_dkg_verify_columns(kb_ctx* ctx, size_t n, size_t t, size_t ndealers, size_t ver_lo, size_t ver_hi, int fmt, const void* d_commits, const void* d_shares, void* d_verdict,
+                              void* stream)
+{
+    if (!ctx || !kb_columns_args_ok(n, t, 0, ndealers, ver_lo, ver_hi, fmt)) return KB_ERR_ARG;
+    if (ndealers == 0) return KB_OK;
+    if (!d_commits || !d_shares || !d_verdict) return KB_ERR_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    KB_DEV_ENTER(st);
+    KB_DEV_RETURN(st, kb_dkg_columns_run(ctx, n, t, ndealers, ver_lo, ver_hi, d_commits, fmt == KB_POINT_LIMBS40, (const uint8_t*)d_shares, (uint8_t*)d_verdict, st));
 }
 
 int kb_dev_pripoly_eval(kb_ctx* ctx, size_t npoly, size_t t, const void* d_coeffs, size_t n, void* d_out, void* stream)

@@ -64,6 +64,7 @@ struct kb_ctx {
     // pinned host memory at the end of a KB_ROUND_CHECK_BATCHED round, rc_ev recorded after that copy
     int round_check;
     int rc_chunks;           // KB_RC_CHUNKS: chunks per window of the multi-scalar multiplication (0 = by size)
+    int dkg_columns;         // KB_DKG_COLUMNS: 1 = always / 0 = never the column kernel for a partial verifier range (default: by size)
     int rc_valid;            // the last round call was batched: rc_host / rc_ev hold its count
     uint32_t* rc_host;
     cudaEvent_t rc_ev;
@@ -148,7 +149,8 @@ int kb_dev_end(kb_ctx* ctx, cudaStream_t st);
 //   32..45  two lanes of the pipelined host-buffer verify
 //   46..63  protocol-level entry points (capi_proto.cu) and the multi-device context
 //   54      the partition of kb_dev_keyset_verify_pk (capi_keyset.cu)
-//   55..63  the batched share checks of a DKG round (capi_poly.cu kb_dkg_rc_run)
+//   55..63  the batched share checks of a DKG round (capi_poly.cu kb_dkg_rc_run); 55..61 also the share checks of a
+//           verifier range (kb_dkg_columns_run)
 
 // ---- drivers shared between translation units (each defined in the file named) -------------------------------------
 // capi_verify.cu: the two launches of a signature-verification batch on device buffers

@@ -167,16 +167,16 @@ KB_FN void kb_rc_chunk(ge_p3& tot, const uint32_t* ent, const uint8_t* bkt, size
         ge_add<true>(tot, tot, c);
     }
 }
-// W = sum_k 256^k sum_c part(k, c); load(k, c, P) fetches the result of chunk c of window k
-template <typename LD>
+// W = sum_k 256^k sum_c part(k, c) over NW windows; load(k, c, P) fetches the result of chunk c of window k
+template <int NW = KB_RC_WINDOWS, typename LD>
 KB_FN void kb_rc_fold(ge_p3& W, size_t nch, LD load)
 {
     ge_p3 P;
     ge_cached c;
     ge_identity(W);
     KB_NOUNROLL
-    for (int k = KB_RC_WINDOWS - 1; k >= 0; k--) {
-        if (k != KB_RC_WINDOWS - 1) {
+    for (int k = NW - 1; k >= 0; k--) {
+        if (k != NW - 1) {
             KB_NOUNROLL
             for (int b = 0; b < 8; b++) ge_dbl_rt(W, W, b == 7);
         }

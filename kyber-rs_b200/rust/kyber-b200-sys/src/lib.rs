@@ -97,6 +97,7 @@ extern "C" {
     pub fn kb_vss_verify_deals_batch(ctx: *mut kb_ctx, npoly: usize, t: usize, commits: *const u8, m: usize, poly_id: *const u32, idx: *const u32, shares: *const u8, verdict: *mut u8) -> c_int;
     pub fn kb_dkg_verify_round(ctx: *mut kb_ctx, n: usize, t: usize, dealer_lo: usize, dealer_hi: usize, commits: *const u8, shares: *const u8, verdict: *mut u8) -> c_int;
     pub fn kb_dkg_verify_round_limbs(ctx: *mut kb_ctx, n: usize, t: usize, dealer_lo: usize, dealer_hi: usize, commit_limbs: *const i32, shares: *const u8, verdict: *mut u8) -> c_int;
+    pub fn kb_dkg_verify_columns(ctx: *mut kb_ctx, n: usize, t: usize, dealer_lo: usize, dealer_hi: usize, ver_lo: usize, ver_hi: usize, fmt: c_int, commits: *const c_void, shares: *const u8, verdict: *mut u8) -> c_int;
     pub fn kb_ctx_set_round_check(ctx: *mut kb_ctx, mode: c_int) -> c_int;
     pub fn kb_ctx_round_fallbacks(ctx: *mut kb_ctx, dealers: *mut u64) -> c_int;
 
@@ -136,6 +137,7 @@ extern "C" {
     pub fn kb_dev_msm_ext(ctx: *mut kb_ctx, n: usize, d_scalars: *const c_void, d_points128: *const c_void, d_out32: *mut c_void, d_partial128: *mut c_void, d_bad_points: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn kb_dev_dkg_verify_round(ctx: *mut kb_ctx, n: usize, t: usize, ndealers: usize, d_commits: *const c_void, d_shares: *const c_void, d_verdict: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn kb_dev_dkg_verify_round_limbs(ctx: *mut kb_ctx, n: usize, t: usize, ndealers: usize, d_commit_limbs: *const c_void, d_shares: *const c_void, d_verdict: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn kb_dev_dkg_verify_columns(ctx: *mut kb_ctx, n: usize, t: usize, ndealers: usize, ver_lo: usize, ver_hi: usize, fmt: c_int, d_commits: *const c_void, d_shares: *const c_void, d_verdict: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn kb_dev_point_sum(ctx: *mut kb_ctx, k: usize, d_partials128: *const c_void, d_out32: *mut c_void, stream: *mut c_void) -> c_int;
 
     pub fn kb_pripoly_eval_batch(ctx: *mut kb_ctx, npoly: usize, t: usize, coeffs: *const u8, n: usize, out: *mut u8) -> c_int;

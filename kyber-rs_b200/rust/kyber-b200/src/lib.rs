@@ -59,6 +59,20 @@ impl Gpu {
         self.check(unsafe { sys::kb_ctx_round_fallbacks(self.ctx, &mut d) })?;
         Ok(d)
     }
+    /// The share checks participants `ver_lo..ver_hi` run in `process_deal` (share/dkg/pedersen/dkg.rs:513-597), for every
+    /// dealer in one call: `polys[d]` is dealer `d`'s committed polynomial and `shares[d * k + c]` the share it sent to
+    /// verifier `ver_lo + c`, `k = ver_hi - ver_lo` (`k = 1` for one node).  `verdict[d * k + c]` is what
+    /// `Aggregator::verify_deal` (vss.rs:899-912) decides; exact in both round-check modes.
+    pub fn dkg_verify_columns(&self, n: usize, polys: &[Vec<EdPoint>], ver_lo: usize, ver_hi: usize, shares: &[EdScalar]) -> Result<Vec<bool>, GpuError> {
+        let t = polys.first().map(|p| p.len()).unwrap_or(0);
+        let k = ver_hi.saturating_sub(ver_lo);
+        assert!(polys.iter().all(|p| p.len() == t) && shares.len() == polys.len() * k);
+        let limbs: Vec<i32> = polys.iter().flat_map(|p| pack_point_limbs(p)).collect();
+        let sh = pack_scalars(shares);
+        let mut verdict = vec![0u8; shares.len()];
+        self.check(unsafe { sys::kb_dkg_verify_columns(self.ctx, n, t, 0, polys.len(), ver_lo, ver_hi, 1, limbs.as_ptr().cast(), sh.as_ptr(), verdict.as_mut_ptr()) })?;
+        Ok(verdict.into_iter().map(|v| v == 1).collect())
+    }
     fn check(&self, rc: i32) -> Result<(), GpuError> {
         match rc {
             sys::KB_OK => Ok(()),
